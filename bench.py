@@ -171,6 +171,32 @@ class ClockSampler:
         return out
 
 
+DUMP_BYTES = 64 * 1024 * 1024  # --dump-outputs writes at most this much
+DUMP_SAMPLE_PIXELS = 1 << 20
+
+
+def write_outputs(directory, arrays):
+    """`--dump-outputs DIR`: each array as DIR/<name>.npy, float64 where the data is float64 (the ray counters
+    are passed as such), float32 otherwise.  An image of more than half of DUMP_BYTES (the 4K frames, the 8K tone-mapped frame)
+    is stored as a fixed sample of DUMP_SAMPLE_PIXELS pixels, drawn without replacement with numpy seed 0:
+    <name>.npy holds their values (pixels x channels), <name>_index.npy their flat indices in ascending order."""
+    out = {}
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        dtype = np.float64 if a.dtype == np.float64 else np.float32
+        if a.size * np.dtype(dtype).itemsize > DUMP_BYTES // 2:
+            pixels = a.reshape(-1, a.shape[-1])
+            index = np.sort(np.random.default_rng(0).choice(pixels.shape[0], DUMP_SAMPLE_PIXELS, replace=False))
+            out[name], out[name + "_index"] = pixels[index].astype(dtype), index.astype(np.float64)
+        else:
+            out[name] = a.astype(dtype)
+    total = sum(a.nbytes for a in out.values())
+    assert total <= DUMP_BYTES, f"--dump-outputs: {total} bytes"
+    os.makedirs(directory, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def cpu_baseline_sample(name, threads, width=None, height=None):
     """The oracle on a bounded sample of the same workload: the same scene and settings at 1 sample per
     pixel — the full frame for demo.txt, a crop-sized frame for the many-sphere scenes (ms per ray there;
@@ -276,6 +302,8 @@ def run_tonemap(args, rank, local_rank, world_size):
         if i >= args.warmup:
             lum_ms.append(st["lum_ms"]); map_ms.append(st["map_ms"]); total_ms.append(st["lum_ms"] + st["map_ms"])
     clocks = sampler.stop()
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, {"ldr": ldr.cpu().numpy(), "luminosity": np.array([st["luminosity"]])})
     # end to end: host image in (pinned), LDR bytes out
     himg = torch.empty((h, w, 3), dtype=torch.float32).pin_memory()
     himg.copy_(img)
@@ -364,9 +392,10 @@ class Session:
 
 
 def measure_device(sess, name, steps, warmup, variant="auto", precision="auto", accel="none", partition="rows",
-                   exchange="allgather", sample_clocks=False):
+                   exchange="allgather", sample_clocks=False, keep_outputs=False):
     """Device-resident arm: scene and image in HBM, CUDA events on the launch stream around render (+ the
-    exchange at N > 1), L2 evicted between timed steps; max over ranks."""
+    exchange at N > 1), L2 evicted between timed steps; max over ranks.  `keep_outputs`: the result's
+    `outputs` holds what the last timed step computed (the frame, and its counters summed over ranks)."""
     from pytracer_b200 import _abi
     from pytracer_b200.device import DeviceScene
     from pytracer_b200.dist import (PeerImages, RowSlabs, partition_params, render_rows_allgather, render_rows_push)
@@ -380,6 +409,7 @@ def measure_device(sess, name, steps, warmup, variant="auto", precision="auto", 
     part_name = "none"
     if G == 1:
         image = torch.empty((H, W, 3), dtype=torch.float32, device="cuda")
+        frame = lambda: image  # noqa: E731
 
         def step():
             scene.render_device(params, image.data_ptr(), 0, sess.stream)
@@ -387,6 +417,7 @@ def measure_device(sess, name, steps, warmup, variant="auto", precision="auto", 
         p = partition_params(params, sess.rank, G, "spp")
         part_name = {_abi.RT_PART_SPP: "spp", _abi.RT_PART_ROWS: "rows"}[p.part_mode] + " + all-reduce"
         image = torch.empty((H, W, 3), dtype=torch.float32, device="cuda")
+        frame = lambda: image  # noqa: E731
 
         def step():
             scene.render_device(p, image.data_ptr(), 0, sess.stream)
@@ -402,12 +433,14 @@ def measure_device(sess, name, steps, warmup, variant="auto", precision="auto", 
                 peers, why = None, why or "the symmetric-memory rendezvous failed on another rank"
         if peers is not None:
             part_name = "rows, pixels stored into every rank's image by the kernel over NVLink (symmetric memory) + barrier"
+            frame = lambda: peers.image  # noqa: E731
 
             def step():
                 render_rows_push(scene, params, comm, peers, sess.stream)
         else:
             slabs = RowSlabs(H, W, G)
             part_name = "rows + in-place NCCL all-gather of the row slabs" + (f" (peer images unavailable: {why})" if why else "")
+            frame = slabs.gathered_image
 
             def step():
                 render_rows_allgather(scene, params, comm, slabs, sess.stream)
@@ -439,13 +472,17 @@ def measure_device(sess, name, steps, warmup, variant="auto", precision="auto", 
     clocks = sampler.stop() if sampler else None
     total_ms = sess.reduce(sum(a.elapsed_time(b) for a, b in events), "max")
     rays = int(round(sess.reduce(float(rays_rank), "sum")))
+    outputs = None
+    if keep_outputs:
+        counters = [sess.reduce(float(st[k]), "sum") for k in ("rays_closest", "rays_shadow", "samples")]
+        outputs = {"image": frame().cpu().numpy(), "counters": np.array(counters, dtype=np.float64)}
     scene.close()
     k_ms = statistics.mean(kernel_ms)
     precision_used = {1: "f32", 2: "f64", 3: "hybrid"}.get(st.get("precision_used"), "?")
     return dict(value=rays / (total_ms * 1e-3), ms_per_step=total_ms / max(1, steps), rays_per_step=rays // max(1, steps),
                 kernel_ms=k_ms, rays_per_launch_rank=rays_rank / max(1, steps), launches=launches, wall=wall, clocks=clocks,
                 partition=part_name, precision_used=precision_used, desc=desc, flops_per_ray=flops_per_ray, n_sph=n_sph,
-                H=H, W=W, variant=variant, accel=accel)
+                H=H, W=W, variant=variant, accel=accel, outputs=outputs)
 
 
 def measure_e2e(sess, name, iters, warmup, variant="auto", precision="auto", accel="none"):
@@ -556,7 +593,9 @@ def run_ours(args, rank, local_rank, world_size):
     sess = Session(rank, local_rank, world_size)
     name = args.workload
     m = measure_device(sess, name, args.steps, args.warmup, variant=args.variant, precision=args.precision, accel=args.accel,
-                       partition=args.partition, exchange=args.exchange, sample_clocks=True)
+                       partition=args.partition, exchange=args.exchange, sample_clocks=True, keep_outputs=bool(args.dump_outputs))
+    if args.dump_outputs and rank == 0:
+        write_outputs(args.dump_outputs, m["outputs"])
     e2e = measure_e2e(sess, name, args.steps, args.warmup, variant=args.variant, precision=args.precision, accel=args.accel)
 
     # ---- the other BASELINE configs, measured in the same job (1-2 steps each; `--no-extra` skips them)
@@ -622,7 +661,14 @@ def main():
     ap.add_argument("--no-extra", action="store_true", help="skip the `configs` sub-results (configs 4 and 5)")
     ap.add_argument("--scale", type=int, default=1, help="divide width and height by this (quick experiments only; "
                     "a scaled run is NOT the benchmark and says so in config)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed (the frame "
+                    "and its ray counters; tonemap: the 8-bit frame and the luminosity) as DIR/<name>.npy, at most 64 MB: "
+                    "the inputs are seeded, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference" and args.workload != "tonemap":
+        ap.error("--dump-outputs writes the outputs of the device path (--impl ours)")
     global SCALE
     SCALE = max(1, args.scale)
     rank = int(os.environ.get("RANK", "0"))

@@ -14,7 +14,7 @@ from pytracer_b200.device import DeviceScene
 from pytracer_b200.flatten import flatten_camera, flatten_world
 from pytracer_b200.params import make_params
 from pytracer_b200.pcg import PCG
-from util import assert_luminance_agreement, assert_mc_agreement, c1_params, demo_flat, golden, luminosity, scene2_flat
+from util import assert_luminance_agreement, assert_mc_agreement, c1_params, demo_flat, golden, luminosity, scene2_flat, sha256_of
 
 pytestmark = pytest.mark.gpu
 
@@ -166,8 +166,12 @@ def test_config2_1080p_bit_exact_hit_index_and_colours():
         counts = np.bincount(hit.ravel() + 1, minlength=4)
         assert counts.tolist() == [484487, 518387, 1002874, 67852]
         assert np.allclose(rgb.astype(np.float64).reshape(-1, 3).mean(0), g[f"{algo}_mean"], rtol=1e-6)
-        if algo != "onoff":
-            assert_colors_close(rgb, g[f"{algo}_rgb_f32"], rel=REL)
+        if algo == "flat":
+            assert_colors_close(rgb, g["flat_rgb_f32"], rel=REL)
+        elif algo == "pointlight":  # the reference's image is stored as a digest; the oracle renders it bit for bit
+            want = oracle.render(fs, make_params(1920, 1080, cam, algo, 0), want_hit=False)["rgb"].astype(np.float32)
+            assert sha256_of(want) == str(g["pointlight_rgb_f32_sha256"])
+            assert_colors_close(rgb, want, rel=REL)
         assert [stats["rays_closest"], stats["rays_shadow"]] == g[f"{algo}_rays"].tolist()
 
 

@@ -7,7 +7,7 @@ import pytest
 from oracle import oracle
 from pytracer_b200.params import make_params
 from pytracer_b200.pcg import PCG
-from util import c1_params, demo_flat, golden, scene2_flat
+from util import c1_params, demo_flat, golden, scene2_flat, sha256_of
 
 
 def test_pcg_known_answers():
@@ -147,7 +147,7 @@ def test_1080p_config2_bit_exact():
     counts = np.bincount(r["hit_index"].ravel() + 1, minlength=4)
     assert counts.tolist() == [484487, 518387, 1002874, 67852]  # BASELINE.md golden anchors
     r = oracle.render(fs, make_params(1920, 1080, cam, "pointlight", 0))
-    assert np.array_equal(r["rgb"].astype(np.float32), g["pointlight_rgb_f32"])
+    assert sha256_of(r["rgb"].astype(np.float32)) == str(g["pointlight_rgb_f32_sha256"])
     assert [r["rays_closest"], r["rays_shadow"]] == g["pointlight_rays"].tolist() == [2073600, 1589113]
 
 

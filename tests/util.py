@@ -1,5 +1,6 @@
 """Shared helpers of the test-suite: golden fixtures (outputs of the unmodified reference, see
 tests/golden/make_golden.py) and scene rebuilding from them."""
+import hashlib
 import os
 
 import numpy as np
@@ -14,6 +15,11 @@ GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 def golden(name):
     return np.load(os.path.join(GOLDEN, name))
+
+
+def sha256_of(a) -> str:
+    """Digest of an array's bytes: what a fixture keeps of an image too large to store."""
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
 
 
 def camera_from(vec) -> _abi.rt_camera:
