@@ -260,6 +260,36 @@ int rt_render_device(rt_scene* scene, const rt_render_params* params, void* d_ou
                      int32_t* d_out_hit_index, void* stream);
 int rt_render_finish(rt_scene* scene, void* stream, rt_stats* stats);
 
+/* ---- path tracing with a per-pixel error map and noise-targeted passes ----
+ * Pass p (p = 0, 1, ...) of a pixel is that pixel of the (p+1)-th consecutive fire_all_rays with the same
+ * tracer and renderer: jitter stream advanced by p * 2 * W * H * S^2 draws, pt_state by p PCG steps, sample
+ * indices k = pix * S^2 + s.  Pass 0 traces every pixel; every further pass traces, in ascending order, the
+ * pixels whose relative error e = max_c SE_c / max(mean_c, error_floor) is still above target_error and that
+ * have passes left.  A pass's squared standard error comes from batch sums of its S^2 samples,
+ * SE^2 = sum_b (T_b - n_b m)^2 / (n_b (B - 1) S^2).  A pixel with P passes reports mean = (sum of pass means,
+ * fp32, in pass order) / P, SE = sqrt(sum of SE^2) / P and P * S^2 samples; with P = 1 the mean is rt_render's
+ * pixel bit for bit.  Path tracing, WARP variant (AUTO picks it), fp32, S >= 2, RT_PART_NONE, RT_RNG_STREAMS,
+ * no peer images, no out_f64: anything else is RT_ERR_INVALID.  Host buffers, blocking; one device. */
+typedef struct rt_adaptive_params {
+  double target_error;        /* e threshold; <= 0: one pass, error map only */
+  double error_floor;         /* absolute radiance floor of the relative error (> 0) */
+  int32_t max_passes;         /* >= 1; pass p uses the PCG states defined above */
+  int32_t _pad;
+} rt_adaptive_params;
+typedef struct rt_adaptive_stats {
+  uint64_t rays_closest, rays_shadow, samples;
+  float kernel_ms;            /* CUDA events around all passes (render, combine, select) and the final kernel */
+  float total_ms;             /* the whole call, device->host copies included */
+  int32_t passes;             /* passes actually run */
+  int32_t n_launches;
+  int64_t pixels_in_pass[16]; /* first 16 passes: list length traced in each */
+  int32_t overflow;           /* non-zero: a warp work stack overflowed, the image is invalid (RT_ERR_OVERFLOW) */
+  int32_t _pad;
+} rt_adaptive_stats;
+/* out_rgb float[H][W][3] mean; out_err float[H][W][3] SE (optional); out_samples int32[H][W] (optional) */
+int rt_render_adaptive(rt_scene* scene, const rt_render_params* params, const rt_adaptive_params* ap,
+                       float* out_rgb, float* out_err, int32_t* out_samples, rt_adaptive_stats* stats);
+
 /* ---- Renderer.__call__(ray) for explicit rays (render.py:52,65,99,157) ----
  * rays: double[n][8] = origin xyz, dir xyz, tmin, tmax; depth int32[n] (NULL = 0).
  * pcg_state_inc: {state, inc} of PathTracer.pcg, read and written back (rays are traced

@@ -145,6 +145,35 @@ class rt_tonemap_stats(C.Structure):
         return {name: getattr(self, name) for name, _ in self._fields_}
 
 
+class rt_adaptive_params(C.Structure):
+    _fields_ = [
+        ("target_error", C.c_double),
+        ("error_floor", C.c_double),
+        ("max_passes", C.c_int32),
+        ("_pad", C.c_int32),
+    ]
+
+
+class rt_adaptive_stats(C.Structure):
+    _fields_ = [
+        ("rays_closest", C.c_uint64),
+        ("rays_shadow", C.c_uint64),
+        ("samples", C.c_uint64),
+        ("kernel_ms", C.c_float),
+        ("total_ms", C.c_float),
+        ("passes", C.c_int32),
+        ("n_launches", C.c_int32),
+        ("pixels_in_pass", C.c_int64 * 16),
+        ("overflow", C.c_int32),
+        ("_pad", C.c_int32),
+    ]
+
+    def as_dict(self) -> dict:
+        d = {name: getattr(self, name) for name, _ in self._fields_ if name != "_pad"}
+        d["pixels_in_pass"] = [int(v) for v in self.pixels_in_pass[: min(self.passes, 16)]]
+        return d
+
+
 class rt_hit(C.Structure):
     _fields_ = [
         ("shape", C.c_int32),

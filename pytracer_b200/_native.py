@@ -33,6 +33,8 @@ _PROTOTYPES = {
     "rt_render_multi": (C.c_int, [C.POINTER(_P), C.c_int32, C.POINTER(_abi.rt_render_params), _P, _P, C.POINTER(_abi.rt_stats)]),
     "rt_render_device": (C.c_int, [_P, C.POINTER(_abi.rt_render_params), _P, _P, _P]),
     "rt_render_finish": (C.c_int, [_P, _P, C.POINTER(_abi.rt_stats)]),
+    "rt_render_adaptive": (C.c_int, [_P, C.POINTER(_abi.rt_render_params), C.POINTER(_abi.rt_adaptive_params), _P, _P, _P,
+                                     C.POINTER(_abi.rt_adaptive_stats)]),
     "rt_trace_rays": (C.c_int, [_P, C.POINTER(_abi.rt_render_params), _P, _P, C.c_int32, _P, _P]),
     "rt_intersect": (C.c_int, [_P, C.c_int32, C.c_int32, _P, C.c_int32, _P]),
     "rt_is_point_visible": (C.c_int, [_P, C.c_int32, _P, C.c_int32, _P]),

@@ -13,6 +13,7 @@ nvcc $ARCH $COMMON -c rt_kernels_f32.cu -o $B/rt_kernels_f32.o & pids+=($!)
 nvcc $ARCH $COMMON --fmad=false -c rt_kernels_f64.cu -o $B/rt_kernels_f64.o & pids+=($!)
 nvcc $ARCH $COMMON -c rt_api.cu -o $B/rt_api.o & pids+=($!)
 nvcc $ARCH $COMMON --fmad=false -c rt_tonemap.cu -o $B/rt_tonemap.o & pids+=($!)
+nvcc $ARCH $COMMON -c rt_adaptive.cu -o $B/rt_adaptive.o & pids+=($!)
 for pid in "${pids[@]}"; do wait "$pid"; done  # set -e: a failed translation unit fails the build
-nvcc $ARCH -shared -o $OUT $B/rt_kernels_f32.o $B/rt_kernels_f64.o $B/rt_api.o $B/rt_tonemap.o -lcudart_static -lpthread -ldl -lrt
+nvcc $ARCH -shared -o $OUT $B/rt_kernels_f32.o $B/rt_kernels_f64.o $B/rt_api.o $B/rt_tonemap.o $B/rt_adaptive.o -lcudart_static -lpthread -ldl -lrt
 [ -f $OUT ] && echo "built $(realpath $OUT)"

@@ -61,6 +61,9 @@ struct Workspace {
   size_t hdr_out_cap = 0;
   void* co = nullptr;  // per-(origin, sphere) gate records of the hybrid resolve kernel
   size_t co_cap = 0;
+  void* adaptive = nullptr;  // rt_render_adaptive: per-pixel sums, pass outputs, pixel lists
+  size_t adaptive_cap = 0;
+  int32_t* count_host = nullptr;  // pinned: the length of the next pass's pixel list
 };
 
 struct rt_scene {
@@ -723,6 +726,120 @@ extern "C" int rt_render_multi(rt_scene* const* scenes, int32_t n_scenes, const 
   cudaSetDevice(entry_device);
   if (rc != RT_OK) { memcpy(g_err, first_error, sizeof(g_err)); return rc; }
   if (stats) *stats = total;
+  return RT_OK;
+}
+
+// x -> MULT x + inc applied `delta` times (PCG.advance on the host, pcg.py)
+static uint64_t lcg_advance(uint64_t state, uint64_t inc, uint64_t delta) {
+  uint64_t acc_mult = 1, acc_plus = 0, cur_mult = RT_PCG_MULT, cur_plus = inc;
+  for (; delta; delta >>= 1) {
+    if (delta & 1) { acc_mult *= cur_mult; acc_plus = acc_plus * cur_mult + cur_plus; }
+    cur_plus = (cur_mult + 1) * cur_plus;
+    cur_mult *= cur_mult;
+  }
+  return acc_mult * state + acc_plus;
+}
+
+// Path tracing with an error map and noise-targeted passes (rt_api.h).  Every per-pixel quantity stays on
+// the device for the whole call: pass p runs the error-map path tracer over the current pixel list (pass 0:
+// the image), rt_adaptive.cu folds its means and SE^2 into the per-pixel sums and writes the next list;
+// the host reads one count per pass.
+extern "C" int rt_render_adaptive(rt_scene* s, const rt_render_params* p, const rt_adaptive_params* ap, float* out_rgb, float* out_err,
+                                  int32_t* out_samples, rt_adaptive_stats* stats) {
+  if (!s || !p || !ap || !out_rgb) return fail(RT_ERR_INVALID, "rt_render_adaptive: null argument");
+  if (p->algorithm != RT_ALGO_PATHTRACING) return fail(RT_ERR_INVALID, "rt_render_adaptive: path tracing only");
+  if (p->samples_per_side < 2) return fail(RT_ERR_INVALID, "rt_render_adaptive: samples_per_side %d (the error map needs >= 2)", p->samples_per_side);
+  if (p->variant != RT_VARIANT_AUTO && p->variant != RT_VARIANT_WARP) return fail(RT_ERR_INVALID, "rt_render_adaptive: the warp variant only");
+  if (p->precision != RT_PRECISION_AUTO && p->precision != RT_PRECISION_F32) return fail(RT_ERR_INVALID, "rt_render_adaptive: fp32 only");
+  if (p->part_mode != RT_PART_NONE || p->n_peer_images != 0 || p->out_f64 || p->rng_mode != RT_RNG_STREAMS)
+    return fail(RT_ERR_INVALID, "rt_render_adaptive: one device, RT_PART_NONE, RT_RNG_STREAMS, an fp32 image and no peer images");
+  if (p->num_of_rays < 1 || p->max_depth < 0) return fail(RT_ERR_INVALID, "rt_render_adaptive: num_of_rays %d, max_depth %d", p->num_of_rays, p->max_depth);
+  if (ap->max_passes < 1 || !(ap->error_floor > 0.0) || std::isnan(ap->target_error))
+    return fail(RT_ERR_INVALID, "rt_render_adaptive: max_passes %d, error_floor %g, target_error %g", ap->max_passes, ap->error_floor, ap->target_error);
+  if ((long long)p->width * p->height >= (1ll << 31)) return fail(RT_ERR_INVALID, "rt_render_adaptive: image too large");
+  CU(cudaSetDevice(s->device));
+  RenderArgs a;
+  int rc = fill_args(s, p, &a);
+  if (rc != RT_OK) return rc;
+  Workspace* ws = s->ws;
+  const int n = p->width * p->height;
+  const int S2 = p->samples_per_side * p->samples_per_side;
+  const int max_passes = ap->target_error > 0.0 ? ap->max_passes : 1;
+  if (p->accel != RT_ACCEL_NONE && p->accel != RT_ACCEL_BVH) return fail(RT_ERR_INVALID, "accel %d", p->accel);
+  const int accel = (p->accel == RT_ACCEL_BVH && s->n_spheres > 0) ? RT_ACCEL_BVH : RT_ACCEL_NONE;
+  cudaStream_t st = 0;
+  if (accel == RT_ACCEL_BVH && (rc = ensure_bvh(s, st)) != RT_OK) return rc;
+  SceneView<float> v32 = view_of<float>(s);
+  v32.accel = accel;
+  // device layout: pass mean / SE^2 per list entry, per-pixel sums and pass counts, two lists, flags, tile counts
+  const size_t n3 = 3 * (size_t)n * sizeof(float), tiles = (size_t)n / 2048 + 2;
+  auto al = [](size_t x) { return (x + 255) / 256 * 256; };
+  const size_t o_em = 0, o_ev = o_em + al(n3), o_sm = o_ev + al(n3), o_sv = o_sm + al(n3), o_np = o_sv + al(n3);
+  const size_t o_l0 = o_np + al((size_t)n * 4), o_l1 = o_l0 + al((size_t)n * 4), o_fl = o_l1 + al((size_t)n * 4);
+  const size_t o_bc = o_fl + al((size_t)n), o_cnt = o_bc + al(tiles * 4), total = o_cnt + 256;
+  if ((rc = ensure(&ws->adaptive, &ws->adaptive_cap, total)) != RT_OK) return rc;
+  if (!ws->count_host) CU(cudaMallocHost((void**)&ws->count_host, sizeof(int32_t)));
+  unsigned char* base = (unsigned char*)ws->adaptive;
+  float *em = (float*)(base + o_em), *ev = (float*)(base + o_ev), *sm = (float*)(base + o_sm), *sv = (float*)(base + o_sv);
+  int32_t* n_pass = (int32_t*)(base + o_np);
+  int32_t* lists[2] = {(int32_t*)(base + o_l0), (int32_t*)(base + o_l1)};
+  uint8_t* flags = base + o_fl;
+  int32_t *block_counts = (int32_t*)(base + o_bc), *d_count = (int32_t*)(base + o_cnt);
+
+  rt_adaptive_stats out;
+  memset(&out, 0, sizeof(out));
+  LaunchInfo info = {0, RT_VARIANT_WARP};
+  CU(cudaEventRecord(ws->t0, st));
+  CU(cudaMemsetAsync(ws->counters, 0, CNT_SLOTS * sizeof(unsigned long long), st));
+  CU(cudaEventRecord(ws->ev0, st));
+  const uint64_t draws_per_image = 2ull * (uint64_t)n * (uint64_t)S2;
+  long long n_cur = n;
+  int passes = 0;
+  for (int pass = 0; pass < max_passes && n_cur > 0; ++pass) {
+    // pass p = the (p+1)-th consecutive image: ImageTracer.pcg after p images, PathTracer.pcg after p random() calls
+    a.aa_state = lcg_advance(p->aa_state, p->aa_inc, (uint64_t)pass * draws_per_image);
+    a.pt_state = lcg_advance(p->pt_state, a.pt_inc, (uint64_t)pass);
+    ErrArgs e;
+    memset(&e, 0, sizeof(e));
+    e.pix_list = pass == 0 ? nullptr : lists[pass & 1];
+    e.n_list = n_cur;
+    e.err_mean = em;
+    e.err_var = ev;
+    CU(cudaMemsetAsync(ws->counters + CNT_TASK, 0, sizeof(unsigned long long), st));
+    const char* why = nullptr;
+    cudaError_t err = launch_pt_warp_err(v32, a, e, st, s->sm_count, &info, &why, s->bvh_n_nodes, s->bvh_n_prims, s->bvh_depth);
+    if (err != cudaSuccess) return fail(why ? RT_ERR_INVALID : RT_ERR_CUDA, "rt_render_adaptive: %s", why ? why : cudaGetErrorString(err));
+    err = launch_adaptive_combine(e, pass, max_passes, (float)ap->target_error, (float)ap->error_floor, sm, sv, n_pass, flags, block_counts,
+                                  d_count, lists[(pass + 1) & 1], n, st, &info);
+    if (err != cudaSuccess) return fail(RT_ERR_CUDA, "rt_render_adaptive: %s", cudaGetErrorString(err));
+    if (pass < 16) out.pixels_in_pass[pass] = n_cur;
+    passes = pass + 1;
+    if (pass + 1 < max_passes) {  // the one host read of the pass: how many pixels the next pass traces
+      CU(cudaMemcpyAsync(ws->count_host, d_count, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+      CU(cudaStreamSynchronize(st));
+      n_cur = *ws->count_host;
+    }
+  }
+  cudaError_t err = launch_adaptive_final(sm, sv, n_pass, S2, n, em, out_err ? ev : nullptr, out_samples ? lists[0] : nullptr, st, &info);
+  if (err != cudaSuccess) return fail(RT_ERR_CUDA, "rt_render_adaptive: %s", cudaGetErrorString(err));
+  CU(cudaEventRecord(ws->ev1, st));
+  CU(cudaMemcpyAsync(out_rgb, em, n3, cudaMemcpyDeviceToHost, st));
+  if (out_err) CU(cudaMemcpyAsync(out_err, ev, n3, cudaMemcpyDeviceToHost, st));
+  if (out_samples) CU(cudaMemcpyAsync(out_samples, lists[0], (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+  CU(cudaMemcpyAsync(ws->counters_host, ws->counters, CNT_SLOTS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+  CU(cudaEventRecord(ws->t1, st));
+  CU(cudaStreamSynchronize(st));
+  out.rays_closest = ws->counters_host[CNT_CLOSEST];
+  out.rays_shadow = ws->counters_host[CNT_SHADOW];
+  out.samples = ws->counters_host[CNT_SAMPLES];
+  out.overflow = (int32_t)ws->counters_host[CNT_OVERFLOW];
+  out.passes = passes;
+  out.n_launches = info.n_launches;
+  CU(cudaEventElapsedTime(&out.kernel_ms, ws->ev0, ws->ev1));
+  CU(cudaEventElapsedTime(&out.total_ms, ws->t0, ws->t1));
+  s->pending = false;
+  if (stats) *stats = out;
+  if (out.overflow) return fail(RT_ERR_OVERFLOW, "a warp work stack overflowed; the image is invalid");
   return RT_OK;
 }
 

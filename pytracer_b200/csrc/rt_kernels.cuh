@@ -55,6 +55,23 @@ __host__ __device__ inline PixelMap make_pixel_map(const RenderArgs& a) {
   return pm;
 }
 
+// List mode of the pixel map (the error-map kernels' sparse passes): with e.pix_list set, the tasks run over
+// its n_list entries and entry p is the full-image pixel pix_list[p]; otherwise over the image
+__host__ __device__ inline PixelMap make_pixel_map_list(const RenderArgs& a, const ErrArgs& e) {
+  PixelMap pm = make_pixel_map(a);
+  if (e.pix_list) pm.n_pixels = e.n_list;
+  return pm;
+}
+RT_DEV void locate_listed(const PixelMap& pm, const ErrArgs& e, long long p, int& col, int& row) {
+  if (e.pix_list) {
+    const unsigned px = (unsigned)__ldg(e.pix_list + p);
+    row = (int)(px / (unsigned)pm.width);
+    col = (int)(px - (unsigned)row * (unsigned)pm.width);
+  } else {
+    pm.locate(p, col, row);
+  }
+}
+
 RT_DEV bool stratum_is_mine(const RenderArgs& a, int s) {
   return !(a.part_mode == RT_PART_SPP && a.part_count > 1) || (s % a.part_count) == a.part_rank;
 }

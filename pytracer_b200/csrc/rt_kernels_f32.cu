@@ -18,6 +18,12 @@ cudaError_t launch_pt_warp(const SceneView<float>& sc, const RenderArgs& a, cuda
   return launch_pt_warp_impl(sc, a, st, sm_count, info, why_not);
 }
 
+cudaError_t launch_pt_warp_err(const SceneView<float>& sc, const RenderArgs& a, const ErrArgs& e, cudaStream_t st, int sm_count,
+                               LaunchInfo* info, const char** why_not, int n_nodes, int n_prims, int tree_depth) {
+  if (sc.accel) return launch_pt_warp_bvh<true>(sc, a, st, sm_count, info, why_not, n_nodes, n_prims, tree_depth, e);
+  return launch_pt_warp_impl<true>(sc, a, st, sm_count, info, why_not, e);
+}
+
 // FP32 FMA throughput probe: the denominator of the roofline this path is bound by.
 __global__ void __launch_bounds__(256) k_ffma(float* out, int iters, float a, float b) {
   float x0 = threadIdx.x, x1 = x0 + 1.f, x2 = x0 + 2.f, x3 = x0 + 3.f, x4 = x0 + 4.f, x5 = x0 + 5.f, x6 = x0 + 6.f, x7 = x0 + 7.f;

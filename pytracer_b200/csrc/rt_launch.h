@@ -23,6 +23,17 @@ struct RenderArgs {
   JumpTable jump;          // for the jitter stream (aa_inc)
 };
 
+// What the error-map instantiations of the warp path tracers read besides RenderArgs (the last kernel
+// parameter of every instantiation, so that the others keep their parameter offsets and code)
+struct ErrArgs {
+  const int32_t* pix_list; // non-null: the task source is this list of full-image pixels (row * width + col)
+  long long n_list;        // entries of pix_list
+  float* err_mean;         // [entries][3] pass mean of each traced pixel (list entry, or pixel index without a list)
+  float* err_var;          // [entries][3] squared standard error of that mean
+  int err_bpp;             // batches per pixel slot of a task (32 / G), set by the launcher
+  unsigned err_magic;      // multiply-shift magic of x / err_bpp for x < 32
+};
+
 struct LaunchInfo {
   int32_t n_launches;
   int32_t variant;
@@ -39,6 +50,17 @@ template <typename T> cudaError_t launch_pt_mega(const SceneView<T>& sc, const R
 // (n_nodes / n_prims / tree_depth describe the sphere hierarchy and are read only when sc.accel != 0)
 cudaError_t launch_pt_warp(const SceneView<float>& sc, const RenderArgs& a, cudaStream_t st, int sm_count, LaunchInfo* info, const char** why_not,
                            int n_nodes, int n_prims, int tree_depth);
+// the same kernels instantiated with per-pixel error accumulation (ERR): no image is stored; every traced
+// pixel gets its pass mean (the value launch_pt_warp stores, bit for bit) and squared standard error in
+// e.err_mean / e.err_var, indexed by list entry (e.pix_list) or pixel; needs S >= 2 and no partition
+cudaError_t launch_pt_warp_err(const SceneView<float>& sc, const RenderArgs& a, const ErrArgs& e, cudaStream_t st, int sm_count,
+                               LaunchInfo* info, const char** why_not, int n_nodes, int n_prims, int tree_depth);
+// rt_adaptive.cu: fold a pass into the per-pixel sums, then compact the pixels still to trace
+cudaError_t launch_adaptive_combine(const ErrArgs& e, int pass, int max_passes, float target, float floor_, float* sum_m, float* sum_v,
+                                    int32_t* n_pass, uint8_t* flags, int32_t* block_counts, int32_t* d_count, int32_t* next_list, int n_pixels,
+                                    cudaStream_t st, LaunchInfo* info);
+cudaError_t launch_adaptive_final(const float* sum_m, const float* sum_v, const int32_t* n_pass, int spp, int n_pixels, float* rgb, float* err,
+                                  int32_t* samples, cudaStream_t st, LaunchInfo* info);
 
 // single-stream probes behind rt_trace_rays / rt_intersect / ... (n items, one thread walks them
 // in order when a PCG stream is shared, otherwise one thread per item)

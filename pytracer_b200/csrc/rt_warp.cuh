@@ -47,6 +47,67 @@ struct WarpCfg {
   unsigned long long n_samples;  // samples this launch traces (all tasks), added to the counter once
 };
 
+// ---- error map (ERR instantiations) --------------------------------------------------------------------
+// The L samples a pixel traces in one pass fall into B = min(L, 32 / G) batches: sample ls goes to batch
+// ls mod (32 / G) and every ray of its tree inherits that batch through the 5-bit slot of its scatter record
+// (slot = pixel in task * (32 / G) + batch).  The warp keeps the 32 batch sums [32][3] in shared memory;
+// the squared standard error of the pass mean m follows from them when the task ends:
+//   SE^2 = sum_b (T_b - n_b m)^2 / (n_b (B - 1) L)
+// (unbiased for independent samples; B = L gives s^2 / L).
+RT_DEV int err_batch_of(const ErrArgs& cfg, int ls) {
+  return cfg.err_bpp == 32 ? (ls & 31) : ls - (int)(((unsigned)ls * cfg.err_magic) >> 16) * cfg.err_bpp;  // (ls < 32 when G > 1)
+}
+// Adds this lane's contribution to batch `slot` (all lanes call; `on`: the lane traced a ray).  Lanes of one
+// record are contiguous and share the slot: a segmented scan over runs of equal slots, then one shared
+// atomic per run, as ACC_SEG does for pixels.
+RT_DEV void err_batch_add(float* bsum, int slot, bool on, V3<float> c, int lane) {
+  const unsigned FULL = 0xffffffffu;
+  if (__ballot_sync(FULL, on && (c.x != 0.f || c.y != 0.f || c.z != 0.f)) == 0u) return;
+  const int key = on ? slot : 32 + lane;
+  const int prev = __shfl_up_sync(FULL, key, 1);
+  const unsigned heads = __ballot_sync(FULL, lane == 0 || prev != key);
+  const int seg_start = 31 - __clz(heads & (0xffffffffu >> (31 - lane)));
+#pragma unroll
+  for (int d = 1; d < 32; d <<= 1) {
+    const float r = __shfl_up_sync(FULL, c.x, d);
+    const float g = __shfl_up_sync(FULL, c.y, d);
+    const float b = __shfl_up_sync(FULL, c.z, d);
+    if (lane - d >= seg_start) { c.x += r; c.y += g; c.z += b; }
+  }
+  const bool tail = lane == 31 || ((heads >> (lane + 1)) & 1u);
+  if (on && tail && (c.x != 0.f || c.y != 0.f || c.z != 0.f)) {
+    atomicAdd(&bsum[3 * slot + 0], c.x);
+    atomicAdd(&bsum[3 * slot + 1], c.y);
+    atomicAdd(&bsum[3 * slot + 2], c.z);
+  }
+}
+// Pass mean m (the value the plain kernel stores, identical in all lanes) and SE^2 of pixel g of the task
+// to list entry `entry`.  All lanes call.
+RT_DEV void err_store(const ErrArgs& e, int L, const float* bsum, int g, long long entry, V3<float> m, int lane) {
+  const unsigned FULL = 0xffffffffu;
+  const int bpp = e.err_bpp, B = min(L, bpp);
+  float tr = 0.f, tg = 0.f, tb = 0.f;
+  if (lane < B) {
+    const float n = (float)((L - 1 - lane) / bpp + 1);
+    const float* t = bsum + 3 * (g * bpp + lane);
+    const float dr = fmaf(-n, m.x, t[0]), dg = fmaf(-n, m.y, t[1]), db = fmaf(-n, m.z, t[2]);
+    tr = dr * dr / n; tg = dg * dg / n; tb = db * db / n;
+  }
+#pragma unroll
+  for (int d = 16; d > 0; d >>= 1) {
+    tr += __shfl_xor_sync(FULL, tr, d);
+    tg += __shfl_xor_sync(FULL, tg, d);
+    tb += __shfl_xor_sync(FULL, tb, d);
+  }
+  if (lane == 0) {
+    const float k = 1.f / ((float)(B - 1) * (float)L);
+    float* o = e.err_mean + 3 * entry;
+    o[0] = m.x; o[1] = m.y; o[2] = m.z;
+    float* v = e.err_var + 3 * entry;
+    v[0] = tr * k; v[1] = tg * k; v[2] = tb * k;
+  }
+}
+
 // SMALL instantiation: every table of the scene lives in shared memory at FIXED offsets (capacity for
 // the largest small scene, 3.3 KB), re-packed by the staging loop into what the per-ray code reads:
 //   SM_INVM / SM_M   [16][12] fp32 transforms (three LDS.128 per shape)
@@ -215,10 +276,12 @@ RT_DEV int own_stratum(const RenderArgs& a, int ls) {
 enum { ACC_REG = 0, ACC_LANES = 1, ACC_SEG = 2 };
 #define RT_ACC_LANES_MAX_GROUP 8
 
-template <bool SHAPES_SMEM, int ACC, bool SMALL>
+// ERR: error-map instantiation (see err_batch_add): tasks over ea.pix_list when set, and instead of the image
+// every pixel's pass mean and SE^2 go to ea.err_mean / ea.err_var; the slot of a scatter record is then the batch.
+template <bool SHAPES_SMEM, int ACC, bool SMALL, bool ERR = false>
 __global__ void __launch_bounds__(SMALL ? RT_SMALL_THREADS : RT_WARP_MAX_THREADS, SMALL ? RT_SMALL_MINB : 2)
 k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ RenderArgs a,
-          const __grid_constant__ WarpCfg cfg) {
+          const __grid_constant__ WarpCfg cfg, const __grid_constant__ ErrArgs ea) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const unsigned FULL = 0xffffffffu;
   const int warp = threadIdx.x >> 5;
@@ -258,9 +321,11 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
   constexpr bool MULTI_SLOT = ACC != ACC_REG;
   int* slot_rays = reinterpret_cast<int*>(smem_raw + wofs + (size_t)(cfg.cap + 1) * sizeof(ScatterRec));  // [32], multi-pixel tasks + RT_HIT_RAY_COUNT
   float* acc = reinterpret_cast<float*>(slot_rays + 32);   // ACC_SEG: [32][3]; ACC_LANES: [G][3][32]
+  // ERR: batch sums [32][3] behind the accumulator (ACC_REG has neither slot_rays nor acc: they go there)
+  float* bsum = ACC == ACC_REG ? reinterpret_cast<float*>(slot_rays) : acc + (ACC == ACC_SEG ? 96 : 96 * cfg.group);
   const bool count_rays = a.out_hit != nullptr && a.hit_mode == RT_HIT_RAY_COUNT;
 
-  const PixelMap pm = make_pixel_map(a);
+  const PixelMap pm = ERR ? make_pixel_map_list(a, ea) : make_pixel_map(a);
   const int N = a.num_of_rays;
   const int S2 = a.S > 0 ? a.S * a.S : 1;
   const int G = cfg.group, L = cfg.per_pixel;
@@ -281,7 +346,8 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
     uint64_t aa_task = a.aa_state;
     if (ACC == ACC_REG && a.S > 0 && p0 < pm.n_pixels) {
       int col, row;
-      pm.locate(p0, col, row);
+      if (ERR) locate_listed(pm, ea, p0, col, row);
+      else pm.locate(p0, col, row);
       aa_task = pcg_jump(a.aa_state, 2ull * (unsigned long long)((long long)row * a.width + col) * S2, a.jump);
     }
     float sr = 0.f, sg = 0.f, sb_ = 0.f;  // lane-private sums (single-slot tasks)
@@ -291,6 +357,10 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
       if (ACC == ACC_SEG) { for (int i = lane; i < 96; i += 32) acc[i] = 0.f; }
       else { for (int i = 0; i < 3 * cfg.group; ++i) acc[i * 32 + lane] = 0.f; }
       slot_rays[lane] = 0;
+      __syncwarp();
+    }
+    if (ERR) {
+      for (int i = lane; i < 96; i += 32) bsum[i] = 0.f;
       __syncwarp();
     }
 
@@ -310,16 +380,19 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
         Pcg rng;
         long long pix = 0;
         bool last_of_pixel = false;
+        int rslot = 0;  // ERR: the slot field of this ray's records, the batch (`slot` stays the pixel in the task)
         if (primary_phase) {
           const int j = round * 32 + lane;
           slot = j / L;
           const int ls = j - slot * L;
           const long long p = p0 + slot;
+          if (ERR) rslot = slot * ea.err_bpp + err_batch_of(ea, ls);
           active = (j < G * L) && (p < pm.n_pixels);
           task_rays += (unsigned)min(max(task_prims - round * 32, 0), 32);
           if (active) {
             int col, row;
-            pm.locate(p, col, row);
+            if (ERR) locate_listed(pm, ea, p, col, row);
+            else pm.locate(p, col, row);
             pix = (long long)row * a.width + col;
             const int s = own_stratum(a, ls);
             const unsigned long long k = (unsigned long long)pix * S2 + s;
@@ -367,6 +440,7 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
           if (active) {
             const int meta = __float_as_int(rec.a.w);
             slot = meta & 31;
+            if (ERR) { rslot = slot; slot = (int)(((unsigned)rslot * ea.err_magic) >> 16); }  // the batch's pixel in the task
             depth = (meta >> 6) & 1023;
             origin = (int)((unsigned)meta >> 16);
             if (origin == 0xFFFF) origin = -1;
@@ -468,7 +542,7 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
                   const V3<float> nd = (brdf_kind == RT_BRDF_DIFFUSE) ? normal : specular_dir<float>(ray.d, normal);
                   const V3<float> w = inv_n * mul3(thr, hit_color);
                   out.a = make_float4(point.x, point.y, point.z,
-                                      __int_as_float(slot | (brdf_kind << 5) | ((depth + 1) << 6) |
+                                      __int_as_float((ERR ? rslot : slot) | (brdf_kind << 5) | ((depth + 1) << 6) |
                                                      ((best < 0xFFFF ? best : 0xFFFF) << 16)));
                   out.b = make_float4(nd.x, nd.y, nd.z, w.x);
                   out.c = make_float4(w.y, w.z, __uint_as_float((uint32_t)rng.state), __uint_as_float((uint32_t)(rng.state >> 32)));
@@ -479,6 +553,7 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
         }
 
         // ---------------- accumulate
+        if (ERR) err_batch_add(bsum, rslot, active, contrib, lane);
         if (ACC == ACC_SEG) {
           // lanes of one record (or one pixel, for primaries) are contiguous: segmented scan
 #pragma unroll
@@ -523,7 +598,12 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
     n_rays += task_rays;
 
     // ---------------- write the pixels of this task
-    if (ACC == ACC_SEG) {
+    if (ERR && ACC == ACC_SEG) {
+      __syncwarp();
+      for (int g = 0; g < G && p0 + g < pm.n_pixels; ++g)
+        err_store(ea, L, bsum, g, p0 + g, mk3<float>(acc[3 * g] * inv_spp, acc[3 * g + 1] * inv_spp, acc[3 * g + 2] * inv_spp), lane);
+      __syncwarp();
+    } else if (ACC == ACC_SEG) {
       __syncwarp();
       const long long p = p0 + lane;
       if (lane < G && p < pm.n_pixels) {
@@ -545,7 +625,9 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
           b += __shfl_xor_sync(FULL, b, d);
         }
         const long long p = p0 + g;
-        if (lane == 0 && p < pm.n_pixels) {
+        if (ERR) {
+          if (p < pm.n_pixels) err_store(ea, L, bsum, g, p, mk3<float>(r * inv_spp, gr * inv_spp, b * inv_spp), lane);
+        } else if (lane == 0 && p < pm.n_pixels) {
           int col, row;
           pm.locate(p, col, row);
           store_pixel<float>(a, pm.at(p, col, row), mk3<float>(r * inv_spp, gr * inv_spp, b * inv_spp));
@@ -560,7 +642,13 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
         sg += __shfl_xor_sync(FULL, sg, d);
         sb_ += __shfl_xor_sync(FULL, sb_, d);
       }
-      if (lane == 0 && p0 < pm.n_pixels) {
+      if (ERR) {
+        if (p0 < pm.n_pixels) {
+          __syncwarp();  // the batch sums of the task are complete
+          err_store(ea, L, bsum, 0, p0, mk3<float>(sr * inv_spp, sg * inv_spp, sb_ * inv_spp), lane);
+        }
+        __syncwarp();
+      } else if (lane == 0 && p0 < pm.n_pixels) {
         int col, row;
         pm.locate(p0, col, row);
         store_pixel<float>(a, pm.at(p0, col, row), mk3<float>(sr * inv_spp, sg * inv_spp, sb_ * inv_spp));
@@ -573,9 +661,10 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
   if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(a.counters + CNT_SAMPLES, cfg.n_samples);
 }
 
+template <bool ERR = false>
 inline cudaError_t launch_pt_warp_impl(const SceneView<float>& sc, const RenderArgs& a, cudaStream_t st,
-                                       int sm_count, LaunchInfo* info, const char** why_not) {
-  PixelMap pm = make_pixel_map(a);
+                                       int sm_count, LaunchInfo* info, const char** why_not, ErrArgs ea = ErrArgs()) {
+  PixelMap pm = ERR ? make_pixel_map_list(a, ea) : make_pixel_map(a);
   const int S2 = a.S > 0 ? a.S * a.S : 1;
   int L = S2;
   if (a.part_mode == RT_PART_SPP && a.part_count > 1)
@@ -614,10 +703,14 @@ inline cudaError_t launch_pt_warp_impl(const SceneView<float>& sc, const RenderA
   const size_t limit = 200 * 1024;
   int warps = (small ? RT_SMALL_THREADS : RT_WARP_MAX_THREADS) / 32;
   size_t per_warp = 0, smem = 0;
+  // (the accumulator choice below sums a pixel's samples in a different order per mode, so it is made on the
+  // footprint without the batch sums: the ERR instantiation then stores the plain kernel's image bit for bit)
+  bool with_err = false;
   auto footprint = [&](int mode, int w, size_t& pw) {
     pw = (size_t)(cap + 1) * sizeof(ScatterRec);
     if (mode == ACC_SEG) pw += 32 * sizeof(int) + 96 * sizeof(float);
     if (mode == ACC_LANES) pw += 32 * sizeof(int) + (size_t)cfg.group * 96 * sizeof(float);
+    if (with_err) pw += 96 * sizeof(float);  // batch sums
     return cfg.shape_bytes + pw * w;
   };
   // The accumulator columns of ACC_LANES cost 384 B per pixel and warp; where that takes a resident
@@ -634,6 +727,7 @@ inline cudaError_t launch_pt_warp_impl(const SceneView<float>& sc, const RenderA
     if (const char* env = getenv("RT_WARP_ACC")) { const int m = atoi(env); if (m == ACC_LANES || m == ACC_SEG) acc_mode = m; }
 #endif
   }
+  with_err = ERR;
   for (;; warps >>= 1) {
     smem = footprint(acc_mode, warps, per_warp);
     if (smem <= limit || warps == 1) break;
@@ -649,10 +743,16 @@ inline cudaError_t launch_pt_warp_impl(const SceneView<float>& sc, const RenderA
   cfg.inv_w = 1.0 / (double)a.width;
   cfg.inv_h = 1.0 / (double)a.height;
   cfg.inv_s = a.S > 0 ? 1.0 / (double)a.S : 1.0;
+  ea.err_bpp = 32 / cfg.group;
+  ea.err_magic = (65536u + (unsigned)ea.err_bpp - 1u) / (unsigned)ea.err_bpp;  // x / bpp for x < 32
+  if (ERR && (a.S < 2 || cfg.group > RT_ACC_LANES_MAX_GROUP || L != S2)) {
+    *why_not = "the error map needs samples_per_side >= 2 and no partition";
+    return cudaErrorInvalidValue;
+  }
 
-  void (*kern)(const SceneView<float>, const RenderArgs, const WarpCfg);
+  void (*kern)(const SceneView<float>, const RenderArgs, const WarpCfg, const ErrArgs);
 #define RT_PICK(ACCM)                                                                   \
-  (small ? k_pt_warp<true, ACCM, true> : (shapes_smem ? k_pt_warp<true, ACCM, false> : k_pt_warp<false, ACCM, false>))
+  (small ? k_pt_warp<true, ACCM, true, ERR> : (shapes_smem ? k_pt_warp<true, ACCM, false, ERR> : k_pt_warp<false, ACCM, false, ERR>))
   if (acc_mode == ACC_REG) kern = RT_PICK(ACC_REG);
   else if (acc_mode == ACC_LANES) kern = RT_PICK(ACC_LANES);
   else kern = RT_PICK(ACC_SEG);
@@ -666,7 +766,7 @@ inline cudaError_t launch_pt_warp_impl(const SceneView<float>& sc, const RenderA
   long long blocks = (long long)per_sm * sm_count;  // persistent: every block stays resident
   long long needed = (cfg.n_tasks + warps - 1) / warps;
   if (blocks > needed) blocks = needed;
-  kern<<<(unsigned)blocks, warps * 32, smem, st>>>(sc, a, cfg);
+  kern<<<(unsigned)blocks, warps * 32, smem, st>>>(sc, a, cfg, ea);
   if (info) { info->n_launches += 1; info->variant = RT_VARIANT_WARP; }
   return cudaGetLastError();
 }

@@ -54,9 +54,11 @@ struct WarpBvhCfg {
   int n_nodes, n_prims;
 };
 
+// ERR: error-map instantiation, as k_pt_warp's (rt_warp.cuh err_batch_add)
+template <bool ERR = false>
 __global__ void __launch_bounds__(RT_WARP_MAX_THREADS, RT_BVH_MINB)
 k_pt_warp_bvh(const __grid_constant__ SceneView<float> sc, const __grid_constant__ RenderArgs a,
-              const __grid_constant__ WarpBvhCfg bcfg) {
+              const __grid_constant__ WarpBvhCfg bcfg, const __grid_constant__ ErrArgs ea) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const WarpCfg& cfg = bcfg.w;
   const unsigned FULL = 0xffffffffu;
@@ -77,11 +79,13 @@ k_pt_warp_bvh(const __grid_constant__ SceneView<float> sc, const __grid_constant
   int* slot_rays = RT_BVH_REC_GLOBAL ? reinterpret_cast<int*>(wbase) : reinterpret_cast<int*>(cur + 1);  // [32]
   float* acc = reinterpret_cast<float*>(slot_rays + 32);  // [G][3][32]
   float2* walk_stacks = reinterpret_cast<float2*>(acc + cfg.group * 96);  // [stack_entries][32]
+  float* bsum = reinterpret_cast<float*>(walk_stacks + bcfg.stack_entries * 32);  // ERR: [32][3] batch sums
   const bool count_rays = a.out_hit != nullptr && a.hit_mode == RT_HIT_RAY_COUNT;
   const float* planes = sc.invm + 12 * (size_t)sc.n_spheres;
   const int n_planes = sc.n_shapes - sc.n_spheres;
 
-  const PixelMap pm = make_pixel_map(a);
+  const PixelMap pm = ERR ? make_pixel_map_list(a, ea) : make_pixel_map(a);
+  auto locate = [&](long long p, int& col, int& row) { if (ERR) locate_listed(pm, ea, p, col, row); else pm.locate(p, col, row); };
   const int N = a.num_of_rays;
   const int S2 = a.S > 0 ? a.S * a.S : 1;
   const int G = cfg.group, L = cfg.per_pixel;
@@ -99,6 +103,7 @@ k_pt_warp_bvh(const __grid_constant__ SceneView<float> sc, const __grid_constant
     const int task_prims = (int)min((long long)G, pm.n_pixels - p0) * L;
     for (int i = 0; i < 3 * G; ++i) acc[i * 32 + lane] = 0.f;
     slot_rays[lane] = 0;
+    if (ERR) { for (int i = lane; i < 96; i += 32) bsum[i] = 0.f; }
     __syncwarp();
 
     // ---- per-lane state that lives across iterations
@@ -107,6 +112,7 @@ k_pt_warp_bvh(const __grid_constant__ SceneView<float> sc, const __grid_constant
     V3<float> thr = mk3<float>(1.f, 1.f, 1.f);
     uint64_t rng_state = 0;
     int slot = 0, depth = 0, origin = -1;
+    int rslot = 0;  // ERR: the slot field of this ray's records, the batch (`slot` stays the pixel in the task)
     long long pix = -1;  // >= 0: a primary ray whose hit goes to out_hit[pix]
     float best_t = Num<float>::inf();
     int best = -1;
@@ -126,8 +132,9 @@ k_pt_warp_bvh(const __grid_constant__ SceneView<float> sc, const __grid_constant
           const int j = prim_next + rank;
           slot = j / L;
           const int ls = j - slot * L;
+          if (ERR) rslot = slot * ea.err_bpp + err_batch_of(ea, ls);
           int col, row;
-          pm.locate(p0 + slot, col, row);
+          locate(p0 + slot, col, row);
           const long long px = (long long)row * a.width + col;
           const int s = own_stratum(a, ls);
           const unsigned long long k = (unsigned long long)px * S2 + s;
@@ -180,6 +187,7 @@ k_pt_warp_bvh(const __grid_constant__ SceneView<float> sc, const __grid_constant
         if (get) {
           const int meta = __float_as_int(rec.a.w);
           slot = meta & 31;
+          if (ERR) { rslot = slot; slot = (int)(((unsigned)rslot * ea.err_magic) >> 16); }  // the batch's pixel in the task
           depth = (meta >> 6) & 1023;
           origin = (int)((unsigned)meta >> 16);
           if (origin == 0xFFFF) origin = -1;
@@ -283,7 +291,7 @@ k_pt_warp_bvh(const __grid_constant__ SceneView<float> sc, const __grid_constant
                 const V3<float> nd = (mat.brdf_kind == RT_BRDF_DIFFUSE) ? normal : specular_dir<float>(ray.d, normal);
                 const V3<float> w = inv_n * mul3(thr, hit_color);
                 out.a = make_float4(point.x, point.y, point.z,
-                                    __int_as_float(slot | (mat.brdf_kind << 5) | ((depth + 1) << 6) |
+                                    __int_as_float((ERR ? rslot : slot) | (mat.brdf_kind << 5) | ((depth + 1) << 6) |
                                                    ((best < 0xFFFF ? best : 0xFFFF) << 16)));
                 out.b = make_float4(nd.x, nd.y, nd.z, w.x);
                 out.c = make_float4(w.y, w.z, __uint_as_float((uint32_t)rng.state), __uint_as_float((uint32_t)(rng.state >> 32)));
@@ -295,6 +303,7 @@ k_pt_warp_bvh(const __grid_constant__ SceneView<float> sc, const __grid_constant
         colm[0] += contrib.x; colm[32] += contrib.y; colm[64] += contrib.z;
         busy = false;
       }
+      if (ERR) err_batch_add(bsum, rslot, done, contrib, lane);
       // ---------------- push the new records: one ballot gives every lane its slot
       const unsigned pmask = __ballot_sync(FULL, push);
       const int npush = __popc(pmask);
@@ -318,7 +327,9 @@ k_pt_warp_bvh(const __grid_constant__ SceneView<float> sc, const __grid_constant
         b += __shfl_xor_sync(FULL, b, d);
       }
       const long long p = p0 + g;
-      if (lane == 0 && p < pm.n_pixels) {
+      if (ERR) {
+        if (p < pm.n_pixels) err_store(ea, L, bsum, g, p, mk3<float>(r * inv_spp, gr * inv_spp, b * inv_spp), lane);
+      } else if (lane == 0 && p < pm.n_pixels) {
         int col, row;
         pm.locate(p, col, row);
         store_pixel<float>(a, pm.at(p, col, row), mk3<float>(r * inv_spp, gr * inv_spp, b * inv_spp));
@@ -332,9 +343,11 @@ k_pt_warp_bvh(const __grid_constant__ SceneView<float> sc, const __grid_constant
   if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(a.counters + CNT_SAMPLES, cfg.n_samples);
 }
 
+template <bool ERR = false>
 inline cudaError_t launch_pt_warp_bvh(const SceneView<float>& sc, const RenderArgs& a, cudaStream_t st,
-                                      int sm_count, LaunchInfo* info, const char** why_not, int n_nodes, int n_prims, int tree_depth) {
-  PixelMap pm = make_pixel_map(a);
+                                      int sm_count, LaunchInfo* info, const char** why_not, int n_nodes, int n_prims, int tree_depth,
+                                      ErrArgs ea = ErrArgs()) {
+  PixelMap pm = ERR ? make_pixel_map_list(a, ea) : make_pixel_map(a);
   const int S2 = a.S > 0 ? a.S * a.S : 1;
   int L = S2;
   if (a.part_mode == RT_PART_SPP && a.part_count > 1)
@@ -369,7 +382,7 @@ inline cudaError_t launch_pt_warp_bvh(const SceneView<float>& sc, const RenderAr
   size_t per_warp = 0, smem = 0;
   for (;; warps >>= 1) {
     per_warp = (RT_BVH_REC_GLOBAL ? 0 : (size_t)(cap + 1) * sizeof(ScatterRec)) + 32 * sizeof(int) + (size_t)group * 96 * sizeof(float) +
-               (size_t)b.stack_entries * 32 * sizeof(float2);
+               (size_t)b.stack_entries * 32 * sizeof(float2) + (ERR ? 96 * sizeof(float) : 0);
     b.tree_bytes = ((tree_bytes + per_warp * warps + 1024) * RT_BVH_MINB <= 227 * 1024) ? (int)tree_bytes : 0;
     smem = b.tree_bytes + per_warp * warps;
     if (smem <= limit || warps == 1) break;
@@ -386,6 +399,9 @@ inline cudaError_t launch_pt_warp_bvh(const SceneView<float>& sc, const RenderAr
   cfg.inv_w = 1.0 / (double)a.width;
   cfg.inv_h = 1.0 / (double)a.height;
   cfg.inv_s = a.S > 0 ? 1.0 / (double)a.S : 1.0;
+  ea.err_bpp = 32 / cfg.group;
+  ea.err_magic = (65536u + (unsigned)ea.err_bpp - 1u) / (unsigned)ea.err_bpp;
+  if (ERR && (a.S < 2 || L != S2)) { *why_not = "the error map needs samples_per_side >= 2 and no partition"; return cudaErrorInvalidValue; }
   b.refill_at = 12;  // measured with 24 warps per SM (profiles/r2_bvh_sweep2.log): 8 | 12 | 16 | 20 | 24 -> 6.14 | 6.17 | 6.12 | 5.98 | 5.87 Grays/s
 #ifdef RT_TUNING
   if (const char* env = getenv("RT_BVH_REFILL_AT")) b.refill_at = atoi(env);
@@ -399,10 +415,10 @@ inline cudaError_t launch_pt_warp_bvh(const SceneView<float>& sc, const RenderAr
   if (b.inner_min < 0) b.inner_min = 0;
   if (b.inner_min > 31) b.inner_min = 31;
 
-  cudaError_t e = cudaFuncSetAttribute(k_pt_warp_bvh, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit);
+  cudaError_t e = cudaFuncSetAttribute(k_pt_warp_bvh<ERR>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)limit);
   if (e != cudaSuccess) return e;
   int per_sm = 0;
-  e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_pt_warp_bvh, warps * 32, smem);
+  e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_pt_warp_bvh<ERR>, warps * 32, smem);
   if (e != cudaSuccess) return e;
   if (per_sm < 1) per_sm = 1;
   long long blocks = (long long)per_sm * sm_count;  // persistent: every block stays resident
@@ -425,7 +441,7 @@ inline cudaError_t launch_pt_warp_bvh(const SceneView<float>& sc, const RenderAr
     }
     b.rec_pool = pool[dev];
   }
-  k_pt_warp_bvh<<<(unsigned)blocks, warps * 32, smem, st>>>(sc, a, b);
+  k_pt_warp_bvh<ERR><<<(unsigned)blocks, warps * 32, smem, st>>>(sc, a, b, ea);
   if (info) { info->n_launches += 1; info->variant = RT_VARIANT_WARP; }
   return cudaGetLastError();
 }

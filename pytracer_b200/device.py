@@ -79,6 +79,23 @@ class DeviceScene:
             params.replay_states = None
         return out, hit, stats.as_dict()
 
+    def render_adaptive(self, params: _abi.rt_render_params, target_error: float = 0.0, max_passes: int = 1,
+                        error_floor: float = 1e-2, out: Optional[np.ndarray] = None):
+        """rt_render_adaptive: (mean image, SE image, samples per pixel, stats) as float32 [H][W][3] x 2 and
+        int32 [H][W]; ``max_passes`` passes of ``params.samples_per_side ** 2`` samples at most per pixel."""
+        H, W = params.height, params.width
+        if out is None:
+            out = np.empty((H, W, 3), dtype=np.float32)
+        assert out.dtype == np.float32 and out.shape == (H, W, 3) and out.flags.c_contiguous
+        err = np.empty((H, W, 3), dtype=np.float32)
+        samples = np.empty((H, W), dtype=np.int32)
+        ap = _abi.rt_adaptive_params()
+        ap.target_error, ap.error_floor, ap.max_passes = float(target_error), float(error_floor), int(max_passes)
+        stats = _abi.rt_adaptive_stats()
+        _native.check(self._lib.rt_render_adaptive(self._handle, C.byref(params), C.byref(ap), _ptr(out), _ptr(err), _ptr(samples),
+                                                   C.byref(stats)))
+        return out, err, samples, stats.as_dict()
+
     def render_device(self, params: _abi.rt_render_params, out_ptr: int, hit_ptr: int = 0, stream: int = 0) -> None:
         """rt_render_device: enqueue on ``stream`` writing to device memory at ``out_ptr``."""
         _native.check(self._lib.rt_render_device(self._handle, C.byref(params), C.c_void_p(out_ptr),

@@ -17,6 +17,7 @@ copies them into one page-locked host image shared by the ranks of the node, whi
 """
 from __future__ import annotations
 
+from dataclasses import dataclass, field
 from typing import Optional
 
 import numpy as np
@@ -27,6 +28,16 @@ from .params import make_params
 from .pcg import PCG
 from .render import CudaRenderer
 from .scene import Color, Point, Ray, Vec
+
+
+@dataclass
+class AdaptiveResult:
+    """What ``fire_all_rays_adaptive`` returns besides the image: the standard error of every pixel's mean
+    (float32 [H][W][3]), the samples every pixel received (int32 [H][W]), the passes run and the call's counters."""
+    error: np.ndarray
+    samples: np.ndarray
+    passes: int
+    stats: dict = field(default_factory=dict)
 
 
 class ImageTracer:
@@ -62,6 +73,52 @@ class ImageTracer:
         self.pcg.advance(self._draws_per_image())
         if callback:
             callback(col=self.image.width - 1, row=self.image.height - 1, **callback_kwargs)
+
+    def fire_all_rays_adaptive(self, renderer, target_error: float = 0.0, max_samples_per_pixel: Optional[int] = None,
+                               error_floor: float = 1e-2, callback=None, callback_time_s: float = 2.0, **callback_kwargs) -> AdaptiveResult:
+        """Path-traced image with a per-pixel Monte Carlo error map, optionally refined where it is noisy.
+
+        Pass 0 is exactly ``fire_all_rays(renderer)``; every further pass traces ``samples_per_side ** 2`` more
+        samples, for the pixels whose relative error max_c SE_c / max(mean_c, error_floor) is still above
+        ``target_error``, until they meet it or hold ``max_samples_per_pixel`` samples (default: one pass, the
+        error map only).  Pass p of a pixel is that pixel of the (p+1)-th consecutive ``fire_all_rays``; a pixel
+        with P passes holds the mean of its P pass values.  ``self.image`` receives the mean image, and
+        ``self.pcg`` and ``renderer.pcg`` are left where ``passes`` consecutive ``fire_all_rays`` leave them."""
+        spp = self.samples_per_side ** 2
+        if not isinstance(renderer, CudaRenderer) or renderer.algorithm != "pathtracing":
+            raise ValueError("fire_all_rays_adaptive needs a path-tracing CudaRenderer")
+        if self.samples_per_side < 2:
+            raise ValueError(f"the error map needs samples_per_side >= 2 (got {self.samples_per_side})")
+        if not (isinstance(renderer.gpus, int) and renderer.gpus == 1):
+            raise ValueError("adaptive rendering runs on one device (gpus=1)")
+        if renderer.variant == "mega" or renderer.precision in ("f64", "hybrid"):
+            raise ValueError("adaptive rendering uses the fp32 warp path tracer (variant auto/warp, precision auto/f32)")
+        if not np.isfinite(target_error) or target_error < 0:
+            raise ValueError(f"target_error must be finite and >= 0 (got {target_error})")
+        if not (np.isfinite(error_floor) and error_floor > 0):
+            raise ValueError(f"error_floor must be > 0 (got {error_floor})")
+        if max_samples_per_pixel is None:
+            max_samples_per_pixel = spp
+        if int(max_samples_per_pixel) != max_samples_per_pixel or max_samples_per_pixel < spp or max_samples_per_pixel % spp:
+            raise ValueError(f"max_samples_per_pixel ({max_samples_per_pixel}) must be a positive multiple of the "
+                             f"samples per pass ({spp})")
+        max_passes = int(max_samples_per_pixel) // spp
+        if max_passes >= 2 ** 31:
+            raise ValueError(f"max_samples_per_pixel ({max_samples_per_pixel}) is too large")
+        if callback:
+            callback(col=0, row=0, **callback_kwargs)
+        scene = renderer.device_scene()
+        rgb, err, samples, stats = scene.render_adaptive(self._params(renderer), target_error, max_passes, error_floor,
+                                                         out=self._adoptable_buffer())
+        passes = stats["passes"]
+        self.last_stats = renderer.last_stats = stats
+        for _ in range(passes):  # where `passes` consecutive fire_all_rays leave both generators
+            renderer.pcg.random()
+        self.pcg.advance(passes * self._draws_per_image())
+        install_array(self.image, rgb)
+        if callback:
+            callback(col=self.image.width - 1, row=self.image.height - 1, **callback_kwargs)
+        return AdaptiveResult(error=err, samples=samples, passes=passes, stats=stats)
 
     # -- the product path
     def _fire_cuda(self, renderer: CudaRenderer, comm=None) -> None:

@@ -59,6 +59,29 @@ def load_scene(path: str, variables, parser: str):
             sys.exit(1)
 
 
+def adaptive_cli_problem(algorithm, samples_per_pixel, gpus, variant, precision, target_error, max_samples_per_pixel,
+                         error_floor):
+    """Why `render --error-output / --target-error / --max-samples-per-pixel` cannot run as asked (None: it can)."""
+    if algorithm != "pathtracing":
+        return "--error-output, --target-error and --max-samples-per-pixel need --algorithm pathtracing"
+    if samples_per_pixel < 4:
+        return f"the error map needs at least 4 samples per pixel per pass (got {samples_per_pixel})"
+    if gpus != 1:
+        return "adaptive rendering runs on one GPU (--gpus 1)"
+    if variant == "mega" or precision == "f64":
+        return "adaptive rendering uses the fp32 warp path tracer (--variant auto|warp, --precision auto|f32)"
+    if target_error is not None and (not target_error >= 0 or target_error == float("inf")):
+        return f"--target-error must be a finite number >= 0 (got {target_error})"
+    if not error_floor > 0:
+        return f"--error-floor must be > 0 (got {error_floor})"
+    if (target_error is not None and target_error > 0) != (max_samples_per_pixel is not None):
+        return "--target-error and --max-samples-per-pixel go together"
+    if max_samples_per_pixel is not None and (max_samples_per_pixel < samples_per_pixel or max_samples_per_pixel % samples_per_pixel):
+        return (f"--max-samples-per-pixel ({max_samples_per_pixel}) must be a positive multiple of "
+                f"--samples-per-pixel ({samples_per_pixel})")
+    return None
+
+
 @click.group()
 def cli():
     pass
@@ -83,9 +106,15 @@ def cli():
 @click.option("--gpus", type=int, default=1, help="GPUs of this node to render on: interleaved rows, one rt_render_multi call from this process")
 @click.option("--launcher", type=click.Choice(["inprocess", "torchrun"]), default="inprocess",
               help="with --gpus N: drive the N devices from this process (default) or re-launch under torchrun, one process per GPU")
+@click.option("--error-output", type=str, default=None, help="PFM file to receive the standard error of every pixel (path tracing)")
+@click.option("--target-error", type=float, default=None,
+              help="render adaptively: trace more passes of --samples-per-pixel samples where the relative error is above this")
+@click.option("--max-samples-per-pixel", type=int, default=None, help="with --target-error: samples per pixel at most")
+@click.option("--error-floor", type=float, default=1e-2, help="radiance below which the relative error is taken against this floor")
 @click.argument("input_scene_name", type=str)
 def render(width, height, algorithm, pfm_output, png_output, num_of_rays, max_depth, init_state, init_seq,
-           samples_per_pixel, declare_float, variant, precision, parser, accel, gpus, launcher, input_scene_name):
+           samples_per_pixel, declare_float, variant, precision, parser, accel, gpus, launcher, error_output, target_error,
+           max_samples_per_pixel, error_floor, input_scene_name):
     import os
 
     if gpus > 1 and launcher == "torchrun" and "WORLD_SIZE" not in os.environ:  # one process per GPU: hand the same command line to torchrun
@@ -102,6 +131,13 @@ def render(width, height, algorithm, pfm_output, png_output, num_of_rays, max_de
     if samples_per_side ** 2 != samples_per_pixel:
         print(f"Error, the number of samples per pixel ({samples_per_pixel}) must be a perfect square")
         return
+    adaptive = error_output is not None or target_error is not None or max_samples_per_pixel is not None
+    if adaptive:
+        problem = adaptive_cli_problem(algorithm, samples_per_pixel, gpus, variant, precision, target_error,
+                                       max_samples_per_pixel, error_floor)
+        if problem:
+            print(f"Error, {problem}")
+            sys.exit(1)
     scene = load_scene(input_scene_name, build_variable_table(declare_float), parser)
     image = HdrImage(width, height)
     print(f"Generating a {width}×{height} image")
@@ -129,17 +165,34 @@ def render(width, height, algorithm, pfm_output, png_output, num_of_rays, max_de
 
         comm = TorchComm.from_env()
     start = perf_counter()
-    tracer.fire_all_rays(renderer, comm=comm)
+    result = None
+    if adaptive:
+        result = tracer.fire_all_rays_adaptive(renderer, target_error=target_error or 0.0,
+                                               max_samples_per_pixel=max_samples_per_pixel, error_floor=error_floor)
+    else:
+        tracer.fire_all_rays(renderer, comm=comm)
     elapsed = perf_counter() - start
     st = tracer.last_stats
     rays = st.get("rays_closest", 0) + st.get("rays_shadow", 0)
     print(f"Rendering completed in {elapsed:.3f} s ({rays} rays, {rays / max(elapsed, 1e-9) / 1e6:.1f} Mrays/s, "
           f"kernel {st.get('kernel_ms', 0.0):.2f} ms)")
+    if result is not None:
+        print(f"{result.passes} pass(es) of {samples_per_pixel} samples; pixels per pass: "
+              f"{', '.join(str(n) for n in st['pixels_in_pass'])}; {st['samples']} samples in all "
+              f"({st['samples'] / (width * height):.1f} per pixel)")
     if comm is not None and comm.rank != 0:
         return
     with open(pfm_output, "wb") as outf:
         image.write_pfm(outf)
     print(f"HDR demo image written to {pfm_output}")
+    if result is not None and error_output is not None:
+        from .hdrimage import install_array
+
+        err_image = HdrImage(width, height)
+        install_array(err_image, result.error)
+        with open(error_output, "wb") as outf:
+            err_image.write_pfm(outf)
+        print(f"Standard error of every pixel written to {error_output}")
     try:
         from .tonemap import write_ldr_image
 
