@@ -52,6 +52,19 @@ for variant in ("auto", "warp", "mega"):
 rgb, _, st = sc.render(make_params(16, 9, cam, algorithm="pathtracing", samples_per_side=1, num_of_rays=1, max_depth=2000, rr_limit=2))
 assert st["variant_used"] == _abi.RT_VARIANT_MEGA and np.isfinite(rgb).all()
 
+# error-map instantiations (rt_render_adaptive) at frames of one task, a partial last task and one row: one
+# pass over the image, and three passes of which the later ones trace pixel lists
+for scene, camera, accels in ((sc, cam, ("none",)), (big, rs.camera, ("none", "bvh"))):
+    for accel in accels:
+        for w, h in ((1, 1), (7, 3), (33, 1)):
+            for spp in (2, 3):
+                for passes in (1, 3):
+                    p = make_params(w, h, camera, algorithm="pathtracing", samples_per_side=spp, num_of_rays=3, max_depth=3,
+                                    accel=accel, aa_pcg=PCG(42, 54), pt_pcg=PCG(45, 54))
+                    mean, err, samples, st = scene.render_adaptive(p, 1e-6 if passes > 1 else 0.0, passes)
+                    assert np.isfinite(mean).all() and np.isfinite(err).all() and (err >= 0).all() and st["overflow"] == 0
+                    assert st["passes"] <= passes and ((samples >= spp * spp) & (samples <= passes * spp * spp)).all()
+
 img = np.random.default_rng(1).random((37, 53, 3), dtype=np.float32) * 4
 tonemap.average_luminosity(img)
 tonemap.tone_map(img, 0.7, None, 1.0)

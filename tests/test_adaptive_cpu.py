@@ -1,12 +1,14 @@
 """Adaptive path tracing without a device: the C-ABI structs of rt_render_adaptive against gcc's layout, the
-argument checks of CudaImageTracer.fire_all_rays_adaptive (ValueError before any device call) and the
-`render` command refusing option combinations it cannot run."""
+argument checks of CudaImageTracer.fire_all_rays_adaptive (ValueError before any device call), the
+`render` command refusing option combinations it cannot run, and the host references the GPU error-map tests
+compare with (tests/util.py batch_se2 and replay_adaptive)."""
 import ctypes
 import os
 import subprocess
 import tempfile
 import textwrap
 
+import numpy as np
 import pytest
 from click.testing import CliRunner
 
@@ -16,6 +18,7 @@ from pytracer_b200.imagetracer import CudaImageTracer
 from pytracer_b200.main import cli
 from pytracer_b200.pcg import PCG
 from pytracer_b200.render import FlatRenderer, PathTracer
+from util import batch_se2, replay_adaptive, same_partition
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -102,3 +105,53 @@ def test_render_command_refuses_adaptive_combinations_it_cannot_run(tmp_path, ar
     assert result.exit_code != 0, result.output
     assert "Error," in result.output and message in result.output, result.output
     assert not (tmp_path / "o.pfm").exists()
+
+
+def test_batch_se2_is_the_documented_estimator():
+    rng = np.random.default_rng(3)
+    # one-sample batches (bpp >= L): the sample variance over L
+    for L, bpp in ((4, 4), (9, 10), (16, 32), (25, 32)):
+        x = rng.normal(2.0, 0.5, size=(7, 3, L))
+        assert np.allclose(batch_se2(x, bpp), x.var(-1, ddof=1) / L, rtol=1e-12, atol=0), (L, bpp)
+    # a layout given as labels equals the same layout given as bpp; the rounding bound is positive
+    x = rng.normal(size=(5, 36))
+    se2, bound = batch_se2(x, 32, bound=True)
+    assert np.array_equal(se2, batch_se2(x, np.arange(36) % 32)) and (bound > 0).all()
+    # unbiased for independent samples also where the batch sizes differ (n_b in {2, 1})
+    for L, bpp in ((9, 8), (36, 32)):
+        x = rng.normal(0.0, 1.5, size=(100_000, L))
+        ratio = batch_se2(x, bpp).mean() / (1.5 ** 2 / L)
+        print(f"L = {L}, bpp = {bpp}: mean SE^2 / (sigma^2 / L) = {ratio:.4f}")
+        assert abs(ratio - 1.0) <= 0.01, (L, bpp, ratio)
+    assert same_partition(np.arange(9) % 10, np.arange(9)) and not same_partition(np.arange(9) % 8, np.arange(9))
+    assert same_partition([3, 3, 1, 1], [0, 0, 2, 2]) and not same_partition([0, 0, 1, 1], [0, 1, 0, 1])
+
+
+def test_replay_adaptive_on_a_hand_made_example():
+    """Three pixels, target 0.12, floor 0.01, three passes: pixel 0 is dark and stops after pass 0 because of the
+    floor (without it e would be 1); pixel 1 misses the target after pass 0 and meets it after pass 1; pixel 2
+    never does and stops at the pass limit.  NaN marks inputs of passes a pixel is not listed in."""
+    nan = np.nan
+    means = np.array([[[0.001] * 3, [0.5] * 3, [0.2] * 3],
+                      [[nan] * 3, [0.7] * 3, [0.2] * 3],
+                      [[nan] * 3, [nan] * 3, [0.2] * 3]], dtype=np.float32)[:, None]
+    errs = np.array([[[0.001] * 3, [0.1, 0.0, 0.1], [0.2] * 3],
+                     [[nan] * 3, [0.05, 0.0, 0.05], [0.2] * 3],
+                     [[nan] * 3, [nan] * 3, [0.2] * 3]], dtype=np.float32)[:, None]
+    r = replay_adaptive(means, errs, 0.12, 0.01, 3)
+    assert r["passes"].tolist() == [[1, 2, 3]] and r["pixels_in_pass"] == [3, 2, 1] and not r["ambiguous"].any()
+    f = np.float32
+    assert np.array_equal(r["mean"][0, :, 0], [f(0.001), (f(0.5) + f(0.7)) / f(2), ((f(0.2) + f(0.2)) + f(0.2)) / f(3)])
+    e1 = np.sqrt(f(0.1) ** 2.0 + f(0.05) ** 2.0) / 2
+    assert np.allclose(r["err"][0, :, 0], [f(0.001), e1, np.sqrt(3 * f(0.2) ** 2.0) / 3], rtol=1e-12)
+    assert r["err"][0, 1, 1] == 0.0
+    # without the floor the dark pixel misses the target in every pass
+    dark_m, dark_e = means.copy(), errs.copy()
+    dark_m[:, 0, 0], dark_e[:, 0, 0] = 0.001, 0.001
+    r = replay_adaptive(dark_m, dark_e, 0.12, 1e-6, 3)
+    assert r["passes"].tolist() == [[3, 2, 3]] and r["pixels_in_pass"] == [3, 3, 2]
+    # one pass, or a target no pixel misses: nothing is listed again
+    assert replay_adaptive(means, errs, 0.12, 0.01, 1)["pixels_in_pass"] == [3]
+    assert replay_adaptive(means, errs, float("inf"), 1e3, 3)["passes"].tolist() == [[1, 1, 1]]
+    # a value at the target is ambiguous
+    assert replay_adaptive(means, errs, 1.0, 1e-6, 3)["ambiguous"].tolist() == [[True, False, True]]

@@ -47,6 +47,84 @@ def c1_params(cam, **kw):
     return make_params(160, 120, cam, **args)
 
 
+def batch_se2(x, bpp, bound=False):
+    """SE^2 of the pass mean from batch sums, in fp64, as DESIGN.md §5.5 documents it (rt_warp.cuh err_store).
+
+    `x`: per-sample values [..., L], the last axis in sample order.  `bpp`: an int (sample s goes to batch
+    s mod bpp, the kernel's layout with bpp = 32 / G), or an int array of L batch labels (any other layout).
+    With T_b, n_b the sum and size of batch b, B the number of batches and m the mean of the L samples:
+        SE^2 = sum_b (T_b - n_b m)^2 / (n_b (B - 1) L)
+    With `bound=True` also returns how far an fp32 kernel's value may lie from it: every T_b and m off by at
+    most delta_b = 1e-5 (sum_{s in b} |x_s| + n_b |m|) (sums of non-negative contributions), which moves
+    (T_b - n_b m)^2 by at most 2 |T_b - n_b m| delta_b + delta_b^2; plus 4 ulp of the result for the final
+    products and the square root of the stored SE."""
+    x = np.asarray(x, dtype=np.float64)
+    L = x.shape[-1]
+    labels = np.arange(L) % bpp if np.isscalar(bpp) else np.asarray(bpp)
+    _, b = np.unique(labels, return_inverse=True)
+    onehot = np.zeros((L, int(b.max()) + 1))
+    onehot[np.arange(L), b] = 1.0
+    n = onehot.sum(0)
+    B = onehot.shape[1]
+    assert B >= 2, "one batch has no spread"
+    m = x.mean(-1, keepdims=True)
+    d = x @ onehot - n * m
+    k = 1.0 / ((B - 1) * L)
+    se2 = (d * d / n).sum(-1) * k
+    if not bound:
+        return se2
+    delta = 1e-5 * (np.abs(x) @ onehot + n * np.abs(m))
+    return se2, ((2.0 * np.abs(d) * delta + delta * delta) / n).sum(-1) * k + 4.0 * 2.0 ** -23 * se2
+
+
+def same_partition(a, b) -> bool:
+    """Whether two label arrays group the same samples together (whatever the labels are called)."""
+    def canonical(v):  # labels renamed 0, 1, ... in order of first appearance
+        _, first, inverse = np.unique(np.asarray(v), return_index=True, return_inverse=True)
+        return np.argsort(np.argsort(first))[inverse]
+
+    return np.array_equal(canonical(a), canonical(b))
+
+
+def replay_adaptive(per_pass_means, per_pass_errs, target, floor, max_passes, band=1e-5):
+    """Host replica of rt_render_adaptive's passes (rt_adaptive.cu) from what every pass would give each pixel.
+
+    `per_pass_means` / `per_pass_errs`: [K][H][W][3] float32, the mean and SE of pass p for every pixel (K >=
+    the passes that run).  Per pixel, over the passes it is listed in: sum_m += m_p in fp32 (numpy's float32
+    add rounds like __fadd_rn), sum_v += err_p^2 in fp64 (the kernel adds SE_p^2 in fp32; only err_p = sqrt(SE_p^2)
+    is observable, so sum_v is approximate), P += 1; the pixel is listed again when passes remain and
+        e = max_c (sqrt(sum_v) / P) / max(sum_m / P, floor) > float32(target).
+    Returns mean = sum_m / P (float32, exact), err = sqrt(sum_v) / P, `passes` (P per pixel), `pixels_in_pass`
+    and `ambiguous`: pixels whose e came within a relative `band` of the target in some pass, where the
+    approximate sum_v cannot tell which way the kernel decided."""
+    m = np.asarray(per_pass_means, dtype=np.float32)
+    v = np.asarray(per_pass_errs, dtype=np.float64) ** 2
+    t = float(np.float32(target))
+    fl = np.float32(floor)
+    sum_m, sum_v = m[0].copy(), v[0].copy()
+    P = np.ones(m.shape[1:3], dtype=np.int32)
+    listed = np.ones(m.shape[1:3], dtype=bool)
+    ambiguous = np.zeros_like(listed)
+    pixels_in_pass = [int(listed.sum())]
+    for p in range(max_passes):
+        if p > 0:
+            sum_m[listed] = sum_m[listed] + m[p][listed]
+            sum_v[listed] += v[p][listed]
+            P[listed] += 1
+        if p + 1 >= max_passes:
+            break
+        Pf = P[..., None].astype(np.float64)
+        e = (np.sqrt(sum_v) / Pf / np.maximum(sum_m / P[..., None].astype(np.float32), fl)).max(-1)
+        if np.isfinite(t):
+            ambiguous |= listed & (np.abs(e / t - 1.0) < band)
+        listed = listed & (e > t)
+        if not listed.any():
+            break
+        pixels_in_pass.append(int(listed.sum()))
+    return dict(mean=sum_m / P[..., None].astype(np.float32), err=np.sqrt(sum_v) / P[..., None], passes=P,
+                pixels_in_pass=pixels_in_pass, ambiguous=ambiguous)
+
+
 def luminosity(rgb):
     """Color.luminosity, colors.py:59-61, per pixel."""
     return (rgb.max(axis=-1) + rgb.min(axis=-1)) / 2
