@@ -115,6 +115,8 @@ RT_DEV void err_store(const ErrArgs& e, int L, const float* bsum, int g, long lo
 //   SM_SHAPE_MAT     [16] the shape's material as one int4 {brdf_kind, brdf_pigment, emitted_pigment, flags}
 //                    (no material-index indirection)
 //   SM_PIG           [32] 48-byte pigment records {kind, steps, tex_w, tex_h | c1.xyz, c2.x | c2.yz, texture handle}
+//   SM_JUMP          [32] {mult, plus} of the jitter jump by 2 c k draws (c the partition stride), one-pixel tasks
+//                    (ACC_REG) only: the block is SM_JUMP_BYTES longer there
 #define RT_SMALL_MAX_SPHERES 8
 #define RT_SMALL_MAX_SHAPES 16
 #define RT_SMALL_MAX_MATERIALS 16
@@ -126,7 +128,9 @@ enum {
   SM_SHAPE_MAT = SM_ORIG + RT_SMALL_MAX_SHAPES * 4,
   SM_PIG = SM_SHAPE_MAT + RT_SMALL_MAX_SHAPES * 16,
   SM_PIG_STRIDE = 48,
-  SM_BYTES = SM_PIG + RT_SMALL_MAX_PIGMENTS * SM_PIG_STRIDE
+  SM_BYTES = SM_PIG + RT_SMALL_MAX_PIGMENTS * SM_PIG_STRIDE,
+  SM_JUMP = SM_BYTES,
+  SM_JUMP_BYTES = 32 * 16
 };
 #ifndef RT_SMALL_THREADS
 #define RT_SMALL_THREADS 256
@@ -173,6 +177,11 @@ RT_DEV int ldsic(uint32_t a) {
   asm volatile("ld.shared.s32 %0, [%1];" : "=r"(v) : "r"(a));
   return v;
 }
+RT_DEV ulonglong2 lds2u64c(uint32_t a) {
+  ulonglong2 v;
+  asm volatile("ld.shared.v2.u64 {%0, %1}, [%2];" : "=l"(v.x), "=l"(v.y) : "r"(a));
+  return v;
+}
 RT_DEV Rows3 lds_rows(uint32_t a) {
   Rows3 m;
   m.r0 = lds4c(a); m.r1 = lds4c(a + 16); m.r2 = lds4c(a + 32);
@@ -185,28 +194,37 @@ RT_DEV Rows3 lds_rows(uint32_t a) {
 // unbounded (tmax = inf, ray.py:31), so only tmin is tested.  Spheres and planes keep separate minima
 // (strict '<': the first of each kind wins a tie like world.py:62) and the rare sphere-vs-plane tie is
 // resolved once at the end on the index in World.shapes.
+// Both walks are unrolled to the SMALL capacity with one warp-uniform exit per shape (the counts are kernel
+// parameters, read from the constant bank): no loop counter, and every table offset is an immediate off `sb`
+// (spheres) or off the first plane's address (planes).  A runtime-bounded loop cost ~15 instructions of
+// header per shape, as much as a plane test.
 RT_DEV void closest_small(uint32_t sb, int n_spheres, int n_shapes, const Ray<float>& r, int origin, float& best_t, int& best) {
   const float inf = Num<float>::inf();
   float ts = inf, tp = inf;
   int is = -1, ip = -1;
-  uint32_t a = sb + SM_INVM;
-#pragma unroll 1
-  for (int i = 0; i < n_spheres; ++i, a += 48) {
+#pragma unroll
+  for (int i = 0; i < RT_SMALL_MAX_SPHERES; ++i) {
+    if (i >= n_spheres) break;
     float tm, half;
-    bool ok = sphere_cross_rows(lds_rows(a), r, tm, half);
+    bool ok = sphere_cross_rows(lds_rows(sb + SM_INVM + 48 * i), r, tm, half);
     const float t1 = tm - half;
     float t = (t1 > r.tmin) ? t1 : tm + half;   // the first root beyond tmin, shapes.py:112-119
     if (i == origin) { t = 2.0f * tm; ok = true; }  // see sphere_t_at
     if (ok && t > r.tmin && t < ts) { ts = t; is = i; }
   }
-#pragma unroll 1
-  for (int i = n_spheres; i < n_shapes; ++i, a += 48) {
-    const float4 row = lds4c(a + 32);
+  // plane k is shape n_spheres + k
+  const uint32_t pb = sb + SM_INVM + 48 * (uint32_t)n_spheres;
+  const int n_planes = n_shapes - n_spheres, porigin = origin - n_spheres;
+#pragma unroll
+  for (int k = 0; k < RT_SMALL_MAX_SHAPES; ++k) {
+    if (k >= n_planes) break;
+    const float4 row = lds4c(pb + 48 * k + 32);
     const float oz = fmaf(r.o.x, row.x, fmaf(r.o.y, row.y, fmaf(r.o.z, row.z, row.w)));
     const float dz = fmaf(r.d.x, row.x, fmaf(r.d.y, row.y, r.d.z * row.z));
     const float t = -oz * fast_rcp(dz);
-    if (!(fabsf(dz) < 1e-5f) && t > r.tmin && t < tp && i != origin) { tp = t; ip = i; }
+    if (!(fabsf(dz) < 1e-5f) && t > r.tmin && t < tp && k != porigin) { tp = t; ip = k; }
   }
+  if (ip >= 0) ip += n_spheres;
   bool plane = tp < ts;
   if (tp == ts && ip >= 0 && is >= 0) plane = ldsic(sb + SM_ORIG + 4 * ip) < ldsic(sb + SM_ORIG + 4 * is);
   best_t = plane ? tp : ts;
@@ -301,6 +319,17 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
       o[1] = make_float4(pg.c1[0], pg.c1[1], pg.c1[2], pg.c2[0]);
       o[2] = make_float4(pg.c2[1], pg.c2[2], __uint_as_float((uint32_t)pg.tex), __uint_as_float((uint32_t)((unsigned long long)pg.tex >> 32)));
     }
+    if (ACC == ACC_REG && threadIdx.x < 32) {  // x -> mult x + plus = LCG^(2 c k), composed from a.jump
+      const unsigned long long c = (a.part_mode == RT_PART_SPP && a.part_count > 1) ? (unsigned long long)a.part_count : 1ull;
+      uint64_t d = 2ull * c * threadIdx.x, mult = 1, plus = 0;
+      while (d != 0) {
+        const int b = __ffsll((long long)d) - 1;
+        mult = a.jump.mult[b] * mult;
+        plus = a.jump.mult[b] * plus + a.jump.plus[b];
+        d &= d - 1;
+      }
+      reinterpret_cast<ulonglong2*>(smem_raw + SM_JUMP)[threadIdx.x] = make_ulonglong2(mult, plus);
+    }
     __syncthreads();
   } else if (SHAPES_SMEM) {
     stage_bytes(smem_raw, sc.packed, (size_t)sc.n_pairs * 96 + (size_t)(sc.n_shapes - sc.n_spheres) * 48);
@@ -315,7 +344,7 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
   const uint32_t smem0 = (uint32_t)__cvta_generic_to_shared(smem_raw);
   // (lane 0's value of a lane-dependent expression: a shuffle of a warp-uniform value would be folded away)
   const uint32_t sb = __shfl_sync(FULL, smem0 + (uint32_t)lane0, 0);  // staged scene tables (SMALL)
-  const int wofs = (SMALL ? (int)SM_BYTES : cfg.shape_bytes) + warp * cfg.per_warp_bytes;
+  const int wofs = (SMALL ? (int)SM_BYTES + (ACC == ACC_REG ? (int)SM_JUMP_BYTES : 0) : cfg.shape_bytes) + warp * cfg.per_warp_bytes;
   const uint32_t wb = __shfl_sync(FULL, smem0 + (uint32_t)(wofs + lane0), 0);  // this warp's record stack
   const uint32_t curb = wb + (uint32_t)cfg.cap * (uint32_t)sizeof(ScatterRec);  // the partly consumed record
   constexpr bool MULTI_SLOT = ACC != ACC_REG;
@@ -382,6 +411,11 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
         bool last_of_pixel = false;
         int rslot = 0;  // ERR: the slot field of this ray's records, the batch (`slot` stays the pixel in the task)
         if (primary_phase) {
+          // SMALL one-pixel tasks: sample ls = 32 round + lane has stratum own_stratum(32 round) + c lane (c the
+          // partition stride), so its jitter state J_2s(aa_task) is the lane's table entry applied to one
+          // warp-uniform jump per round (affine maps mod 2^64 compose exactly)
+          uint64_t aa_round = 0;
+          if (SMALL && ACC == ACC_REG && a.S > 0) aa_round = pcg_jump(aa_task, 2ull * (unsigned)own_stratum(a, round * 32), a.jump);
           const int j = round * 32 + lane;
           slot = j / L;
           const int ls = j - slot * L;
@@ -398,7 +432,10 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
             const unsigned long long k = (unsigned long long)pix * S2 + s;
             Pcg aa;
             aa.inc = a.aa_inc;
-            if (ACC == ACC_REG) aa.state = (a.S > 0) ? pcg_jump(aa_task, 2ull * (unsigned)s, a.jump) : 0;
+            if (SMALL && ACC == ACC_REG) {
+              const ulonglong2 jl = lds2u64c(sb + SM_JUMP + 16 * lane);
+              aa.state = (a.S > 0) ? jl.x * aa_round + jl.y : 0;
+            } else if (ACC == ACC_REG) aa.state = (a.S > 0) ? pcg_jump(aa_task, 2ull * (unsigned)s, a.jump) : 0;
             else aa.state = (a.S > 0) ? pcg_jump(a.aa_state, 2ull * k, a.jump) : 0;
             ray = primary_ray_mul(a, cfg.inv_w, cfg.inv_h, cfg.inv_s, col, row, s, aa);
             rng = pcg_seed(a.pt_state, (a.pt_inc >> 1) + k);
@@ -699,7 +736,7 @@ inline cudaError_t launch_pt_warp_impl(const SceneView<float>& sc, const RenderA
   long long cap = a.num_of_rays == 1 ? prims + 32 : prims + 32ll * (long long)a.max_depth;
   if (cap < 64) cap = 64;
   int acc_mode = cfg.group == 1 ? ACC_REG : (cfg.group <= RT_ACC_LANES_MAX_GROUP ? ACC_LANES : ACC_SEG);
-  cfg.shape_bytes = small ? (int)SM_BYTES : (shapes_smem ? (int)((shape_bytes + 15) / 16 * 16) : 0);
+  cfg.shape_bytes = small ? (int)SM_BYTES + (acc_mode == ACC_REG ? (int)SM_JUMP_BYTES : 0) : (shapes_smem ? (int)((shape_bytes + 15) / 16 * 16) : 0);
   const size_t limit = 200 * 1024;
   int warps = (small ? RT_SMALL_THREADS : RT_WARP_MAX_THREADS) / 32;
   size_t per_warp = 0, smem = 0;
