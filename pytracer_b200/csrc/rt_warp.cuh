@@ -17,6 +17,8 @@
 // uniforms are the halves of z, a roulette draw is a PCG32 step from z — so the image depends only
 // on (sample index, position in the tree) and not on lane assignment, GPU count or partition.
 #pragma once
+#include <type_traits>
+
 #include "rt_kernels.cuh"
 
 #define RT_WARP_MAX_THREADS 256
@@ -109,8 +111,11 @@ RT_DEV void err_store(const ErrArgs& e, int L, const float* bsum, int g, long lo
 }
 
 // SMALL instantiation: every table of the scene lives in shared memory at FIXED offsets (capacity for
-// the largest small scene, 3.3 KB), re-packed by the staging loop into what the per-ray code reads:
-//   SM_INVM / SM_M   [16][12] fp32 transforms (three LDS.128 per shape)
+// the largest small scene, 3.6 KB), re-packed by the staging loop into what the per-ray code reads:
+//   SM_INVM / SM_M   [16][12] fp32 transforms, rows 0 and 1 interleaved column by column for the paired FP32
+//                    pipe: {r0.x, r1.x, r0.y, r1.y}, {r0.z, r1.z, r0.w, r1.w}, then row 2 (three LDS.128 per shape)
+//   SM_PLANE2        [8][8] row 2 of the inverse transforms of planes 2j and 2j + 1, interleaved:
+//                    {x, x', y, y'}, {z, z', w, w'} (the odd plane of an odd count pairs with zeros)
 //   SM_ORIG          [16] index in World.shapes
 //   SM_SHAPE_MAT     [16] the shape's material as one int4 {brdf_kind, brdf_pigment, emitted_pigment, flags}
 //                    (no material-index indirection)
@@ -125,7 +130,8 @@ enum {
   SM_INVM = 0,
   SM_M = SM_INVM + RT_SMALL_MAX_SHAPES * 48,
   SM_ORIG = SM_M + RT_SMALL_MAX_SHAPES * 48,
-  SM_SHAPE_MAT = SM_ORIG + RT_SMALL_MAX_SHAPES * 4,
+  SM_PLANE2 = SM_ORIG + RT_SMALL_MAX_SHAPES * 4,
+  SM_SHAPE_MAT = SM_PLANE2 + RT_SMALL_MAX_SHAPES / 2 * 32,
   SM_PIG = SM_SHAPE_MAT + RT_SMALL_MAX_SHAPES * 16,
   SM_PIG_STRIDE = 48,
   SM_BYTES = SM_PIG + RT_SMALL_MAX_PIGMENTS * SM_PIG_STRIDE,
@@ -143,6 +149,15 @@ RT_DEV void stage_words(void* sh, const void* g, int bytes) {  // 4-byte granula
   const uint32_t* src = reinterpret_cast<const uint32_t*>(g);
   uint32_t* dst = reinterpret_cast<uint32_t*>(sh);
   for (int i = threadIdx.x; i < bytes / 4; i += blockDim.x) dst[i] = __ldg(src + i);
+}
+
+// SM_INVM / SM_M layout from row-major [n][12] (see the table list above)
+RT_DEV void stage_xf_pairs(void* sh, const float* g, int n_shapes) {
+  float* dst = reinterpret_cast<float*>(sh);
+  for (int i = threadIdx.x; i < n_shapes * 12; i += blockDim.x) {
+    const int k = i % 12, src = k < 8 ? ((k & 1) << 2) + (k >> 1) : k;  // 0 4 1 5 2 6 3 7 8 9 10 11
+    dst[i] = __ldg(g + (i - k) + src);
+  }
 }
 
 // ---- shared memory by 32-bit window address ------------------------------------------------------
@@ -182,11 +197,6 @@ RT_DEV ulonglong2 lds2u64c(uint32_t a) {
   asm volatile("ld.shared.v2.u64 {%0, %1}, [%2];" : "=l"(v.x), "=l"(v.y) : "r"(a));
   return v;
 }
-RT_DEV Rows3 lds_rows(uint32_t a) {
-  Rows3 m;
-  m.r0 = lds4c(a); m.r1 = lds4c(a + 16); m.r2 = lds4c(a + 32);
-  return m;
-}
 
 // Closest hit over a handful of shapes staged at `sb` (demo.txt: one sphere, two planes): World.ray_intersection
 // (world.py:51-69) without a sweep / candidate list, every shape tested directly and without branches —
@@ -198,6 +208,73 @@ RT_DEV Rows3 lds_rows(uint32_t a) {
 // parameters, read from the constant bank): no loop counter, and every table offset is an immediate off `sb`
 // (spheres) or off the first plane's address (planes).  A runtime-bounded loop cost ~15 instructions of
 // header per shape, as much as a plane test.
+//
+// The per-ray arithmetic runs partly on the paired FP32 pipe (fma.rn.f32x2, SASS FFMA2), on operands the staged
+// tables hold as register pairs: rows 0 and 1 of a transform column by column (one packed FMA chain gives
+// {x', y'} of a point or a direction), and the plane rows two planes at a time.  The ray's components enter as
+// scalar broadcast operands.  Each half of a packed FMA is one fmaf and a packed product is one fp32 product,
+// so every value is the same IEEE operation in the same association as in the scalar forms of rt_device.cuh
+// (sphere_cross_rows, local_hit_rows, world_frame_rows): the image is the same bit for bit.
+struct XfPairs {  // a SM_INVM / SM_M entry in registers
+  f32x2 x, y, z, w;  // {r0.c, r1.c} for the columns c = x, y, z, w
+  float4 r2;
+};
+RT_DEV XfPairs lds_xf(uint32_t a) {
+  XfPairs m;
+  const ulonglong2 p = lds2u64c(a), q = lds2u64c(a + 16);
+  m.x = p.x; m.y = p.y; m.z = q.x; m.w = q.y;
+  m.r2 = lds4c(a + 32);
+  return m;
+}
+RT_DEV f32x2 bc2(float v) { return pk2(v, v); }  // a scalar broadcast operand of a packed instruction
+// {x', y'} of M p + t (fmaf(r.x, p.x, fmaf(r.y, p.y, fmaf(r.z, p.z, r.w))) per row) and of M v
+// (fmaf(r.x, v.x, fmaf(r.y, v.y, r.z * v.z)))
+RT_DEV f32x2 xf_point01(const XfPairs& m, V3<float> p) { return fma2(m.x, bc2(p.x), fma2(m.y, bc2(p.y), fma2(m.z, bc2(p.z), m.w))); }
+RT_DEV f32x2 xf_vec01(const XfPairs& m, V3<float> v) { return fma2(m.x, bc2(v.x), fma2(m.y, bc2(v.y), mul2(m.z, bc2(v.z)))); }
+// sphere_cross_rows on a staged entry
+RT_DEV bool sphere_cross_small(const XfPairs& M, const Ray<float>& r, float& tm, float& half) {
+  const float4 r2 = M.r2;
+  const f32x2 pxy = xf_point01(M, r.o), dxy = xf_vec01(M, r.d);
+  float px, py, dx, dy;
+  upk2(pxy, px, py); upk2(dxy, dx, dy);
+  const float pz = fmaf(r2.x, r.o.x, fmaf(r2.y, r.o.y, fmaf(r2.z, r.o.z, r2.w)));
+  const float dz = fmaf(r2.x, r.d.x, fmaf(r2.y, r.d.y, r2.z * r.d.z));
+  const float a = fmaf(dx, dx, fmaf(dy, dy, dz * dz));
+  const float hb = fmaf(px, dx, fmaf(py, dy, pz * dz));
+  const float inv = fast_rcp(a);
+  const float s = hb * inv;
+  float qx, qy;
+  upk2(fma2(dxy, bc2(-s), pxy), qx, qy);
+  const float qz = fmaf(-s, dz, pz);
+  const float w = (1.0f - fmaf(qx, qx, fmaf(qy, qy, qz * qz))) * inv;
+  tm = -s;
+  half = fast_sqrt(fmaxf(w, 0.0f));
+  return w > 0.0f;
+}
+// local_hit_rows and world_frame_rows on staged entries
+RT_DEV LocalHit<float> local_hit_rows(const XfPairs& M, const Ray<float>& r, float t) {
+  LocalHit<float> L;
+  V3<float> o;
+  upk2(xf_point01(M, r.o), o.x, o.y);
+  upk2(xf_vec01(M, r.d), L.d.x, L.d.y);
+  o.z = fmaf(r.o.x, M.r2.x, fmaf(r.o.y, M.r2.y, fmaf(r.o.z, M.r2.z, M.r2.w)));
+  L.d.z = fmaf(r.d.x, M.r2.x, fmaf(r.d.y, M.r2.y, r.d.z * M.r2.z));
+  L.hp = o + t * L.d;
+  return L;
+}
+RT_DEV void world_frame_rows(const XfPairs& I, const XfPairs& M, const LocalHit<float>& L, bool sphere, V3<float>& point, V3<float>& normal) {
+  upk2(xf_point01(M, L.hp), point.x, point.y);
+  point.z = fmaf(L.hp.x, M.r2.x, fmaf(L.hp.y, M.r2.y, fmaf(L.hp.z, M.r2.z, M.r2.w)));
+  V3<float> n;
+  if (sphere) n = (dot(L.hp, L.d) < 0.f) ? L.hp : -L.hp;  // shapes.py:45-54
+  else n = mk3<float>(0.f, 0.f, (L.d.z < 0.f) ? 1.f : -1.f);
+  float i0x, i1x, i0y, i1y, i0z, i1z;
+  upk2(I.x, i0x, i1x); upk2(I.y, i0y, i1y); upk2(I.z, i0z, i1z);
+  n = mk3<float>(fmaf(n.x, i0x, fmaf(n.y, i1x, n.z * I.r2.x)),   // transpose of the inverse
+                 fmaf(n.x, i0y, fmaf(n.y, i1y, n.z * I.r2.y)),
+                 fmaf(n.x, i0z, fmaf(n.y, i1z, n.z * I.r2.z)));
+  normal = normalize(n);
+}
 RT_DEV void closest_small(uint32_t sb, int n_spheres, int n_shapes, const Ray<float>& r, int origin, float& best_t, int& best) {
   const float inf = Num<float>::inf();
   float ts = inf, tp = inf;
@@ -206,23 +283,28 @@ RT_DEV void closest_small(uint32_t sb, int n_spheres, int n_shapes, const Ray<fl
   for (int i = 0; i < RT_SMALL_MAX_SPHERES; ++i) {
     if (i >= n_spheres) break;
     float tm, half;
-    bool ok = sphere_cross_rows(lds_rows(sb + SM_INVM + 48 * i), r, tm, half);
+    bool ok = sphere_cross_small(lds_xf(sb + SM_INVM + 48 * i), r, tm, half);
     const float t1 = tm - half;
     float t = (t1 > r.tmin) ? t1 : tm + half;   // the first root beyond tmin, shapes.py:112-119
     if (i == origin) { t = 2.0f * tm; ok = true; }  // see sphere_t_at
     if (ok && t > r.tmin && t < ts) { ts = t; is = i; }
   }
-  // plane k is shape n_spheres + k
-  const uint32_t pb = sb + SM_INVM + 48 * (uint32_t)n_spheres;
+  // plane k is shape n_spheres + k; planes 2j and 2j + 1 go through one packed chain
   const int n_planes = n_shapes - n_spheres, porigin = origin - n_spheres;
 #pragma unroll
-  for (int k = 0; k < RT_SMALL_MAX_SHAPES; ++k) {
-    if (k >= n_planes) break;
-    const float4 row = lds4c(pb + 48 * k + 32);
-    const float oz = fmaf(r.o.x, row.x, fmaf(r.o.y, row.y, fmaf(r.o.z, row.z, row.w)));
-    const float dz = fmaf(r.d.x, row.x, fmaf(r.d.y, row.y, r.d.z * row.z));
-    const float t = -oz * fast_rcp(dz);
-    if (!(fabsf(dz) < 1e-5f) && t > r.tmin && t < tp && k != porigin) { tp = t; ip = k; }
+  for (int j = 0; j < RT_SMALL_MAX_SHAPES / 2; ++j) {
+    if (2 * j >= n_planes) break;
+    const ulonglong2 p = lds2u64c(sb + SM_PLANE2 + 32 * j), q = lds2u64c(sb + SM_PLANE2 + 32 * j + 16);
+    float oz[2], dz[2];
+    upk2(fma2(p.x, bc2(r.o.x), fma2(p.y, bc2(r.o.y), fma2(q.x, bc2(r.o.z), q.y))), oz[0], oz[1]);
+    upk2(fma2(p.x, bc2(r.d.x), fma2(p.y, bc2(r.d.y), mul2(q.x, bc2(r.d.z)))), dz[0], dz[1]);
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+      const int k = 2 * j + h;
+      if (k >= n_planes) break;
+      const float t = -oz[h] * fast_rcp(dz[h]);
+      if (!(fabsf(dz[h]) < 1e-5f) && t > r.tmin && t < tp && k != porigin) { tp = t; ip = k; }
+    }
   }
   if (ip >= 0) ip += n_spheres;
   bool plane = tp < ts;
@@ -305,8 +387,12 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
   const int warp = threadIdx.x >> 5;
   ScanSrc<float> src = global_src<float>(sc);
   if (SMALL) {
-    stage_words(smem_raw + SM_INVM, sc.invm, sc.n_shapes * 48);
-    stage_words(smem_raw + SM_M, sc.m, sc.n_shapes * 48);
+    stage_xf_pairs(smem_raw + SM_INVM, sc.invm, sc.n_shapes);
+    stage_xf_pairs(smem_raw + SM_M, sc.m, sc.n_shapes);
+    for (int i = threadIdx.x; i < RT_SMALL_MAX_SHAPES * 4; i += blockDim.x) {  // {x, x', y, y', z, z', w, w'} per plane pair
+      const int k = sc.n_spheres + 2 * (i >> 3) + (i & 1);
+      reinterpret_cast<float*>(smem_raw + SM_PLANE2)[i] = k < sc.n_shapes ? __ldg(sc.invm + 12 * k + 8 + ((i & 7) >> 1)) : 0.f;
+    }
     stage_words(smem_raw + SM_ORIG, sc.orig, sc.n_shapes * 4);
     for (int i = threadIdx.x; i < sc.n_shapes; i += blockDim.x) {
       const DevMaterial& mt = sc.materials[sc.material[i]];
@@ -527,7 +613,7 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
             // of a tree are its leaves, whose children render.py:100-101 cuts — for those only the emitted
             // colour matters, which for a uniform pigment needs no record at all.
             int brdf_kind, brdf_pig, emit_pig, mf;
-            Rows3 im;
+            typename std::conditional<SMALL, XfPairs, Rows3>::type im;
             const bool sphere = best < sc.n_spheres;
             if (SMALL) {
               const int4 mt = lds4ic(sb + SM_SHAPE_MAT + 16 * best);
@@ -536,9 +622,9 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
               const DevMaterial& mat = sc.materials[sc.material[best]];
               brdf_kind = mat.brdf_kind; brdf_pig = mat.brdf_pigment; emit_pig = mat.emitted_pigment; mf = mat.flags;
             }
-            auto rows_of = [&](bool inverse) -> Rows3 {
-              if (SMALL) return lds_rows(sb + (inverse ? SM_INVM : SM_M) + 48 * best);
-              return rows_at((inverse ? sc.invm : sc.m) + 12 * (size_t)best);
+            auto rows_of = [&](bool inverse) -> decltype(im) {
+              if constexpr (SMALL) return lds_xf(sb + (inverse ? SM_INVM : SM_M) + 48 * best);
+              else return rows_at((inverse ? sc.invm : sc.m) + 12 * (size_t)best);
             };
             auto pig_uniform = [&](int idx) -> V3<float> {
               if (SMALL) { const float4 q = lds4c(sb + SM_PIG + idx * SM_PIG_STRIDE + 16); return mk3<float>(q.x, q.y, q.z); }
@@ -575,7 +661,9 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
                 if (go_on && lum > 0.f) {
                   push = true;
                   V3<float> point, normal;
-                  world_frame_rows(im, rows_of(false), lh, sphere, point, normal);
+                  // (SMALL reloads the inverse: held across the shading above, its 12 registers made ptxas spill
+                  // loop state at the 80-register cap)
+                  world_frame_rows(SMALL ? rows_of(true) : im, rows_of(false), lh, sphere, point, normal);
                   const V3<float> nd = (brdf_kind == RT_BRDF_DIFFUSE) ? normal : specular_dir<float>(ray.d, normal);
                   const V3<float> w = inv_n * mul3(thr, hit_color);
                   out.a = make_float4(point.x, point.y, point.z,

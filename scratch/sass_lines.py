@@ -89,10 +89,15 @@ def main():
     op = lambda t: t.split()[1] if t.startswith("@") else t.split()[0]
     print(f"{args.kernel}: {total} SASS instructions, {sum(op(t).startswith('STL') for _, t in insts)} STL, "
           f"{sum(op(t).startswith('LDL') for _, t in insts)} LDL, {sum(op(t).startswith('CALL') for _, t in insts)} CALL")
+    # FP32-pipe opcodes per region: packed (FFMA2 / FMUL2 / FADD2) against scalar, and the moves that form pairs
+    fp_classes = (("packed", ("FFMA2", "FMUL2", "FADD2")), ("scalar", ("FFMA", "FMUL", "FADD")), ("mov", ("MOV", "PRMT")))
+    fp_of = lambda t: next((c for c, ops in fp_classes if op(t).split(".")[0] in ops), None)
+    per_region_fp = collections.Counter((region_of(chain), fp_of(t)) for chain, t in insts)
     if regions:
         for name, lo, hi in regions + [("other", 0, 0)]:
             span = f"{args.file}:{lo}-{hi}" if name != "other" else ""
-            print(f"  region {name:12s} {per_region[name]:6d}  {span}")
+            fp = "  ".join(f"{c} {per_region_fp[(name, c)]:4d}" for c, _ in fp_classes)
+            print(f"  region {name:12s} {per_region[name]:6d}  {fp}  {span}")
     for (f, n), k in sorted(per_line.items(), key=lambda kv: -kv[1])[:args.top]:
         print(f"  {f}:{n:<5d} {k:6d}")
 
