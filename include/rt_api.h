@@ -265,16 +265,25 @@ int rt_render_finish(rt_scene* scene, void* stream, rt_stats* stats);
  * tracer and renderer: jitter stream advanced by p * 2 * W * H * S^2 draws, pt_state by p PCG steps, sample
  * indices k = pix * S^2 + s.  Pass 0 traces every pixel; every further pass traces, in ascending order, the
  * pixels whose relative error e = max_c SE_c / max(mean_c, error_floor) is still above target_error and that
- * have passes left.  A pass's squared standard error comes from batch sums of its S^2 samples,
- * SE^2 = sum_b (T_b - n_b m)^2 / (n_b (B - 1) S^2).  A pixel with P passes reports mean = (sum of pass means,
+ * have passes left.  A pass's squared standard error comes from batch sums of its S^2 samples (sample s in batch
+ * s mod B' with B' = 32 / G, G = pixels per warp task, B = min(S^2, B') batches); `estimator` picks the formula:
+ *   RT_ERR_EST_BATCH  (default): SE^2 = sum_b (T_b - n_b m)^2 / (n_b (B - 1) S^2), unbiased for independent
+ *                     samples, too large where stratification removes variance (it treats strata as independent);
+ *   RT_ERR_EST_PAIRED (S even): collapsed strata, SE^2 = sum_j (T_2j - T_2j+1)^2 / S^4 over j < B / 2.  Batches
+ *                     2j and 2j + 1 hold horizontally adjacent strata in equal numbers, so each difference sums
+ *                     pair differences; the estimate is conservative and tight where radiance is smooth across
+ *                     two strata, with B / 2 degrees of freedom (half the batch estimator's).
+ * A pixel with P passes reports mean = (sum of pass means,
  * fp32, in pass order) / P, SE = sqrt(sum of SE^2) / P and P * S^2 samples; with P = 1 the mean is rt_render's
  * pixel bit for bit.  Path tracing, WARP variant (AUTO picks it), fp32, S >= 2, RT_PART_NONE, RT_RNG_STREAMS,
- * no peer images, no out_f64: anything else is RT_ERR_INVALID.  Host buffers, blocking; one device. */
+ * no peer images, no out_f64, a known estimator (RT_ERR_EST_PAIRED: S even): anything else is RT_ERR_INVALID.
+ * Host buffers, blocking; one device. */
+enum { RT_ERR_EST_BATCH = 0, RT_ERR_EST_PAIRED = 1 };
 typedef struct rt_adaptive_params {
   double target_error;        /* e threshold; <= 0: one pass, error map only */
   double error_floor;         /* absolute radiance floor of the relative error (> 0) */
   int32_t max_passes;         /* >= 1; pass p uses the PCG states defined above */
-  int32_t _pad;
+  int32_t estimator;          /* RT_ERR_EST_*: how a pass's SE^2 is formed (0 = batch) */
 } rt_adaptive_params;
 typedef struct rt_adaptive_stats {
   uint64_t rays_closest, rays_shadow, samples;

@@ -24,6 +24,8 @@ RT_MAX_PEERS = 8
 ACCELS = {"none": 0, "bvh": 1}  # RT_ACCEL_*
 
 RT_OK, RT_ERR_INVALID, RT_ERR_CUDA, RT_ERR_NO_DEVICE, RT_ERR_OVERFLOW = 0, -1, -2, -3, -4
+RT_ERR_EST_BATCH, RT_ERR_EST_PAIRED = 0, 1
+ERROR_ESTIMATORS = {"batch": 0, "paired": 1}
 
 c_double3 = C.c_double * 3
 
@@ -150,7 +152,7 @@ class rt_adaptive_params(C.Structure):
         ("target_error", C.c_double),
         ("error_floor", C.c_double),
         ("max_passes", C.c_int32),
-        ("_pad", C.c_int32),
+        ("estimator", C.c_int32),
     ]
 
 

@@ -756,6 +756,10 @@ extern "C" int rt_render_adaptive(rt_scene* s, const rt_render_params* p, const 
   if (p->num_of_rays < 1 || p->max_depth < 0) return fail(RT_ERR_INVALID, "rt_render_adaptive: num_of_rays %d, max_depth %d", p->num_of_rays, p->max_depth);
   if (ap->max_passes < 1 || !(ap->error_floor > 0.0) || std::isnan(ap->target_error))
     return fail(RT_ERR_INVALID, "rt_render_adaptive: max_passes %d, error_floor %g, target_error %g", ap->max_passes, ap->error_floor, ap->target_error);
+  if (ap->estimator != RT_ERR_EST_BATCH && ap->estimator != RT_ERR_EST_PAIRED)
+    return fail(RT_ERR_INVALID, "rt_render_adaptive: estimator %d", ap->estimator);
+  if (ap->estimator == RT_ERR_EST_PAIRED && p->samples_per_side % 2)  // a stratum without a partner
+    return fail(RT_ERR_INVALID, "rt_render_adaptive: the paired estimator needs an even samples_per_side (got %d)", p->samples_per_side);
   if ((long long)p->width * p->height >= (1ll << 31)) return fail(RT_ERR_INVALID, "rt_render_adaptive: image too large");
   CU(cudaSetDevice(s->device));
   RenderArgs a;
@@ -805,6 +809,7 @@ extern "C" int rt_render_adaptive(rt_scene* s, const rt_render_params* p, const 
     e.n_list = n_cur;
     e.err_mean = em;
     e.err_var = ev;
+    e.estimator = ap->estimator;
     CU(cudaMemsetAsync(ws->counters + CNT_TASK, 0, sizeof(unsigned long long), st));
     const char* why = nullptr;
     cudaError_t err = launch_pt_warp_err(v32, a, e, st, s->sm_count, &info, &why, s->bvh_n_nodes, s->bvh_n_prims, s->bvh_depth);

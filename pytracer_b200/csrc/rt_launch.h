@@ -32,6 +32,7 @@ struct ErrArgs {
   float* err_var;          // [entries][3] squared standard error of that mean
   int err_bpp;             // batches per pixel slot of a task (32 / G), set by the launcher
   unsigned err_magic;      // multiply-shift magic of x / err_bpp for x < 32
+  int32_t estimator;       // RT_ERR_EST_*: how err_store forms SE^2 from the batch sums
 };
 
 struct LaunchInfo {

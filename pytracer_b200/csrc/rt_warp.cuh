@@ -56,6 +56,10 @@ struct WarpCfg {
 // the squared standard error of the pass mean m follows from them when the task ends:
 //   SE^2 = sum_b (T_b - n_b m)^2 / (n_b (B - 1) L)
 // (unbiased for independent samples; B = L gives s^2 / L).
+// RT_ERR_EST_PAIRED (S even) collapses pairs of strata instead: strata 2k and 2k + 1 (horizontal neighbours)
+// land in batches 2j and 2j + 1 (bpp is even), so D_j = T_2j - T_2j+1 sums the pair differences of group j and
+//   SE^2 = sum_j D_j^2 / L^2,   j < min(L, bpp) / 2
+// (E[D_j^2] >= the pairs' variances: conservative under stratification, tight where radiance is smooth).
 RT_DEV int err_batch_of(const ErrArgs& cfg, int ls) {
   return cfg.err_bpp == 32 ? (ls & 31) : ls - (int)(((unsigned)ls * cfg.err_magic) >> 16) * cfg.err_bpp;  // (ls < 32 when G > 1)
 }
@@ -88,8 +92,15 @@ RT_DEV void err_batch_add(float* bsum, int slot, bool on, V3<float> c, int lane)
 RT_DEV void err_store(const ErrArgs& e, int L, const float* bsum, int g, long long entry, V3<float> m, int lane) {
   const unsigned FULL = 0xffffffffu;
   const int bpp = e.err_bpp, B = min(L, bpp);
+  const bool paired = e.estimator == RT_ERR_EST_PAIRED;  // (a kernel parameter: warp-uniform)
   float tr = 0.f, tg = 0.f, tb = 0.f;
-  if (lane < B) {
+  if (paired) {
+    if (lane < B / 2) {
+      const float* t = bsum + 3 * (g * bpp + 2 * lane);
+      const float dr = t[0] - t[3], dg = t[1] - t[4], db = t[2] - t[5];
+      tr = __fmul_rn(dr, dr); tg = __fmul_rn(dg, dg); tb = __fmul_rn(db, db);  // (no fusion into the first add below)
+    }
+  } else if (lane < B) {
     const float n = (float)((L - 1 - lane) / bpp + 1);
     const float* t = bsum + 3 * (g * bpp + lane);
     const float dr = fmaf(-n, m.x, t[0]), dg = fmaf(-n, m.y, t[1]), db = fmaf(-n, m.z, t[2]);
@@ -102,7 +113,7 @@ RT_DEV void err_store(const ErrArgs& e, int L, const float* bsum, int g, long lo
     tb += __shfl_xor_sync(FULL, tb, d);
   }
   if (lane == 0) {
-    const float k = 1.f / ((float)(B - 1) * (float)L);
+    const float k = paired ? 1.f / ((float)L * (float)L) : 1.f / ((float)(B - 1) * (float)L);
     float* o = e.err_mean + 3 * entry;
     o[0] = m.x; o[1] = m.y; o[2] = m.z;
     float* v = e.err_var + 3 * entry;

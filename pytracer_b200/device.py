@@ -80,9 +80,10 @@ class DeviceScene:
         return out, hit, stats.as_dict()
 
     def render_adaptive(self, params: _abi.rt_render_params, target_error: float = 0.0, max_passes: int = 1,
-                        error_floor: float = 1e-2, out: Optional[np.ndarray] = None):
+                        error_floor: float = 1e-2, out: Optional[np.ndarray] = None, estimator: str = "batch"):
         """rt_render_adaptive: (mean image, SE image, samples per pixel, stats) as float32 [H][W][3] x 2 and
-        int32 [H][W]; ``max_passes`` passes of ``params.samples_per_side ** 2`` samples at most per pixel."""
+        int32 [H][W]; ``max_passes`` passes of ``params.samples_per_side ** 2`` samples at most per pixel.
+        ``estimator``: "batch" or "paired" (collapsed strata, even samples_per_side), or an RT_ERR_EST_* int."""
         H, W = params.height, params.width
         if out is None:
             out = np.empty((H, W, 3), dtype=np.float32)
@@ -91,6 +92,7 @@ class DeviceScene:
         samples = np.empty((H, W), dtype=np.int32)
         ap = _abi.rt_adaptive_params()
         ap.target_error, ap.error_floor, ap.max_passes = float(target_error), float(error_floor), int(max_passes)
+        ap.estimator = _abi.ERROR_ESTIMATORS[estimator] if isinstance(estimator, str) else int(estimator)
         stats = _abi.rt_adaptive_stats()
         _native.check(self._lib.rt_render_adaptive(self._handle, C.byref(params), C.byref(ap), _ptr(out), _ptr(err), _ptr(samples),
                                                    C.byref(stats)))

@@ -75,7 +75,8 @@ class ImageTracer:
             callback(col=self.image.width - 1, row=self.image.height - 1, **callback_kwargs)
 
     def fire_all_rays_adaptive(self, renderer, target_error: float = 0.0, max_samples_per_pixel: Optional[int] = None,
-                               error_floor: float = 1e-2, callback=None, callback_time_s: float = 2.0, **callback_kwargs) -> AdaptiveResult:
+                               error_floor: float = 1e-2, callback=None, callback_time_s: float = 2.0,
+                               error_estimator: str = "batch", **callback_kwargs) -> AdaptiveResult:
         """Path-traced image with a per-pixel Monte Carlo error map, optionally refined where it is noisy.
 
         Pass 0 is exactly ``fire_all_rays(renderer)``; every further pass traces ``samples_per_side ** 2`` more
@@ -83,7 +84,10 @@ class ImageTracer:
         ``target_error``, until they meet it or hold ``max_samples_per_pixel`` samples (default: one pass, the
         error map only).  Pass p of a pixel is that pixel of the (p+1)-th consecutive ``fire_all_rays``; a pixel
         with P passes holds the mean of its P pass values.  ``self.image`` receives the mean image, and
-        ``self.pcg`` and ``renderer.pcg`` are left where ``passes`` consecutive ``fire_all_rays`` leave them."""
+        ``self.pcg`` and ``renderer.pcg`` are left where ``passes`` consecutive ``fire_all_rays`` leave them.
+        ``error_estimator`` forms each pass's SE from the stratified samples: "batch" treats them as independent
+        (conservative); "paired" collapses pairs of horizontally adjacent strata, which credits stratification
+        and so reports less where radiance is smooth within the pixel (even ``samples_per_side`` only)."""
         spp = self.samples_per_side ** 2
         if not isinstance(renderer, CudaRenderer) or renderer.algorithm != "pathtracing":
             raise ValueError("fire_all_rays_adaptive needs a path-tracing CudaRenderer")
@@ -97,6 +101,10 @@ class ImageTracer:
             raise ValueError(f"target_error must be finite and >= 0 (got {target_error})")
         if not (np.isfinite(error_floor) and error_floor > 0):
             raise ValueError(f"error_floor must be > 0 (got {error_floor})")
+        if error_estimator not in _abi.ERROR_ESTIMATORS:
+            raise ValueError(f"error_estimator must be one of {sorted(_abi.ERROR_ESTIMATORS)} (got {error_estimator!r})")
+        if error_estimator == "paired" and self.samples_per_side % 2:
+            raise ValueError(f"the paired error estimator needs an even samples_per_side (got {self.samples_per_side})")
         if max_samples_per_pixel is None:
             max_samples_per_pixel = spp
         if int(max_samples_per_pixel) != max_samples_per_pixel or max_samples_per_pixel < spp or max_samples_per_pixel % spp:
@@ -109,7 +117,7 @@ class ImageTracer:
             callback(col=0, row=0, **callback_kwargs)
         scene = renderer.device_scene()
         rgb, err, samples, stats = scene.render_adaptive(self._params(renderer), target_error, max_passes, error_floor,
-                                                         out=self._adoptable_buffer())
+                                                         out=self._adoptable_buffer(), estimator=error_estimator)
         passes = stats["passes"]
         self.last_stats = renderer.last_stats = stats
         for _ in range(passes):  # where `passes` consecutive fire_all_rays leave both generators

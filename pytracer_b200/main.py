@@ -60,7 +60,7 @@ def load_scene(path: str, variables, parser: str):
 
 
 def adaptive_cli_problem(algorithm, samples_per_pixel, gpus, variant, precision, target_error, max_samples_per_pixel,
-                         error_floor):
+                         error_floor, error_estimator="batch"):
     """Why `render --error-output / --target-error / --max-samples-per-pixel` cannot run as asked (None: it can)."""
     if algorithm != "pathtracing":
         return "--error-output, --target-error and --max-samples-per-pixel need --algorithm pathtracing"
@@ -79,6 +79,9 @@ def adaptive_cli_problem(algorithm, samples_per_pixel, gpus, variant, precision,
     if max_samples_per_pixel is not None and (max_samples_per_pixel < samples_per_pixel or max_samples_per_pixel % samples_per_pixel):
         return (f"--max-samples-per-pixel ({max_samples_per_pixel}) must be a positive multiple of "
                 f"--samples-per-pixel ({samples_per_pixel})")
+    if error_estimator == "paired" and int(sqrt(samples_per_pixel)) % 2:
+        return (f"--error-estimator paired needs an even number of samples per side "
+                f"(--samples-per-pixel 4, 16, 36, 64, ...; got {samples_per_pixel})")
     return None
 
 
@@ -111,10 +114,13 @@ def cli():
               help="render adaptively: trace more passes of --samples-per-pixel samples where the relative error is above this")
 @click.option("--max-samples-per-pixel", type=int, default=None, help="with --target-error: samples per pixel at most")
 @click.option("--error-floor", type=float, default=1e-2, help="radiance below which the relative error is taken against this floor")
+@click.option("--error-estimator", type=click.Choice(["batch", "paired"]), default="batch",
+              help="how the standard error is formed: batch (strata as independent samples) or paired (collapsed pairs "
+                   "of adjacent strata, tighter under stratification; even samples per side)")
 @click.argument("input_scene_name", type=str)
 def render(width, height, algorithm, pfm_output, png_output, num_of_rays, max_depth, init_state, init_seq,
            samples_per_pixel, declare_float, variant, precision, parser, accel, gpus, launcher, error_output, target_error,
-           max_samples_per_pixel, error_floor, input_scene_name):
+           max_samples_per_pixel, error_floor, error_estimator, input_scene_name):
     import os
 
     if gpus > 1 and launcher == "torchrun" and "WORLD_SIZE" not in os.environ:  # one process per GPU: hand the same command line to torchrun
@@ -132,9 +138,12 @@ def render(width, height, algorithm, pfm_output, png_output, num_of_rays, max_de
         print(f"Error, the number of samples per pixel ({samples_per_pixel}) must be a perfect square")
         return
     adaptive = error_output is not None or target_error is not None or max_samples_per_pixel is not None
+    if error_estimator != "batch" and not adaptive:
+        print("Error, --error-estimator applies to --error-output and --target-error")
+        sys.exit(1)
     if adaptive:
         problem = adaptive_cli_problem(algorithm, samples_per_pixel, gpus, variant, precision, target_error,
-                                       max_samples_per_pixel, error_floor)
+                                       max_samples_per_pixel, error_floor, error_estimator)
         if problem:
             print(f"Error, {problem}")
             sys.exit(1)
@@ -168,7 +177,8 @@ def render(width, height, algorithm, pfm_output, png_output, num_of_rays, max_de
     result = None
     if adaptive:
         result = tracer.fire_all_rays_adaptive(renderer, target_error=target_error or 0.0,
-                                               max_samples_per_pixel=max_samples_per_pixel, error_floor=error_floor)
+                                               max_samples_per_pixel=max_samples_per_pixel, error_floor=error_floor,
+                                               error_estimator=error_estimator)
     else:
         tracer.fire_all_rays(renderer, comm=comm)
     elapsed = perf_counter() - start
