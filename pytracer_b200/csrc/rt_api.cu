@@ -542,9 +542,12 @@ extern "C" int rt_render_device(rt_scene* s, const rt_render_params* p, void* d_
   const bool partial_rows = a.part_mode == RT_PART_ROWS && !a.rows_compact && a.n_peers == 0;
   long long S2 = p->samples_per_side > 0 ? (long long)p->samples_per_side * p->samples_per_side : 1;
   const bool no_strata = a.part_mode == RT_PART_SPP && a.part_rank >= S2;
+  // a pixel nobody traces: no shape (-1), or zero rays under RT_HIT_RAY_COUNT, so that the counts of the
+  // ranks add up to those of the whole image
+  const int no_hit = a.hit_mode == RT_HIT_RAY_COUNT ? 0 : 0xff;
   if (partial_rows || no_strata) {
     CU(cudaMemsetAsync(d_out_rgb, 0, px * 3 * (a.out_f64 ? sizeof(double) : sizeof(float)), st));
-    if (d_out_hit) CU(cudaMemsetAsync(d_out_hit, 0xff, px * sizeof(int32_t), st));
+    if (d_out_hit) CU(cudaMemsetAsync(d_out_hit, no_hit, px * sizeof(int32_t), st));
   }
   if (p->accel != RT_ACCEL_NONE && p->accel != RT_ACCEL_BVH) return fail(RT_ERR_INVALID, "accel %d", p->accel);
   const int accel = (p->accel == RT_ACCEL_BVH && s->n_spheres > 0) ? RT_ACCEL_BVH : RT_ACCEL_NONE;
@@ -563,7 +566,7 @@ extern "C" int rt_render_device(rt_scene* s, const rt_render_params* p, void* d_
     long long n = (long long)make_pixel_count(a);
     unsigned long long samples = (unsigned long long)n;
     e = cudaMemsetAsync(d_out_rgb, 0, px * 3 * (a.out_f64 ? sizeof(double) : sizeof(float)), st);
-    if (e == cudaSuccess && d_out_hit) e = cudaMemsetAsync(d_out_hit, 0xff, px * sizeof(int32_t), st);
+    if (e == cudaSuccess && d_out_hit) e = cudaMemsetAsync(d_out_hit, no_hit, px * sizeof(int32_t), st);
     if (e == cudaSuccess) e = cudaMemcpyAsync(s->ws->counters + CNT_SAMPLES, &samples, sizeof(samples), cudaMemcpyHostToDevice, st);
     s->last_info.variant = variant;
   } else if (!pt && precision == RT_PRECISION_HYBRID) {
