@@ -228,6 +228,7 @@ RT_DEV void upk2(f32x2 v, float& lo, float& hi) { asm("mov.b64 {%0, %1}, %2;" : 
 RT_DEV f32x2 fma2(f32x2 a, f32x2 b, f32x2 c) { f32x2 d; asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(a), "l"(b), "l"(c)); return d; }
 RT_DEV f32x2 mul2(f32x2 a, f32x2 b) { f32x2 d; asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b)); return d; }
 RT_DEV f32x2 sub2(f32x2 a, f32x2 b) { f32x2 d; asm("sub.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b)); return d; }
+RT_DEV f32x2 add2(f32x2 a, f32x2 b) { f32x2 d; asm("add.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b)); return d; }
 
 // The sweep's gate delta/4 = (o'.d')^2 - a (|o'|^2 - 1) > 0 is evaluated in fp32 and every decision about a
 // sphere is then taken by sphere_cross on the spheres that pass, so the gate must not LOSE spheres: a

@@ -122,15 +122,18 @@ RT_DEV void err_store(const ErrArgs& e, int L, const float* bsum, int g, long lo
 }
 
 // SMALL instantiation: every table of the scene lives in shared memory at FIXED offsets (capacity for
-// the largest small scene, 3.6 KB), re-packed by the staging loop into what the per-ray code reads:
+// the largest small scene, 3.8 KB), re-packed by the staging loop into what the per-ray code reads:
 //   SM_INVM / SM_M   [16][12] fp32 transforms, rows 0 and 1 interleaved column by column for the paired FP32
 //                    pipe: {r0.x, r1.x, r0.y, r1.y}, {r0.z, r1.z, r0.w, r1.w}, then row 2 (three LDS.128 per shape)
 //   SM_PLANE2        [8][8] row 2 of the inverse transforms of planes 2j and 2j + 1, interleaved:
 //                    {x, x', y, y'}, {z, z', w, w'} (the odd plane of an odd count pairs with zeros)
+//   SM_INVT          [16][4] columns x and y of rows 0 and 1 of the inverse transforms, {r0.x, r0.y, r1.x, r1.y}: with
+//                    row 2 of SM_INVM, the {x, y} pairs of the normal transform (transpose of the inverse)
 //   SM_ORIG          [16] index in World.shapes
 //   SM_SHAPE_MAT     [16] the shape's material as one int4 {brdf_kind, brdf_pigment, emitted_pigment, flags}
 //                    (no material-index indirection)
-//   SM_PIG           [32] 48-byte pigment records {kind, steps, tex_w, tex_h | c1.xyz, c2.x | c2.yz, texture handle}
+//   SM_PIG           [32] 48-byte pigment records {kind, steps, tex_w, tex_h | c1.x, c2.x, c1.y, c1.z | c2.y, c2.z,
+//                    texture handle}: the y and z channels of each colour are a register pair as loaded
 //   SM_JUMP          [32] {mult, plus} of the jitter jump by 2 c k draws (c the partition stride), one-pixel tasks
 //                    (ACC_REG) only: the block is SM_JUMP_BYTES longer there
 #define RT_SMALL_MAX_SPHERES 8
@@ -140,7 +143,8 @@ RT_DEV void err_store(const ErrArgs& e, int L, const float* bsum, int g, long lo
 enum {
   SM_INVM = 0,
   SM_M = SM_INVM + RT_SMALL_MAX_SHAPES * 48,
-  SM_ORIG = SM_M + RT_SMALL_MAX_SHAPES * 48,
+  SM_INVT = SM_M + RT_SMALL_MAX_SHAPES * 48,
+  SM_ORIG = SM_INVT + RT_SMALL_MAX_SHAPES * 16,
   SM_PLANE2 = SM_ORIG + RT_SMALL_MAX_SHAPES * 4,
   SM_SHAPE_MAT = SM_PLANE2 + RT_SMALL_MAX_SHAPES / 2 * 32,
   SM_PIG = SM_SHAPE_MAT + RT_SMALL_MAX_SHAPES * 16,
@@ -262,7 +266,7 @@ RT_DEV bool sphere_cross_small(const XfPairs& M, const Ray<float>& r, float& tm,
   half = fast_sqrt(fmaxf(w, 0.0f));
   return w > 0.0f;
 }
-// local_hit_rows and world_frame_rows on staged entries
+// local_hit_rows on a staged entry
 RT_DEV LocalHit<float> local_hit_rows(const XfPairs& M, const Ray<float>& r, float t) {
   LocalHit<float> L;
   V3<float> o;
@@ -273,19 +277,79 @@ RT_DEV LocalHit<float> local_hit_rows(const XfPairs& M, const Ray<float>& r, flo
   L.hp = o + t * L.d;
   return L;
 }
-RT_DEV void world_frame_rows(const XfPairs& I, const XfPairs& M, const LocalHit<float>& L, bool sphere, V3<float>& point, V3<float>& normal) {
+
+// The shading and scatter arithmetic of the SMALL kernel with {x, y} of each vector as one register pair, z scalar.
+// Every value is the operation of the scalar form (world_frame_rows, diffuse_dir, specular_dir, the shading
+// products) in the association and with the FMA contractions ptxas gave that form, written out as fmaf /
+// __fmul_rn: the dot products of normalize and specular_dir are fmaf(z, z', fmaf(x, x', y * y')), a diffuse
+// direction component is fmaf(n, sin, fmaf(cos, s e2, cos (c e1))).  A packed half is that same operation, so the
+// image is the same bit for bit.
+RT_DEV f32x2 ldsu64c(uint32_t a) {
+  f32x2 v;
+  asm volatile("ld.shared.u64 %0, [%1];" : "=l"(v) : "r"(a));
+  return v;
+}
+RT_DEV float dot_small(float x, float y, float z, float x2, float y2, float z2) { return fmaf(z, z2, fmaf(x, x2, __fmul_rn(y, y2))); }
+// world_frame_rows on staged entries: `inv` and `invt` are the shape's SM_INVM and SM_INVT entries
+RT_DEV void world_frame_small(uint32_t inv, uint32_t invt, const XfPairs& M, const LocalHit<float>& L, bool sphere, V3<float>& point,
+                              f32x2& nxy, float& nz) {
   upk2(xf_point01(M, L.hp), point.x, point.y);
   point.z = fmaf(L.hp.x, M.r2.x, fmaf(L.hp.y, M.r2.y, fmaf(L.hp.z, M.r2.z, M.r2.w)));
   V3<float> n;
   if (sphere) n = (dot(L.hp, L.d) < 0.f) ? L.hp : -L.hp;  // shapes.py:45-54
   else n = mk3<float>(0.f, 0.f, (L.d.z < 0.f) ? 1.f : -1.f);
-  float i0x, i1x, i0y, i1y, i0z, i1z;
-  upk2(I.x, i0x, i1x); upk2(I.y, i0y, i1y); upk2(I.z, i0z, i1z);
-  n = mk3<float>(fmaf(n.x, i0x, fmaf(n.y, i1x, n.z * I.r2.x)),   // transpose of the inverse
-                 fmaf(n.x, i0y, fmaf(n.y, i1y, n.z * I.r2.y)),
-                 fmaf(n.x, i0z, fmaf(n.y, i1z, n.z * I.r2.z)));
-  normal = normalize(n);
+  const ulonglong2 t = lds2u64c(invt), r2 = lds2u64c(inv + 32);  // {r0.x, r0.y}, {r1.x, r1.y};  {r2.x, r2.y}, {r2.z, r2.w}
+  float i0z, i1z, i2z, i2w, mx, my;
+  upk2(ldsu64c(inv + 16), i0z, i1z);
+  upk2(r2.y, i2z, i2w);
+  const f32x2 m = fma2(t.x, bc2(n.x), fma2(t.y, bc2(n.y), mul2(r2.x, bc2(n.z))));  // transpose of the inverse
+  const float mz = fmaf(n.x, i0z, fmaf(n.y, i1z, n.z * i2z));
+  upk2(m, mx, my);
+  const float r = rsqrtf(dot_small(mx, my, mz, mx, my, mz));  // normalize
+  nxy = mul2(bc2(r), m);
+  nz = r * mz;
 }
+// diffuse_dir around the unit normal {nxy, nz}
+RT_DEV V3<float> diffuse_dir_small(f32x2 nxy, float nz, float u1, float u2) {
+  float nx, ny;
+  upk2(nxy, nx, ny);
+  const float sign = (nz > 0.f) ? 1.f : -1.f;  // onb_from_z
+  const float a = -fast_rcp(sign + nz);
+  const float b = __fmul_rn(__fmul_rn(nx, ny), a);
+  const f32x2 e1 = pk2(fmaf(__fmul_rn(__fmul_rn(sign, nx), nx), a, 1.f), __fmul_rn(sign, b));  // e1.z = -sign nx
+  const f32x2 e2 = pk2(b, fmaf(__fmul_rn(ny, ny), a, sign));                                   // e2.z = -ny
+  const float cos_theta = fast_sqrt(u1), sin_theta = fast_sqrt(1.f - u1);
+  const float phi = (float)(2.0 * 3.14159265358979323846) * u2;
+  float s, c;
+  Num<float>::sincos(phi, &s, &c);
+  const f32x2 dxy = fma2(nxy, bc2(sin_theta), fma2(bc2(cos_theta), mul2(e2, bc2(s)), mul2(bc2(cos_theta), mul2(e1, bc2(c)))));
+  V3<float> d;
+  upk2(dxy, d.x, d.y);
+  d.z = fmaf(nz, sin_theta, fmaf(cos_theta, __fmul_rn(s, -ny), __fmul_rn(cos_theta, __fmul_rn(c, __fmul_rn(-sign, nx)))));
+  return d;
+}
+// specular_dir of `in` about the normal {nxy, nz}
+RT_DEV void specular_dir_small(V3<float> in, f32x2 nxy, float nz, f32x2& oxy, float& oz) {
+  float nx, ny, mx, my;
+  upk2(nxy, nx, ny);
+  const float ri = rsqrtf(dot_small(in.x, in.y, in.z, in.x, in.y, in.z));
+  const float rn = rsqrtf(dot_small(nx, ny, nz, nx, ny, nz));
+  const f32x2 mxy = mul2(bc2(rn), nxy);  // (rd's products stay scalar: pairing `in` made ptxas spill at 80 registers)
+  const float dx = ri * in.x, dy = ri * in.y, dz = ri * in.z, mz = rn * nz;
+  upk2(mxy, mx, my);
+  const float dp = dot_small(dx, dy, dz, mx, my, mz);
+  oxy = fma2(bc2(-dp), add2(mxy, mxy), pk2(dx, dy));  // rd - dp (2 n)
+  oz = fmaf(-dp, mz + mz, dz);
+}
+// a * b, for SMALL with {y, z} on one packed product
+template <bool SMALL> RT_DEV V3<float> mul3_k(V3<float> a, V3<float> b) {
+  if constexpr (!SMALL) return mul3(a, b);
+  V3<float> r;
+  r.x = a.x * b.x;
+  upk2(mul2(pk2(a.y, a.z), pk2(b.y, b.z)), r.y, r.z);
+  return r;
+}
+
 RT_DEV void closest_small(uint32_t sb, int n_spheres, int n_shapes, const Ray<float>& r, int origin, float& best_t, int& best) {
   const float inf = Num<float>::inf();
   float ts = inf, tp = inf;
@@ -328,11 +392,11 @@ RT_DEV void closest_small(uint32_t sb, int n_spheres, int n_shapes, const Ray<fl
 RT_DEV V3<float> pigment_color_small(uint32_t pa, float u, float v) {
   const int4 h = lds4ic(pa);
   const float4 q = lds4c(pa + 16);
-  if (h.x == RT_PIGMENT_UNIFORM) return mk3<float>(q.x, q.y, q.z);
+  if (h.x == RT_PIGMENT_UNIFORM) return mk3<float>(q.x, q.z, q.w);
   const float4 w = lds4c(pa + 32);
   if (h.x == RT_PIGMENT_CHECKERED) {
     const int iu = __float2int_rd(u * (float)h.y), iv = __float2int_rd(v * (float)h.y);
-    return (((iu ^ iv) & 1) == 0) ? mk3<float>(q.x, q.y, q.z) : mk3<float>(q.w, w.x, w.y);
+    return (((iu ^ iv) & 1) == 0) ? mk3<float>(q.x, q.z, q.w) : mk3<float>(q.y, w.x, w.y);
   }
   int col = (int)(u * (float)h.z), row = (int)(v * (float)h.w);
   col = min(max(col, 0), h.z - 1);
@@ -400,6 +464,8 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
   if (SMALL) {
     stage_xf_pairs(smem_raw + SM_INVM, sc.invm, sc.n_shapes);
     stage_xf_pairs(smem_raw + SM_M, sc.m, sc.n_shapes);
+    for (int i = threadIdx.x; i < sc.n_shapes * 4; i += blockDim.x)  // {r0.x, r0.y, r1.x, r1.y} of each inverse
+      reinterpret_cast<float*>(smem_raw + SM_INVT)[i] = __ldg(sc.invm + 12 * (i >> 2) + 4 * ((i >> 1) & 1) + (i & 1));
     for (int i = threadIdx.x; i < RT_SMALL_MAX_SHAPES * 4; i += blockDim.x) {  // {x, x', y, y', z, z', w, w'} per plane pair
       const int k = sc.n_spheres + 2 * (i >> 3) + (i & 1);
       reinterpret_cast<float*>(smem_raw + SM_PLANE2)[i] = k < sc.n_shapes ? __ldg(sc.invm + 12 * k + 8 + ((i & 7) >> 1)) : 0.f;
@@ -413,7 +479,7 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
       const DevPigment& pg = sc.pigments[i];
       float4* o = reinterpret_cast<float4*>(smem_raw + SM_PIG + i * SM_PIG_STRIDE);
       o[0] = make_float4(__int_as_float(pg.kind), __int_as_float(pg.steps), __int_as_float(pg.tex_w), __int_as_float(pg.tex_h));
-      o[1] = make_float4(pg.c1[0], pg.c1[1], pg.c1[2], pg.c2[0]);
+      o[1] = make_float4(pg.c1[0], pg.c2[0], pg.c1[1], pg.c1[2]);
       o[2] = make_float4(pg.c2[1], pg.c2[2], __uint_as_float((uint32_t)pg.tex), __uint_as_float((uint32_t)((unsigned long long)pg.tex >> 32)));
     }
     if (ACC == ACC_REG && threadIdx.x < 32) {  // x -> mult x + plus = LCG^(2 c k), composed from a.jump
@@ -458,6 +524,7 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
   // x / N for 0 <= x <= 32 as a multiply-shift (exact for N <= 1024; beyond that x / N is 0 or 1)
   auto div_n = [&](int x) -> int { return cfg.n_magic ? (int)(((unsigned)x * cfg.n_magic) >> 16) : (x >= N ? 1 : 0); };
   const float inv_n = cfg.inv_n, inv_spp = cfg.inv_spp;
+  const int n32 = min(N, 32);
   // rays are counted per task from warp-uniform quantities (every lane holds the same sum)
   unsigned int n_rays = 0;
   bool overflow = false;
@@ -540,9 +607,16 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
           }
           if (ACC == ACC_SEG) seg_start = max(0, slot * L - round * 32);
         } else {
-          const long long avail = (long long)cur_rem + (long long)top * N;
-          if (avail == 0) break;
-          const int take = (int)min(avail, 32ll);
+          int take;
+          if (SMALL) {  // min(cur_rem + top N, 32) in 32 bits: cur_rem < N < 2^31, and min(top, 32) min(N, 32) <= 1024
+            const unsigned avail = (unsigned)cur_rem + (unsigned)min(top, 32) * (unsigned)n32;
+            if (avail == 0u) break;
+            take = (int)min(avail, 32u);
+          } else {
+            const long long avail = (long long)cur_rem + (long long)top * N;
+            if (avail == 0) break;
+            take = (int)min(avail, 32ll);
+          }
           active = lane < take;
           task_rays += (unsigned)take;
           // the first `from_cur` lanes finish the partly consumed record, the others take whole records
@@ -577,7 +651,7 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
             if (ERR) { rslot = slot; slot = (int)(((unsigned)rslot * ea.err_magic) >> 16); }  // the batch's pixel in the task
             depth = (meta >> 6) & 1023;
             origin = (int)((unsigned)meta >> 16);
-            if (origin == 0xFFFF) origin = -1;
+            if (!SMALL && origin == 0xFFFF) origin = -1;  // (closest_small: 0xFFFF matches no shape index)
             thr = mk3<float>(rec.b.w, rec.c.x, rec.c.y);
             const uint64_t base = ((uint64_t)__float_as_uint(rec.c.w) << 32) | (uint64_t)__float_as_uint(rec.c.z);
             rng.state = child_stream(base, child);
@@ -588,7 +662,7 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
             if (((meta >> 5) & 1) == RT_BRDF_DIFFUSE) {
               const float u1 = unit_from_u32((uint32_t)(rng.state >> 32));  // the two halves of the child's stream value
               const float u2 = unit_from_u32((uint32_t)rng.state);
-              ray.d = diffuse_dir<float>(nd, u1, u2);
+              ray.d = SMALL ? diffuse_dir_small(pk2(nd.x, nd.y), nd.z, u1, u2) : diffuse_dir<float>(nd, u1, u2);
               ray.tmin = 1.0e-3f;
             } else {
               ray.d = nd;
@@ -638,7 +712,7 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
               else return rows_at((inverse ? sc.invm : sc.m) + 12 * (size_t)best);
             };
             auto pig_uniform = [&](int idx) -> V3<float> {
-              if (SMALL) { const float4 q = lds4c(sb + SM_PIG + idx * SM_PIG_STRIDE + 16); return mk3<float>(q.x, q.y, q.z); }
+              if (SMALL) { const float4 q = lds4c(sb + SM_PIG + idx * SM_PIG_STRIDE + 16); return mk3<float>(q.x, q.z, q.w); }
               return pig_c1<float>(sc.pigments[idx]);
             };
             auto pig_at = [&](int idx, float u, float v) -> V3<float> {
@@ -651,7 +725,7 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
               // the BRDF colour can change the result: emitted radiance only
               if (!(mf & MAT_EMIT_BLACK)) {
                 if (mf & MAT_UV_EMIT) local_uv<float>(local_hit_rows(rows_of(true), ray, best_t), sphere, u, v);
-                contrib = mul3(thr, (mf & MAT_UV_EMIT) ? pig_at(emit_pig, u, v) : pig_uniform(emit_pig));
+                contrib = mul3_k<SMALL>(thr, (mf & MAT_UV_EMIT) ? pig_at(emit_pig, u, v) : pig_uniform(emit_pig));
               }
             } else {
               const bool scatters = !(mf & MAT_NO_SCATTER);
@@ -659,7 +733,7 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
               if (scatters || (mf & MAT_USES_UV)) { im = rows_of(true); lh = local_hit_rows(im, ray, best_t); }
               if (mf & MAT_USES_UV) local_uv<float>(lh, sphere, u, v);
               if (!(mf & MAT_EMIT_BLACK))
-                contrib = mul3(thr, (mf & MAT_UV_EMIT) ? pig_at(emit_pig, u, v) : pig_uniform(emit_pig));
+                contrib = mul3_k<SMALL>(thr, (mf & MAT_UV_EMIT) ? pig_at(emit_pig, u, v) : pig_uniform(emit_pig));
               if (scatters) {
                 V3<float> hit_color = (mf & MAT_UV_BRDF) ? pig_at(brdf_pig, u, v) : pig_uniform(brdf_pig);
                 const float lum = max3(hit_color);
@@ -671,12 +745,25 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
                 }
                 if (go_on && lum > 0.f) {
                   push = true;
-                  V3<float> point, normal;
-                  // (SMALL reloads the inverse: held across the shading above, its 12 registers made ptxas spill
-                  // loop state at the 80-register cap)
-                  world_frame_rows(SMALL ? rows_of(true) : im, rows_of(false), lh, sphere, point, normal);
-                  const V3<float> nd = (brdf_kind == RT_BRDF_DIFFUSE) ? normal : specular_dir<float>(ray.d, normal);
-                  const V3<float> w = inv_n * mul3(thr, hit_color);
+                  V3<float> point, nd, w;
+                  if constexpr (SMALL) {
+                    // (the inverse is read again here: held across the shading above, its registers made ptxas spill
+                    // loop state at the 80-register cap)
+                    f32x2 nxy, dxy = 0ull;
+                    float nz, dz = 0.f;
+                    world_frame_small(sb + SM_INVM + 48 * best, sb + SM_INVT + 16 * best, rows_of(false), lh, sphere, point, nxy, nz);
+                    if (brdf_kind == RT_BRDF_DIFFUSE) { dxy = nxy; dz = nz; }
+                    else specular_dir_small(ray.d, nxy, nz, dxy, dz);
+                    upk2(dxy, nd.x, nd.y);
+                    nd.z = dz;
+                    w.x = inv_n * (thr.x * hit_color.x);
+                    upk2(mul2(bc2(inv_n), mul2(pk2(thr.y, thr.z), pk2(hit_color.y, hit_color.z))), w.y, w.z);
+                  } else {
+                    V3<float> normal;
+                    world_frame_rows(im, rows_of(false), lh, sphere, point, normal);
+                    nd = (brdf_kind == RT_BRDF_DIFFUSE) ? normal : specular_dir<float>(ray.d, normal);
+                    w = inv_n * mul3(thr, hit_color);
+                  }
                   out.a = make_float4(point.x, point.y, point.z,
                                       __int_as_float((ERR ? rslot : slot) | (brdf_kind << 5) | ((depth + 1) << 6) |
                                                      ((best < 0xFFFF ? best : 0xFFFF) << 16)));
@@ -711,6 +798,9 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
             float* col = acc + (3 * slot) * 32 + lane;
             col[0] += contrib.x; col[32] += contrib.y; col[64] += contrib.z;
           }
+        } else if constexpr (SMALL) {
+          sr += contrib.x;
+          upk2(add2(pk2(sg, sb_), pk2(contrib.y, contrib.z)), sg, sb_);
         } else {
           sr += contrib.x; sg += contrib.y; sb_ += contrib.z;
         }
