@@ -298,6 +298,24 @@ typedef struct rt_adaptive_stats {
 /* out_rgb float[H][W][3] mean; out_err float[H][W][3] SE (optional); out_samples int32[H][W] (optional) */
 int rt_render_adaptive(rt_scene* scene, const rt_render_params* params, const rt_adaptive_params* ap,
                        float* out_rgb, float* out_err, int32_t* out_samples, rt_adaptive_stats* stats);
+/* The same passes, scheduled by a sample budget B = sample_budget (total samples) instead of a threshold.  Passes,
+ * PCG states, the pass values, the reported mean / SE / samples and estimator mean what they mean above; M =
+ * ap->max_passes (>= 1); target_error >= 0 (finite) only says which pixels may be traced again.
+ *   Pass 0 traces every pixel and needs B >= W*H*S^2.  Each pixel holds its e = max_c SE_c / max(mean_c,
+ *   error_floor) (the fp32 value the threshold mode compares) from the last pass that traced it; the candidates
+ *   are the pixels with e > target_error (target 0: every pixel with any error).  After pass p, if p + 1 < M, with
+ *   Q = floor((B - samples spent) / S^2), C = the number of candidates and r = M - 1 - p, the next pass traces
+ *       K = min(C, Q, max(ceil(C / 2), ceil(Q / r)))
+ *   pixels: the first K in the order (e descending, pixel index ascending), listed in ascending pixel order.  The
+ *   call stops when K = 0 or after M passes.  A pixel may skip passes; pass p of a pixel is always that pixel of
+ *   the (p+1)-th fire_all_rays.
+ * So every pass after the first traces at least half of the candidates the budget allows, the last allowed pass
+ * spends what is left, no pixel gets more than M*S^2 samples, and stats->samples <= B with B - samples < S^2
+ * unless the candidates ran out first.  The same scope as rt_render_adaptive, plus B >= W*H*S^2 and a finite
+ * target_error >= 0; anything else is RT_ERR_INVALID. */
+int rt_render_adaptive_budget(rt_scene* scene, const rt_render_params* params, const rt_adaptive_params* ap,
+                              int64_t sample_budget, float* out_rgb, float* out_err, int32_t* out_samples,
+                              rt_adaptive_stats* stats);
 
 /* ---- Renderer.__call__(ray) for explicit rays (render.py:52,65,99,157) ----
  * rays: double[n][8] = origin xyz, dir xyz, tmin, tmax; depth int32[n] (NULL = 0).

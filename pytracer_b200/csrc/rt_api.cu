@@ -743,27 +743,32 @@ static uint64_t lcg_advance(uint64_t state, uint64_t inc, uint64_t delta) {
   return acc_mult * state + acc_plus;
 }
 
-// Path tracing with an error map and noise-targeted passes (rt_api.h).  Every per-pixel quantity stays on
-// the device for the whole call: pass p runs the error-map path tracer over the current pixel list (pass 0:
-// the image), rt_adaptive.cu folds its means and SE^2 into the per-pixel sums and writes the next list;
-// the host reads one count per pass.
-extern "C" int rt_render_adaptive(rt_scene* s, const rt_render_params* p, const rt_adaptive_params* ap, float* out_rgb, float* out_err,
-                                  int32_t* out_samples, rt_adaptive_stats* stats) {
-  if (!s || !p || !ap || !out_rgb) return fail(RT_ERR_INVALID, "rt_render_adaptive: null argument");
-  if (p->algorithm != RT_ALGO_PATHTRACING) return fail(RT_ERR_INVALID, "rt_render_adaptive: path tracing only");
-  if (p->samples_per_side < 2) return fail(RT_ERR_INVALID, "rt_render_adaptive: samples_per_side %d (the error map needs >= 2)", p->samples_per_side);
-  if (p->variant != RT_VARIANT_AUTO && p->variant != RT_VARIANT_WARP) return fail(RT_ERR_INVALID, "rt_render_adaptive: the warp variant only");
-  if (p->precision != RT_PRECISION_AUTO && p->precision != RT_PRECISION_F32) return fail(RT_ERR_INVALID, "rt_render_adaptive: fp32 only");
+// Path tracing with an error map and passes over pixel lists (rt_api.h), the pass loop of rt_render_adaptive
+// (budget < 0: noise-targeted passes) and rt_render_adaptive_budget (budget >= 0 samples: the K pixels of largest
+// relative error).  Every per-pixel quantity stays on the device for the whole call: pass p runs the error-map path
+// tracer over the current pixel list (pass 0: the image), rt_adaptive.cu folds its means and SE^2 into the per-pixel
+// sums and writes the next list; the host reads one count per pass.
+static int render_adaptive_passes(const char* fn, rt_scene* s, const rt_render_params* p, const rt_adaptive_params* ap, long long budget,
+                                  float* out_rgb, float* out_err, int32_t* out_samples, rt_adaptive_stats* stats) {
+  if (!s || !p || !ap || !out_rgb) return fail(RT_ERR_INVALID, "%s: null argument", fn);
+  if (p->algorithm != RT_ALGO_PATHTRACING) return fail(RT_ERR_INVALID, "%s: path tracing only", fn);
+  if (p->samples_per_side < 2) return fail(RT_ERR_INVALID, "%s: samples_per_side %d (the error map needs >= 2)", fn, p->samples_per_side);
+  if (p->variant != RT_VARIANT_AUTO && p->variant != RT_VARIANT_WARP) return fail(RT_ERR_INVALID, "%s: the warp variant only", fn);
+  if (p->precision != RT_PRECISION_AUTO && p->precision != RT_PRECISION_F32) return fail(RT_ERR_INVALID, "%s: fp32 only", fn);
   if (p->part_mode != RT_PART_NONE || p->n_peer_images != 0 || p->out_f64 || p->rng_mode != RT_RNG_STREAMS)
-    return fail(RT_ERR_INVALID, "rt_render_adaptive: one device, RT_PART_NONE, RT_RNG_STREAMS, an fp32 image and no peer images");
-  if (p->num_of_rays < 1 || p->max_depth < 0) return fail(RT_ERR_INVALID, "rt_render_adaptive: num_of_rays %d, max_depth %d", p->num_of_rays, p->max_depth);
+    return fail(RT_ERR_INVALID, "%s: one device, RT_PART_NONE, RT_RNG_STREAMS, an fp32 image and no peer images", fn);
+  if (p->num_of_rays < 1 || p->max_depth < 0) return fail(RT_ERR_INVALID, "%s: num_of_rays %d, max_depth %d", fn, p->num_of_rays, p->max_depth);
   if (ap->max_passes < 1 || !(ap->error_floor > 0.0) || std::isnan(ap->target_error))
-    return fail(RT_ERR_INVALID, "rt_render_adaptive: max_passes %d, error_floor %g, target_error %g", ap->max_passes, ap->error_floor, ap->target_error);
+    return fail(RT_ERR_INVALID, "%s: max_passes %d, error_floor %g, target_error %g", fn, ap->max_passes, ap->error_floor, ap->target_error);
   if (ap->estimator != RT_ERR_EST_BATCH && ap->estimator != RT_ERR_EST_PAIRED)
-    return fail(RT_ERR_INVALID, "rt_render_adaptive: estimator %d", ap->estimator);
+    return fail(RT_ERR_INVALID, "%s: estimator %d", fn, ap->estimator);
   if (ap->estimator == RT_ERR_EST_PAIRED && p->samples_per_side % 2)  // a stratum without a partner
-    return fail(RT_ERR_INVALID, "rt_render_adaptive: the paired estimator needs an even samples_per_side (got %d)", p->samples_per_side);
-  if ((long long)p->width * p->height >= (1ll << 31)) return fail(RT_ERR_INVALID, "rt_render_adaptive: image too large");
+    return fail(RT_ERR_INVALID, "%s: the paired estimator needs an even samples_per_side (got %d)", fn, p->samples_per_side);
+  if ((long long)p->width * p->height >= (1ll << 31)) return fail(RT_ERR_INVALID, "%s: image too large", fn);
+  const long long one_pass = (long long)p->width * p->height * p->samples_per_side * p->samples_per_side;
+  if (budget >= 0 && (budget < one_pass || !std::isfinite(ap->target_error) || ap->target_error < 0.0))
+    return fail(RT_ERR_INVALID, "%s: sample_budget %lld (pass 0 needs %lld), target_error %g (finite, >= 0)", fn, budget, one_pass,
+                ap->target_error);
   CU(cudaSetDevice(s->device));
   RenderArgs a;
   int rc = fill_args(s, p, &a);
@@ -771,19 +776,21 @@ extern "C" int rt_render_adaptive(rt_scene* s, const rt_render_params* p, const 
   Workspace* ws = s->ws;
   const int n = p->width * p->height;
   const int S2 = p->samples_per_side * p->samples_per_side;
-  const int max_passes = ap->target_error > 0.0 ? ap->max_passes : 1;
+  const int max_passes = budget >= 0 || ap->target_error > 0.0 ? ap->max_passes : 1;
   if (p->accel != RT_ACCEL_NONE && p->accel != RT_ACCEL_BVH) return fail(RT_ERR_INVALID, "accel %d", p->accel);
   const int accel = (p->accel == RT_ACCEL_BVH && s->n_spheres > 0) ? RT_ACCEL_BVH : RT_ACCEL_NONE;
   cudaStream_t st = 0;
   if (accel == RT_ACCEL_BVH && (rc = ensure_bvh(s, st)) != RT_OK) return rc;
   SceneView<float> v32 = view_of<float>(s);
   v32.accel = accel;
-  // device layout: pass mean / SE^2 per list entry, per-pixel sums and pass counts, two lists, flags, tile counts
+  // device layout: pass mean / SE^2 per list entry, per-pixel sums and pass counts, two lists, flags, tile counts;
+  // budget mode: e per pixel, the radix select's histogram and state
   const size_t n3 = 3 * (size_t)n * sizeof(float), tiles = (size_t)n / 2048 + 2;
   auto al = [](size_t x) { return (x + 255) / 256 * 256; };
   const size_t o_em = 0, o_ev = o_em + al(n3), o_sm = o_ev + al(n3), o_sv = o_sm + al(n3), o_np = o_sv + al(n3);
   const size_t o_l0 = o_np + al((size_t)n * 4), o_l1 = o_l0 + al((size_t)n * 4), o_fl = o_l1 + al((size_t)n * 4);
-  const size_t o_bc = o_fl + al((size_t)n), o_cnt = o_bc + al(tiles * 4), total = o_cnt + 256;
+  const size_t o_bc = o_fl + al((size_t)n), o_cnt = o_bc + al(tiles * 4), o_ee = o_cnt + 256, o_hist = o_ee + al((size_t)n * 4);
+  const size_t o_sel = o_hist + 256 * 4, total = budget >= 0 ? o_sel + al(sizeof(BudgetSelect)) : o_ee;
   if ((rc = ensure(&ws->adaptive, &ws->adaptive_cap, total)) != RT_OK) return rc;
   if (!ws->count_host) CU(cudaMallocHost((void**)&ws->count_host, sizeof(int32_t)));
   unsigned char* base = (unsigned char*)ws->adaptive;
@@ -792,15 +799,19 @@ extern "C" int rt_render_adaptive(rt_scene* s, const rt_render_params* p, const 
   int32_t* lists[2] = {(int32_t*)(base + o_l0), (int32_t*)(base + o_l1)};
   uint8_t* flags = base + o_fl;
   int32_t *block_counts = (int32_t*)(base + o_bc), *d_count = (int32_t*)(base + o_cnt);
+  float* err_e = (float*)(base + o_ee);
+  int32_t* hist = (int32_t*)(base + o_hist);
+  BudgetSelect* sel = (BudgetSelect*)(base + o_sel);
 
   rt_adaptive_stats out;
   memset(&out, 0, sizeof(out));
   LaunchInfo info = {0, RT_VARIANT_WARP};
   CU(cudaEventRecord(ws->t0, st));
   CU(cudaMemsetAsync(ws->counters, 0, CNT_SLOTS * sizeof(unsigned long long), st));
+  if (budget >= 0) CU(cudaMemsetAsync(hist, 0, o_sel + sizeof(BudgetSelect) - o_hist, st));
   CU(cudaEventRecord(ws->ev0, st));
   const uint64_t draws_per_image = 2ull * (uint64_t)n * (uint64_t)S2;
-  long long n_cur = n;
+  long long n_cur = n, spent = 0;
   int passes = 0;
   for (int pass = 0; pass < max_passes && n_cur > 0; ++pass) {
     // pass p = the (p+1)-th consecutive image: ImageTracer.pcg after p images, PathTracer.pcg after p random() calls
@@ -816,10 +827,18 @@ extern "C" int rt_render_adaptive(rt_scene* s, const rt_render_params* p, const 
     CU(cudaMemsetAsync(ws->counters + CNT_TASK, 0, sizeof(unsigned long long), st));
     const char* why = nullptr;
     cudaError_t err = launch_pt_warp_err(v32, a, e, st, s->sm_count, &info, &why, s->bvh_n_nodes, s->bvh_n_prims, s->bvh_depth);
-    if (err != cudaSuccess) return fail(why ? RT_ERR_INVALID : RT_ERR_CUDA, "rt_render_adaptive: %s", why ? why : cudaGetErrorString(err));
-    err = launch_adaptive_combine(e, pass, max_passes, (float)ap->target_error, (float)ap->error_floor, sm, sv, n_pass, flags, block_counts,
-                                  d_count, lists[(pass + 1) & 1], n, st, &info);
-    if (err != cudaSuccess) return fail(RT_ERR_CUDA, "rt_render_adaptive: %s", cudaGetErrorString(err));
+    if (err != cudaSuccess) return fail(why ? RT_ERR_INVALID : RT_ERR_CUDA, "%s: %s", fn, why ? why : cudaGetErrorString(err));
+    spent += n_cur * S2;
+    if (budget < 0) {
+      err = launch_adaptive_combine(e, pass, max_passes, (float)ap->target_error, (float)ap->error_floor, sm, sv, n_pass, flags, block_counts,
+                                    d_count, lists[(pass + 1) & 1], n, st, &info);
+    } else {
+      err = launch_adaptive_combine_budget(e, pass, (float)ap->error_floor, sm, sv, n_pass, err_e, n, st, &info);
+      if (err == cudaSuccess && pass + 1 < max_passes)  // Q = what the rest of the budget buys, in pixel passes; r = passes left
+        err = launch_adaptive_select_budget(err_e, n, (float)ap->target_error, (budget - spent) / S2, max_passes - 1 - pass, sel, hist, flags,
+                                            block_counts, d_count, lists[(pass + 1) & 1], s->sm_count, st, &info);
+    }
+    if (err != cudaSuccess) return fail(RT_ERR_CUDA, "%s: %s", fn, cudaGetErrorString(err));
     if (pass < 16) out.pixels_in_pass[pass] = n_cur;
     passes = pass + 1;
     if (pass + 1 < max_passes) {  // the one host read of the pass: how many pixels the next pass traces
@@ -829,7 +848,7 @@ extern "C" int rt_render_adaptive(rt_scene* s, const rt_render_params* p, const 
     }
   }
   cudaError_t err = launch_adaptive_final(sm, sv, n_pass, S2, n, em, out_err ? ev : nullptr, out_samples ? lists[0] : nullptr, st, &info);
-  if (err != cudaSuccess) return fail(RT_ERR_CUDA, "rt_render_adaptive: %s", cudaGetErrorString(err));
+  if (err != cudaSuccess) return fail(RT_ERR_CUDA, "%s: %s", fn, cudaGetErrorString(err));
   CU(cudaEventRecord(ws->ev1, st));
   CU(cudaMemcpyAsync(out_rgb, em, n3, cudaMemcpyDeviceToHost, st));
   if (out_err) CU(cudaMemcpyAsync(out_err, ev, n3, cudaMemcpyDeviceToHost, st));
@@ -849,6 +868,17 @@ extern "C" int rt_render_adaptive(rt_scene* s, const rt_render_params* p, const 
   if (stats) *stats = out;
   if (out.overflow) return fail(RT_ERR_OVERFLOW, "a warp work stack overflowed; the image is invalid");
   return RT_OK;
+}
+
+extern "C" int rt_render_adaptive(rt_scene* s, const rt_render_params* p, const rt_adaptive_params* ap, float* out_rgb, float* out_err,
+                                  int32_t* out_samples, rt_adaptive_stats* stats) {
+  return render_adaptive_passes("rt_render_adaptive", s, p, ap, -1, out_rgb, out_err, out_samples, stats);
+}
+
+extern "C" int rt_render_adaptive_budget(rt_scene* s, const rt_render_params* p, const rt_adaptive_params* ap, int64_t sample_budget,
+                                         float* out_rgb, float* out_err, int32_t* out_samples, rt_adaptive_stats* stats) {
+  if (sample_budget < 0) return fail(RT_ERR_INVALID, "rt_render_adaptive_budget: sample_budget %lld", (long long)sample_budget);
+  return render_adaptive_passes("rt_render_adaptive_budget", s, p, ap, sample_budget, out_rgb, out_err, out_samples, stats);
 }
 
 // ------------------------------------------------------------------------------------ probes

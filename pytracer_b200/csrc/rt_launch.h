@@ -60,6 +60,22 @@ cudaError_t launch_pt_warp_err(const SceneView<float>& sc, const RenderArgs& a, 
 cudaError_t launch_adaptive_combine(const ErrArgs& e, int pass, int max_passes, float target, float floor_, float* sum_m, float* sum_v,
                                     int32_t* n_pass, uint8_t* flags, int32_t* block_counts, int32_t* d_count, int32_t* next_list, int n_pixels,
                                     cudaStream_t st, LaunchInfo* info);
+// rt_adaptive.cu, sample-budget mode: the radix select's state between its kernels (device memory, zeroed once a call)
+struct BudgetSelect {
+  unsigned prefix;  // digits of the K-th largest key T picked so far (after the last digit: T)
+  int k_rem;        // rank of T among the keys with this prefix (after the last digit: the ties with key T to take)
+  int K, C;         // pixels the next pass traces, candidates (e > target)
+  int scratch;      // total of the tie-offset scan
+  int pad_[3];
+};
+// fold a pass into the per-pixel sums and store e of every traced pixel in err_e
+cudaError_t launch_adaptive_combine_budget(const ErrArgs& e, int pass, float floor_, float* sum_m, float* sum_v, int32_t* n_pass,
+                                           float* err_e, int n_pixels, cudaStream_t st, LaunchInfo* info);
+// list the K = min(C, Q, max(ceil(C/2), ceil(Q/r))) pixels of largest e (ties: lower pixel index first) in next_list, in
+// ascending order, and K in *d_count; Q = passes of one pixel the budget still pays for, r = passes left; hist: 256 zeros
+cudaError_t launch_adaptive_select_budget(const float* err_e, int n_pixels, float target, long long Q, int r, BudgetSelect* sel,
+                                          int32_t* hist, uint8_t* flags, int32_t* block_counts, int32_t* d_count, int32_t* next_list,
+                                          int sm_count, cudaStream_t st, LaunchInfo* info);
 cudaError_t launch_adaptive_final(const float* sum_m, const float* sum_v, const int32_t* n_pass, int spp, int n_pixels, float* rgb, float* err,
                                   int32_t* samples, cudaStream_t st, LaunchInfo* info);
 

@@ -76,7 +76,8 @@ class ImageTracer:
 
     def fire_all_rays_adaptive(self, renderer, target_error: float = 0.0, max_samples_per_pixel: Optional[int] = None,
                                error_floor: float = 1e-2, callback=None, callback_time_s: float = 2.0,
-                               error_estimator: str = "batch", **callback_kwargs) -> AdaptiveResult:
+                               error_estimator: str = "batch", mean_samples_per_pixel: Optional[int] = None,
+                               **callback_kwargs) -> AdaptiveResult:
         """Path-traced image with a per-pixel Monte Carlo error map, optionally refined where it is noisy.
 
         Pass 0 is exactly ``fire_all_rays(renderer)``; every further pass traces ``samples_per_side ** 2`` more
@@ -87,7 +88,13 @@ class ImageTracer:
         ``self.pcg`` and ``renderer.pcg`` are left where ``passes`` consecutive ``fire_all_rays`` leave them.
         ``error_estimator`` forms each pass's SE from the stratified samples: "batch" treats them as independent
         (conservative); "paired" collapses pairs of horizontally adjacent strata, which credits stratification
-        and so reports less where radiance is smooth within the pixel (even ``samples_per_side`` only)."""
+        and so reports less where radiance is smooth within the pixel (even ``samples_per_side`` only).
+
+        With ``mean_samples_per_pixel`` the call spends a fixed budget of that many samples per pixel on average
+        (mean x width x height in all, the first pass included) instead of a threshold: after pass 0 every pass traces
+        the pixels of largest relative error above ``target_error`` (0: any error), at least half of them while the
+        budget lasts, until the budget or ``max_samples_per_pixel`` (then required: at least the mean and a multiple
+        of ``samples_per_side ** 2``) runs out; include/rt_api.h (rt_render_adaptive_budget) states the rule."""
         spp = self.samples_per_side ** 2
         if not isinstance(renderer, CudaRenderer) or renderer.algorithm != "pathtracing":
             raise ValueError("fire_all_rays_adaptive needs a path-tracing CudaRenderer")
@@ -105,6 +112,13 @@ class ImageTracer:
             raise ValueError(f"error_estimator must be one of {sorted(_abi.ERROR_ESTIMATORS)} (got {error_estimator!r})")
         if error_estimator == "paired" and self.samples_per_side % 2:
             raise ValueError(f"the paired error estimator needs an even samples_per_side (got {self.samples_per_side})")
+        if mean_samples_per_pixel is not None:
+            if int(mean_samples_per_pixel) != mean_samples_per_pixel or mean_samples_per_pixel < spp:
+                raise ValueError(f"mean_samples_per_pixel ({mean_samples_per_pixel}) must be an integer of at least the "
+                                 f"samples of the first pass ({spp})")
+            if max_samples_per_pixel is None or max_samples_per_pixel < mean_samples_per_pixel:
+                raise ValueError(f"mean_samples_per_pixel needs max_samples_per_pixel >= the mean ({mean_samples_per_pixel}; "
+                                 f"got {max_samples_per_pixel})")
         if max_samples_per_pixel is None:
             max_samples_per_pixel = spp
         if int(max_samples_per_pixel) != max_samples_per_pixel or max_samples_per_pixel < spp or max_samples_per_pixel % spp:
@@ -116,8 +130,14 @@ class ImageTracer:
         if callback:
             callback(col=0, row=0, **callback_kwargs)
         scene = renderer.device_scene()
-        rgb, err, samples, stats = scene.render_adaptive(self._params(renderer), target_error, max_passes, error_floor,
-                                                         out=self._adoptable_buffer(), estimator=error_estimator)
+        if mean_samples_per_pixel is None:
+            rgb, err, samples, stats = scene.render_adaptive(self._params(renderer), target_error, max_passes, error_floor,
+                                                             out=self._adoptable_buffer(), estimator=error_estimator)
+        else:
+            budget = int(mean_samples_per_pixel) * self.image.width * self.image.height
+            rgb, err, samples, stats = scene.render_budget(self._params(renderer), budget, max_passes, target_error, error_floor,
+                                                           out=self._adoptable_buffer(), estimator=error_estimator)
+            stats["sample_budget"] = budget
         passes = stats["passes"]
         self.last_stats = renderer.last_stats = stats
         for _ in range(passes):  # where `passes` consecutive fire_all_rays leave both generators
