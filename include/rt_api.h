@@ -316,6 +316,30 @@ int rt_render_adaptive(rt_scene* scene, const rt_render_params* params, const rt
 int rt_render_adaptive_budget(rt_scene* scene, const rt_render_params* params, const rt_adaptive_params* ap,
                               int64_t sample_budget, float* out_rgb, float* out_err, int32_t* out_samples,
                               rt_adaptive_stats* stats);
+/* The same passes, scheduled by a ray budget R = ray_budget (>= 0): closest-hit rays, the quantity
+ * stats->rays_closest counts.  Passes, PCG states, the pass values, the reported mean / SE / samples and estimator
+ * mean what they mean above; M = ap->max_passes (>= 1); target_error >= 0 (finite) and error_floor as in the
+ * sample-budget mode.
+ *   Pass 0 traces every pixel, whatever R is.  Each pixel holds, from the last pass that traced it, its pass count P,
+ *   its e (as above) and n = the closest-hit rays traced for it over all its passes.  Its predicted cost of one more
+ *   pass is w = ceil(n / P) (>= S^2: every sample traces its primary ray).  A candidate (e > target_error) has the key
+ *       fmaxf(__fdiv_rn(e, __fsqrt_rn(__fmul_rn((float)(P + 1), (float)w))), FLT_MIN)   (= e / sqrt((P + 1) w))
+ *   which ranks by e^2 / ((P + 1) w), the drop in relative variance one more pass buys per predicted ray; FLT_MIN
+ *   (a normal number: flush-to-zero cannot drop it) keeps every candidate's key above a non-candidate's 0.  After pass
+ *   p, if p + 1 < M, with R_left = R - the closest-hit rays spent so far (read on the device; R_left <= 0: an empty
+ *   pass), W_c = the sum of w over the candidates and r = M - 1 - p, the spend target is
+ *       T = min(R_left, max(ceil(W_c / 2), ceil(R_left / r)))
+ *   and the next pass traces the longest prefix of the order (key descending, pixel index ascending) whose sum of w
+ *   is <= T, listed in ascending pixel order.  The call stops when that prefix is empty or after M passes.
+ * So every pass after the first has a predicted cost within what is left of the budget, and while the budget lasts
+ * covers at least half of the candidates' predicted cost less one pixel's; no pixel gets more than M*S^2 samples;
+ * and the rays spent exceed R only by how far passes' actual rays exceeded their prediction, or because pass 0 alone
+ * costs more than R.  out_rays int64[H][W] (optional): the closest-hit rays each pixel received (they sum to
+ * stats->rays_closest).  The same scope as rt_render_adaptive, plus R >= 0 and a finite target_error >= 0; anything
+ * else is RT_ERR_INVALID. */
+int rt_render_adaptive_rays(rt_scene* scene, const rt_render_params* params, const rt_adaptive_params* ap,
+                            int64_t ray_budget, float* out_rgb, float* out_err, int32_t* out_samples, int64_t* out_rays,
+                            rt_adaptive_stats* stats);
 
 /* ---- Renderer.__call__(ray) for explicit rays (render.py:52,65,99,157) ----
  * rays: double[n][8] = origin xyz, dir xyz, tmin, tmax; depth int32[n] (NULL = 0).

@@ -37,6 +37,8 @@ _PROTOTYPES = {
                                      C.POINTER(_abi.rt_adaptive_stats)]),
     "rt_render_adaptive_budget": (C.c_int, [_P, C.POINTER(_abi.rt_render_params), C.POINTER(_abi.rt_adaptive_params), C.c_int64, _P,
                                             _P, _P, C.POINTER(_abi.rt_adaptive_stats)]),
+    "rt_render_adaptive_rays": (C.c_int, [_P, C.POINTER(_abi.rt_render_params), C.POINTER(_abi.rt_adaptive_params), C.c_int64, _P,
+                                          _P, _P, _P, C.POINTER(_abi.rt_adaptive_stats)]),
     "rt_trace_rays": (C.c_int, [_P, C.POINTER(_abi.rt_render_params), _P, _P, C.c_int32, _P, _P]),
     "rt_intersect": (C.c_int, [_P, C.c_int32, C.c_int32, _P, C.c_int32, _P]),
     "rt_is_point_visible": (C.c_int, [_P, C.c_int32, _P, C.c_int32, _P]),

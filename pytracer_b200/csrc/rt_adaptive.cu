@@ -9,6 +9,7 @@
 //             counts, one ordered scan of the counts, then every tile writes its pixels at its offset)
 //   final     mean = sum_m / P, SE = sqrt(sum_v) / P, samples = P * S^2 for every pixel
 #include <algorithm>
+#include <cfloat>
 
 #include "rt_launch.h"
 
@@ -16,19 +17,19 @@
 #define RT_AD_ITEMS 8                              // consecutive list entries per thread
 #define RT_AD_TILE (RT_AD_THREADS * RT_AD_ITEMS)
 
-// exclusive block-wide scan of one int per thread (RT_AD_THREADS threads); returns the block total in *total
-__device__ int block_exclusive_scan(int v, int* total) {
-  __shared__ int warp_sums[RT_AD_THREADS / 32];
+// exclusive block-wide scan of one value per thread (RT_AD_THREADS threads); returns the block total in *total
+template <typename T> __device__ T block_exclusive_scan(T v, T* total) {
+  __shared__ T warp_sums[RT_AD_THREADS / 32];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  int x = v;
+  T x = v;
 #pragma unroll
   for (int d = 1; d < 32; d <<= 1) {
-    const int y = __shfl_up_sync(0xffffffffu, x, d);
+    const T y = __shfl_up_sync(0xffffffffu, x, d);
     if (lane >= d) x += y;
   }
   if (lane == 31) warp_sums[warp] = x;
   __syncthreads();
-  int before = 0, all = 0;
+  T before = 0, all = 0;
   for (int w = 0; w < RT_AD_THREADS / 32; ++w) {
     if (w < warp) before += warp_sums[w];
     all += warp_sums[w];
@@ -124,20 +125,20 @@ __global__ void k_adaptive_final(const float* sum_m, const float* sum_v, const i
   }
 }
 
-// ---- sample-budget mode (rt_render_adaptive_budget): the next pass traces the K pixels of largest e
-//   combine   as above, and e of every listed pixel goes to err_e[px] (a pixel keeps its e until traced again)
-//   select    key = e > target ? bits(e) : 0 (e >= 0, so bits order like e); C = #keys > 0; K from C, Q and r on
-//             the device; the K-th largest key T by a radix select over four 8-bit digits (integer histograms,
-//             one block per digit picks the bucket); then every pixel with key > T and the first K - #(key > T)
-//             pixels with key == T in index order (ordered tie ranks: per-tile counts, one ordered scan) are
-//             flagged and compacted like the threshold mode's flags
-__global__ void __launch_bounds__(RT_AD_THREADS)
-k_adaptive_combine_budget(const int32_t* list, int n, const float* em, const float* ev, int pass, float floor_, float* sum_m,
-                          float* sum_v, int32_t* n_pass, float* err_e) {
-  const int i = blockIdx.x * RT_AD_THREADS + threadIdx.x;
-  if (i >= n) return;
-  const int px = list ? list[i] : i;
-  float sm[3], sv[3];
+// ---- budget modes (rt_render_adaptive_budget, rt_render_adaptive_rays): the next pass traces the longest prefix of the
+// order (key descending, pixel index ascending) over the candidates (key > 0) whose weight fits the pass's target T
+//   combine   as above, and per listed pixel (a pixel keeps what it has until traced again):
+//               samples  err_e[px] = e; key = e > target ? bits(e) : 0, weight 1
+//               rays     n_rays[px] += the pass's rays, weight[px] = w = ceil(n_rays / P), err_e[px] = the key as a float
+//                        (e > target ? max(e / sqrt((P + 1) w), FLT_MIN) : 0); the selection then takes target 0
+//   select    W = the candidates' weight and T from W, the budget left and r on the device; a radix select over four
+//             8-bit digits finds the key at which the prefix is cut (64-bit weight histograms; one block per digit picks
+//             the bucket where the weight from the top passes what is left); then every pixel with a larger key is
+//             flagged, and the pixels with that key in index order while their inclusive weight stays within what is
+//             left (ordered: per-tile weights, one ordered scan), and compacted like the threshold mode's flags
+// sum_m, sum_v and n_pass of list entry i (pixel px) after the pass; the new sums in sm, sv; returns P
+__device__ __forceinline__ int combine_entry(int i, int px, const float* em, const float* ev, int pass, float* sum_m, float* sum_v,
+                                             int32_t* n_pass, float* sm, float* sv) {
   int P;
   if (pass == 0) {
     for (int c = 0; c < 3; ++c) { sm[c] = em[3 * (size_t)i + c]; sv[c] = ev[3 * (size_t)i + c]; }
@@ -151,112 +152,178 @@ k_adaptive_combine_budget(const int32_t* list, int n, const float* em, const flo
   }
   for (int c = 0; c < 3; ++c) { sum_m[3 * (size_t)px + c] = sm[c]; sum_v[3 * (size_t)px + c] = sv[c]; }
   n_pass[px] = P;
+  return P;
+}
+
+__global__ void __launch_bounds__(RT_AD_THREADS)
+k_adaptive_combine_budget(const int32_t* list, int n, const float* em, const float* ev, int pass, float floor_, float* sum_m,
+                          float* sum_v, int32_t* n_pass, float* err_e) {
+  const int i = blockIdx.x * RT_AD_THREADS + threadIdx.x;
+  if (i >= n) return;
+  const int px = list ? list[i] : i;
+  float sm[3], sv[3];
+  const int P = combine_entry(i, px, em, ev, pass, sum_m, sum_v, n_pass, sm, sv);
   err_e[px] = adaptive_rel_error(sm, sv, P, floor_);
+}
+
+__global__ void __launch_bounds__(RT_AD_THREADS)
+k_adaptive_combine_rays(const int32_t* list, int n, const float* em, const float* ev, const int32_t* rays, int pass, float target,
+                        float floor_, float* sum_m, float* sum_v, int32_t* n_pass, long long* n_rays, int32_t* weight, float* err_e) {
+  const int i = blockIdx.x * RT_AD_THREADS + threadIdx.x;
+  if (i >= n) return;
+  const int px = list ? list[i] : i;
+  float sm[3], sv[3];
+  const int P = combine_entry(i, px, em, ev, pass, sum_m, sum_v, n_pass, sm, sv);
+  const long long nr = (pass == 0 ? 0ll : n_rays[px]) + rays[i];
+  n_rays[px] = nr;
+  const long long w = (nr + P - 1) / P;  // <= the most rays one pass of the pixel cost: fits an int32
+  weight[px] = (int32_t)w;
+  const float e = adaptive_rel_error(sm, sv, P, floor_);
+  // e^2 / ((P + 1) w): the drop in relative variance one more pass buys, per predicted ray; FLT_MIN (normal, so no
+  // flush to zero drops it) keeps every candidate's key above 0
+  err_e[px] = e > target ? fmaxf(__fdiv_rn(e, __fsqrt_rn(__fmul_rn((float)(P + 1), (float)w))), FLT_MIN) : 0.f;
 }
 
 __device__ __forceinline__ unsigned budget_key(float e, float target) { return e > target ? __float_as_uint(e) : 0u; }
 
-// histogram of digit `digit` (bits 8 digit .. 8 digit + 7) of the candidate keys whose higher digits equal the prefix
-// picked so far; lanes with the same bin are aggregated before the shared atomic
+// weighted histogram of digit `digit` (bits 8 digit .. 8 digit + 7) of the candidate keys whose higher digits equal the
+// prefix picked so far; lanes with the same bin are aggregated before the shared atomic
 __global__ void __launch_bounds__(RT_AD_THREADS)
-k_budget_hist(const float* err_e, int n, float target, int digit, const BudgetSelect* sel, int32_t* hist) {
-  __shared__ int h[256];
-  if (digit < 3 && sel->k_rem == 0) return;  // K = 0: nothing to select
+k_budget_hist(const float* err_e, const int32_t* weight, int n, float target, int digit, const BudgetSelect* sel,
+              unsigned long long* hist) {
+  __shared__ unsigned long long h[256];
+  if (digit < 3 && sel->rem < 0) return;  // the top digit decided: no cut to find
   const unsigned hi_mask = digit == 3 ? 0u : 0xFFFFFFFFu << (8 * (digit + 1));
   const unsigned want = sel->prefix & hi_mask;
+  const int lane = threadIdx.x & 31;
   h[threadIdx.x] = 0;
   __syncthreads();
   for (int base = blockIdx.x * RT_AD_THREADS; base < n; base += gridDim.x * RT_AD_THREADS) {
     const int i = base + threadIdx.x;
     int bin = -1;
+    unsigned w = 0;
     if (i < n) {
       const unsigned key = budget_key(err_e[i], target);
-      if (key && (key & hi_mask) == want) bin = (key >> (8 * digit)) & 255;
+      if (key && (key & hi_mask) == want) {
+        bin = (key >> (8 * digit)) & 255;
+        w = weight ? (unsigned)weight[i] : 1u;
+      }
     }
     const unsigned peers = __match_any_sync(0xffffffffu, bin);
-    if (bin >= 0 && (threadIdx.x & 31) == __ffs(peers) - 1) atomicAdd(&h[bin], __popc(peers));
+    unsigned long long sum = __popc(peers);
+    if (weight) {  // (a kernel parameter: warp-uniform)
+      sum = 0;
+      for (int l = 0; l < 32; ++l) {
+        const unsigned wl = __shfl_sync(0xffffffffu, w, l);
+        if ((peers >> l) & 1u) sum += wl;
+      }
+    }
+    if (bin >= 0 && lane == __ffs(peers) - 1) atomicAdd(&h[bin], sum);
   }
   __syncthreads();
   if (h[threadIdx.x]) atomicAdd(&hist[threadIdx.x], h[threadIdx.x]);
 }
 
-// one block: the bucket of digit `digit` that holds the k_rem-th largest key; at the top digit K comes from
-// C = the number of candidates (all that the histogram counted), Q and r: K = min(C, Q, max(ceil(C/2), ceil(Q/r)))
-__global__ void __launch_bounds__(RT_AD_THREADS) k_budget_pick(int32_t* hist, int digit, long long Q, int r, BudgetSelect* sel) {
+// one block: the bucket of digit `digit` in which the prefix is cut, the one where the weight from the top first exceeds
+// rem; at the top digit the pass's target T = min(left, max(ceil(W/2), ceil(left/r))), W = the candidates' weight (all
+// that the histogram counted), left = budget - *spent (without spent: budget); T = 0 or W <= T needs no cut
+__global__ void __launch_bounds__(RT_AD_THREADS)
+k_budget_pick(unsigned long long* hist, int digit, long long budget, const unsigned long long* spent, int r, BudgetSelect* sel) {
   const int b = 255 - threadIdx.x;  // thread order = buckets from the largest down
-  const int h = hist[b];
+  const long long h = (long long)hist[b];
   hist[b] = 0;  // zero for the next digit or the next pass
-  long long k;
-  if (digit == 3) {
-    k = 0;  // (set below from the block total)
-  } else {
-    k = sel->k_rem;
-    if (k == 0) return;
+  long long rem = 0;
+  if (digit < 3) {
+    rem = sel->rem;
+    if (rem < 0) return;
   }
-  int total;
-  const int above = block_exclusive_scan(h, &total);  // keys in larger buckets
+  long long total;
+  const long long above = block_exclusive_scan(h, &total);  // weight in larger buckets
   if (digit == 3) {
-    const long long C = total;
-    const long long half = (C + 1) / 2, share = (Q + r - 1) / r, wide = half > share ? half : share;
-    k = C < Q ? C : Q;
-    if (wide < k) k = wide;
-    if (threadIdx.x == 0) {
-      sel->C = (int)C;
-      sel->K = (int)k;
-      if (k == 0) { sel->prefix = 0xFFFFFFFFu; sel->k_rem = 0; }  // no key equals or exceeds it: no pixel is flagged
+    const long long W = total, left = spent ? budget - (long long)*spent : budget;
+    long long T = 0;
+    if (left > 0) {
+      const long long half = (W + 1) / 2, share = (left + r - 1) / r;
+      T = left < (half > share ? half : share) ? left : (half > share ? half : share);
     }
-    if (k == 0) return;
+    if (threadIdx.x == 0) {
+      sel->W = W;
+      sel->want = T;
+      // T = 0: no key equals or exceeds the cut, no pixel is flagged; W <= T: every key exceeds it, every candidate is
+      if (T == 0 || W <= T) { sel->prefix = T == 0 ? 0xFFFFFFFFu : 0u; sel->rem = -1; }
+    }
+    if (T == 0 || W <= T) return;
+    rem = T;
   }
-  if (h > 0 && above < k && k <= above + h) {
+  if (above <= rem && rem < above + h) {
     sel->prefix = (digit == 3 ? 0u : sel->prefix) | ((unsigned)b << (8 * digit));
-    sel->k_rem = (int)(k - above);
+    sel->rem = rem - above;
   }
 }
 
-// keys of the tile's RT_AD_ITEMS-per-thread pixels, and how many of the thread's equal T
-__device__ __forceinline__ int budget_tile_keys(const float* err_e, int n, float target, unsigned T, unsigned* key) {
+// keys of the tile's RT_AD_ITEMS-per-thread pixels, and the weight of the thread's pixels whose key equals T
+__device__ __forceinline__ unsigned long long budget_tile_keys(const float* err_e, const int32_t* weight, int n, float target, unsigned T,
+                                                               unsigned* key) {
   const int first = blockIdx.x * RT_AD_TILE + threadIdx.x * RT_AD_ITEMS;
-  int ties = 0;
+  unsigned long long ties = 0;
 #pragma unroll
   for (int k = 0; k < RT_AD_ITEMS; ++k) {
     key[k] = first + k < n ? budget_key(err_e[first + k], target) : 0u;
-    ties += key[k] == T;
+    if (first + k < n && key[k] == T) ties += weight ? (unsigned)weight[first + k] : 1u;
   }
   return ties;
 }
 
-// per tile: the pixels whose key equals T
+// per tile: the weight of the pixels whose key equals T
 __global__ void __launch_bounds__(RT_AD_THREADS)
-k_budget_ties(const float* err_e, int n, float target, const BudgetSelect* sel, int32_t* block_counts) {
+k_budget_ties(const float* err_e, const int32_t* weight, int n, float target, const BudgetSelect* sel, long long* tie_offsets) {
   unsigned key[RT_AD_ITEMS];
-  const int ties = budget_tile_keys(err_e, n, target, sel->prefix, key);
-  int total;
+  const long long ties = (long long)budget_tile_keys(err_e, weight, n, target, sel->prefix, key);
+  long long total;
   block_exclusive_scan(ties, &total);
-  if (threadIdx.x == 0) block_counts[blockIdx.x] = total;
+  if (threadIdx.x == 0) tie_offsets[blockIdx.x] = total;
 }
 
-// flags key > T, and key == T for the ties ranked below k_rem in pixel order (block_counts in: the tiles' tie
-// offsets; out: the tiles' flag counts, as k_adaptive_combine leaves them)
+// one block: as k_adaptive_offsets, in 64 bits
+__global__ void __launch_bounds__(RT_AD_THREADS) k_budget_tie_offsets(long long* tie_offsets, int nb, long long* sum) {
+  long long carry = 0;
+  for (int base = 0; base < nb; base += RT_AD_THREADS) {
+    const int i = base + threadIdx.x;
+    const long long v = i < nb ? tie_offsets[i] : 0;
+    long long total;
+    const long long ex = block_exclusive_scan(v, &total);
+    if (i < nb) tie_offsets[i] = carry + ex;
+    carry += total;
+  }
+  if (threadIdx.x == 0) *sum = carry;
+}
+
+// flags key > T, and key == T in pixel order while the ties' inclusive weight stays <= rem (tie_offsets: the tiles'
+// exclusive tie weights; block_counts out: the tiles' flag counts, as k_adaptive_combine leaves them)
 __global__ void __launch_bounds__(RT_AD_THREADS)
-k_budget_flags(const float* err_e, int n, float target, const BudgetSelect* sel, uint8_t* flags, int32_t* block_counts) {
+k_budget_flags(const float* err_e, const int32_t* weight, int n, float target, const BudgetSelect* sel, const long long* tie_offsets,
+               uint8_t* flags, int32_t* block_counts) {
   const unsigned T = sel->prefix;
-  const int take = sel->k_rem;
-  const int tile_ties = block_counts[blockIdx.x];
+  const long long take = sel->rem;
   unsigned key[RT_AD_ITEMS];
-  const int ties = budget_tile_keys(err_e, n, target, T, key);
-  int total;
-  int rank = tile_ties + block_exclusive_scan(ties, &total);
+  const long long ties = (long long)budget_tile_keys(err_e, weight, n, target, T, key);
+  long long total;
+  long long incl = tie_offsets[blockIdx.x] + block_exclusive_scan(ties, &total);
   const int first = blockIdx.x * RT_AD_TILE + threadIdx.x * RT_AD_ITEMS;
   int count = 0;
 #pragma unroll
   for (int k = 0; k < RT_AD_ITEMS; ++k) {
     bool f = key[k] > T;
-    if (key[k] == T) f = rank++ < take;
+    if (first + k < n && key[k] == T) {
+      incl += weight ? weight[first + k] : 1;
+      f = incl <= take;
+    }
     if (first + k < n) flags[first + k] = f ? 1 : 0;
     count += f;
   }
-  block_exclusive_scan(count, &total);
-  if (threadIdx.x == 0) block_counts[blockIdx.x] = total;
+  int n_flags;
+  block_exclusive_scan(count, &n_flags);
+  if (threadIdx.x == 0) block_counts[blockIdx.x] = n_flags;
 }
 
 cudaError_t launch_adaptive_combine_budget(const ErrArgs& e, int pass, float floor_, float* sum_m, float* sum_v, int32_t* n_pass,
@@ -269,19 +336,30 @@ cudaError_t launch_adaptive_combine_budget(const ErrArgs& e, int pass, float flo
   return cudaGetLastError();
 }
 
-cudaError_t launch_adaptive_select_budget(const float* err_e, int n_pixels, float target, long long Q, int r, BudgetSelect* sel,
-                                          int32_t* hist, uint8_t* flags, int32_t* block_counts, int32_t* d_count, int32_t* next_list,
-                                          int sm_count, cudaStream_t st, LaunchInfo* info) {
+cudaError_t launch_adaptive_combine_rays(const ErrArgs& e, int pass, float target, float floor_, float* sum_m, float* sum_v, int32_t* n_pass,
+                                         long long* n_rays, int32_t* weight, float* err_e, int n_pixels, cudaStream_t st, LaunchInfo* info) {
+  const int n = e.pix_list ? (int)e.n_list : n_pixels;
+  if (n == 0) return cudaSuccess;
+  k_adaptive_combine_rays<<<(n + RT_AD_THREADS - 1) / RT_AD_THREADS, RT_AD_THREADS, 0, st>>>(
+      e.pix_list, n, e.err_mean, e.err_var, e.err_rays, pass, target, floor_, sum_m, sum_v, n_pass, n_rays, weight, err_e);
+  if (info) info->n_launches += 1;
+  return cudaGetLastError();
+}
+
+cudaError_t launch_adaptive_select_budget(const float* err_e, const int32_t* weight, int n_pixels, float target, long long budget,
+                                          const unsigned long long* spent, int r, BudgetSelect* sel, unsigned long long* hist, uint8_t* flags,
+                                          int32_t* block_counts, long long* tie_offsets, int32_t* d_count, int32_t* next_list, int sm_count,
+                                          cudaStream_t st, LaunchInfo* info) {
   const int nb = (n_pixels + RT_AD_TILE - 1) / RT_AD_TILE;
   if (nb == 0) return cudaMemsetAsync(d_count, 0, sizeof(int32_t), st);
   const int hb = std::min((n_pixels + RT_AD_THREADS - 1) / RT_AD_THREADS, std::max(sm_count, 1) * 8);
   for (int digit = 3; digit >= 0; --digit) {
-    k_budget_hist<<<hb, RT_AD_THREADS, 0, st>>>(err_e, n_pixels, target, digit, sel, hist);
-    k_budget_pick<<<1, RT_AD_THREADS, 0, st>>>(hist, digit, Q, r, sel);
+    k_budget_hist<<<hb, RT_AD_THREADS, 0, st>>>(err_e, weight, n_pixels, target, digit, sel, hist);
+    k_budget_pick<<<1, RT_AD_THREADS, 0, st>>>(hist, digit, budget, spent, r, sel);
   }
-  k_budget_ties<<<nb, RT_AD_THREADS, 0, st>>>(err_e, n_pixels, target, sel, block_counts);
-  k_adaptive_offsets<<<1, RT_AD_THREADS, 0, st>>>(block_counts, nb, &sel->scratch);
-  k_budget_flags<<<nb, RT_AD_THREADS, 0, st>>>(err_e, n_pixels, target, sel, flags, block_counts);
+  k_budget_ties<<<nb, RT_AD_THREADS, 0, st>>>(err_e, weight, n_pixels, target, sel, tie_offsets);
+  k_budget_tie_offsets<<<1, RT_AD_THREADS, 0, st>>>(tie_offsets, nb, &sel->scratch);
+  k_budget_flags<<<nb, RT_AD_THREADS, 0, st>>>(err_e, weight, n_pixels, target, sel, tie_offsets, flags, block_counts);
   k_adaptive_offsets<<<1, RT_AD_THREADS, 0, st>>>(block_counts, nb, d_count);
   k_adaptive_scatter<<<nb, RT_AD_THREADS, 0, st>>>(nullptr, n_pixels, flags, block_counts, next_list);
   if (info) info->n_launches += 13;

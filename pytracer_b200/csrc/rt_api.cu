@@ -744,12 +744,15 @@ static uint64_t lcg_advance(uint64_t state, uint64_t inc, uint64_t delta) {
 }
 
 // Path tracing with an error map and passes over pixel lists (rt_api.h), the pass loop of rt_render_adaptive
-// (budget < 0: noise-targeted passes) and rt_render_adaptive_budget (budget >= 0 samples: the K pixels of largest
-// relative error).  Every per-pixel quantity stays on the device for the whole call: pass p runs the error-map path
-// tracer over the current pixel list (pass 0: the image), rt_adaptive.cu folds its means and SE^2 into the per-pixel
-// sums and writes the next list; the host reads one count per pass.
-static int render_adaptive_passes(const char* fn, rt_scene* s, const rt_render_params* p, const rt_adaptive_params* ap, long long budget,
-                                  float* out_rgb, float* out_err, int32_t* out_samples, rt_adaptive_stats* stats) {
+// (ADAPT_THRESHOLD: noise-targeted passes), rt_render_adaptive_budget (ADAPT_SAMPLES: `budget` samples, the pixels of
+// largest relative error first) and rt_render_adaptive_rays (ADAPT_RAYS: `budget` closest-hit rays, the pixels of
+// largest error drop per predicted ray first).  Every per-pixel quantity stays on the device for the whole call: pass p
+// runs the error-map path tracer over the current pixel list (pass 0: the image), rt_adaptive.cu folds its means and
+// SE^2 into the per-pixel sums and writes the next list; the host reads one count per pass.
+enum AdaptiveMode { ADAPT_THRESHOLD, ADAPT_SAMPLES, ADAPT_RAYS };
+static int render_adaptive_passes(const char* fn, rt_scene* s, const rt_render_params* p, const rt_adaptive_params* ap, AdaptiveMode mode,
+                                  long long budget, float* out_rgb, float* out_err, int32_t* out_samples, int64_t* out_rays,
+                                  rt_adaptive_stats* stats) {
   if (!s || !p || !ap || !out_rgb) return fail(RT_ERR_INVALID, "%s: null argument", fn);
   if (p->algorithm != RT_ALGO_PATHTRACING) return fail(RT_ERR_INVALID, "%s: path tracing only", fn);
   if (p->samples_per_side < 2) return fail(RT_ERR_INVALID, "%s: samples_per_side %d (the error map needs >= 2)", fn, p->samples_per_side);
@@ -766,9 +769,11 @@ static int render_adaptive_passes(const char* fn, rt_scene* s, const rt_render_p
     return fail(RT_ERR_INVALID, "%s: the paired estimator needs an even samples_per_side (got %d)", fn, p->samples_per_side);
   if ((long long)p->width * p->height >= (1ll << 31)) return fail(RT_ERR_INVALID, "%s: image too large", fn);
   const long long one_pass = (long long)p->width * p->height * p->samples_per_side * p->samples_per_side;
-  if (budget >= 0 && (budget < one_pass || !std::isfinite(ap->target_error) || ap->target_error < 0.0))
+  if (mode == ADAPT_SAMPLES && (budget < one_pass || !std::isfinite(ap->target_error) || ap->target_error < 0.0))
     return fail(RT_ERR_INVALID, "%s: sample_budget %lld (pass 0 needs %lld), target_error %g (finite, >= 0)", fn, budget, one_pass,
                 ap->target_error);
+  if (mode == ADAPT_RAYS && (budget < 0 || !std::isfinite(ap->target_error) || ap->target_error < 0.0))
+    return fail(RT_ERR_INVALID, "%s: ray_budget %lld (>= 0), target_error %g (finite, >= 0)", fn, budget, ap->target_error);
   CU(cudaSetDevice(s->device));
   RenderArgs a;
   int rc = fill_args(s, p, &a);
@@ -776,7 +781,8 @@ static int render_adaptive_passes(const char* fn, rt_scene* s, const rt_render_p
   Workspace* ws = s->ws;
   const int n = p->width * p->height;
   const int S2 = p->samples_per_side * p->samples_per_side;
-  const int max_passes = budget >= 0 || ap->target_error > 0.0 ? ap->max_passes : 1;
+  const bool budgeted = mode != ADAPT_THRESHOLD, rays = mode == ADAPT_RAYS;
+  const int max_passes = budgeted || ap->target_error > 0.0 ? ap->max_passes : 1;
   if (p->accel != RT_ACCEL_NONE && p->accel != RT_ACCEL_BVH) return fail(RT_ERR_INVALID, "accel %d", p->accel);
   const int accel = (p->accel == RT_ACCEL_BVH && s->n_spheres > 0) ? RT_ACCEL_BVH : RT_ACCEL_NONE;
   cudaStream_t st = 0;
@@ -784,13 +790,16 @@ static int render_adaptive_passes(const char* fn, rt_scene* s, const rt_render_p
   SceneView<float> v32 = view_of<float>(s);
   v32.accel = accel;
   // device layout: pass mean / SE^2 per list entry, per-pixel sums and pass counts, two lists, flags, tile counts;
-  // budget mode: e per pixel, the radix select's histogram and state
+  // budget modes: e (or the key) per pixel, the radix select's histogram, state and tie offsets; ray mode: the pass's rays
+  // per list entry, the rays and the weight per pixel
   const size_t n3 = 3 * (size_t)n * sizeof(float), tiles = (size_t)n / 2048 + 2;
   auto al = [](size_t x) { return (x + 255) / 256 * 256; };
   const size_t o_em = 0, o_ev = o_em + al(n3), o_sm = o_ev + al(n3), o_sv = o_sm + al(n3), o_np = o_sv + al(n3);
   const size_t o_l0 = o_np + al((size_t)n * 4), o_l1 = o_l0 + al((size_t)n * 4), o_fl = o_l1 + al((size_t)n * 4);
   const size_t o_bc = o_fl + al((size_t)n), o_cnt = o_bc + al(tiles * 4), o_ee = o_cnt + 256, o_hist = o_ee + al((size_t)n * 4);
-  const size_t o_sel = o_hist + 256 * 4, total = budget >= 0 ? o_sel + al(sizeof(BudgetSelect)) : o_ee;
+  const size_t o_sel = o_hist + 256 * 8, o_to = o_sel + al(sizeof(BudgetSelect)), o_er = o_to + al(tiles * 8);
+  const size_t o_nr = o_er + al((size_t)n * 4), o_w = o_nr + al((size_t)n * 8);
+  const size_t total = rays ? o_w + al((size_t)n * 4) : budgeted ? o_er : o_ee;
   if ((rc = ensure(&ws->adaptive, &ws->adaptive_cap, total)) != RT_OK) return rc;
   if (!ws->count_host) CU(cudaMallocHost((void**)&ws->count_host, sizeof(int32_t)));
   unsigned char* base = (unsigned char*)ws->adaptive;
@@ -800,15 +809,19 @@ static int render_adaptive_passes(const char* fn, rt_scene* s, const rt_render_p
   uint8_t* flags = base + o_fl;
   int32_t *block_counts = (int32_t*)(base + o_bc), *d_count = (int32_t*)(base + o_cnt);
   float* err_e = (float*)(base + o_ee);
-  int32_t* hist = (int32_t*)(base + o_hist);
+  unsigned long long* hist = (unsigned long long*)(base + o_hist);
   BudgetSelect* sel = (BudgetSelect*)(base + o_sel);
+  long long* tie_offsets = (long long*)(base + o_to);
+  int32_t* err_rays = rays ? (int32_t*)(base + o_er) : nullptr;
+  long long* n_rays = (long long*)(base + o_nr);
+  int32_t* weight = (int32_t*)(base + o_w);
 
   rt_adaptive_stats out;
   memset(&out, 0, sizeof(out));
   LaunchInfo info = {0, RT_VARIANT_WARP};
   CU(cudaEventRecord(ws->t0, st));
   CU(cudaMemsetAsync(ws->counters, 0, CNT_SLOTS * sizeof(unsigned long long), st));
-  if (budget >= 0) CU(cudaMemsetAsync(hist, 0, o_sel + sizeof(BudgetSelect) - o_hist, st));
+  if (budgeted) CU(cudaMemsetAsync(hist, 0, o_sel + sizeof(BudgetSelect) - o_hist, st));
   CU(cudaEventRecord(ws->ev0, st));
   const uint64_t draws_per_image = 2ull * (uint64_t)n * (uint64_t)S2;
   long long n_cur = n, spent = 0;
@@ -824,19 +837,26 @@ static int render_adaptive_passes(const char* fn, rt_scene* s, const rt_render_p
     e.err_mean = em;
     e.err_var = ev;
     e.estimator = ap->estimator;
+    e.err_rays = err_rays;
     CU(cudaMemsetAsync(ws->counters + CNT_TASK, 0, sizeof(unsigned long long), st));
     const char* why = nullptr;
     cudaError_t err = launch_pt_warp_err(v32, a, e, st, s->sm_count, &info, &why, s->bvh_n_nodes, s->bvh_n_prims, s->bvh_depth);
     if (err != cudaSuccess) return fail(why ? RT_ERR_INVALID : RT_ERR_CUDA, "%s: %s", fn, why ? why : cudaGetErrorString(err));
     spent += n_cur * S2;
-    if (budget < 0) {
+    if (mode == ADAPT_THRESHOLD) {
       err = launch_adaptive_combine(e, pass, max_passes, (float)ap->target_error, (float)ap->error_floor, sm, sv, n_pass, flags, block_counts,
                                     d_count, lists[(pass + 1) & 1], n, st, &info);
-    } else {
+    } else if (mode == ADAPT_SAMPLES) {
       err = launch_adaptive_combine_budget(e, pass, (float)ap->error_floor, sm, sv, n_pass, err_e, n, st, &info);
       if (err == cudaSuccess && pass + 1 < max_passes)  // Q = what the rest of the budget buys, in pixel passes; r = passes left
-        err = launch_adaptive_select_budget(err_e, n, (float)ap->target_error, (budget - spent) / S2, max_passes - 1 - pass, sel, hist, flags,
-                                            block_counts, d_count, lists[(pass + 1) & 1], s->sm_count, st, &info);
+        err = launch_adaptive_select_budget(err_e, nullptr, n, (float)ap->target_error, (budget - spent) / S2, nullptr, max_passes - 1 - pass,
+                                            sel, hist, flags, block_counts, tie_offsets, d_count, lists[(pass + 1) & 1], s->sm_count, st, &info);
+    } else {  // the key already holds the target (0 for non-candidates): the selection compares it with 0
+      err = launch_adaptive_combine_rays(e, pass, (float)ap->target_error, (float)ap->error_floor, sm, sv, n_pass, n_rays, weight, err_e, n,
+                                         st, &info);
+      if (err == cudaSuccess && pass + 1 < max_passes)  // what is left of R: R - the rays traced so far, read on the device
+        err = launch_adaptive_select_budget(err_e, weight, n, 0.f, budget, ws->counters + CNT_CLOSEST, max_passes - 1 - pass, sel, hist,
+                                            flags, block_counts, tie_offsets, d_count, lists[(pass + 1) & 1], s->sm_count, st, &info);
     }
     if (err != cudaSuccess) return fail(RT_ERR_CUDA, "%s: %s", fn, cudaGetErrorString(err));
     if (pass < 16) out.pixels_in_pass[pass] = n_cur;
@@ -853,6 +873,7 @@ static int render_adaptive_passes(const char* fn, rt_scene* s, const rt_render_p
   CU(cudaMemcpyAsync(out_rgb, em, n3, cudaMemcpyDeviceToHost, st));
   if (out_err) CU(cudaMemcpyAsync(out_err, ev, n3, cudaMemcpyDeviceToHost, st));
   if (out_samples) CU(cudaMemcpyAsync(out_samples, lists[0], (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+  if (out_rays) CU(cudaMemcpyAsync(out_rays, n_rays, (size_t)n * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
   CU(cudaMemcpyAsync(ws->counters_host, ws->counters, CNT_SLOTS * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
   CU(cudaEventRecord(ws->t1, st));
   CU(cudaStreamSynchronize(st));
@@ -872,13 +893,20 @@ static int render_adaptive_passes(const char* fn, rt_scene* s, const rt_render_p
 
 extern "C" int rt_render_adaptive(rt_scene* s, const rt_render_params* p, const rt_adaptive_params* ap, float* out_rgb, float* out_err,
                                   int32_t* out_samples, rt_adaptive_stats* stats) {
-  return render_adaptive_passes("rt_render_adaptive", s, p, ap, -1, out_rgb, out_err, out_samples, stats);
+  return render_adaptive_passes("rt_render_adaptive", s, p, ap, ADAPT_THRESHOLD, 0, out_rgb, out_err, out_samples, nullptr, stats);
 }
 
 extern "C" int rt_render_adaptive_budget(rt_scene* s, const rt_render_params* p, const rt_adaptive_params* ap, int64_t sample_budget,
                                          float* out_rgb, float* out_err, int32_t* out_samples, rt_adaptive_stats* stats) {
   if (sample_budget < 0) return fail(RT_ERR_INVALID, "rt_render_adaptive_budget: sample_budget %lld", (long long)sample_budget);
-  return render_adaptive_passes("rt_render_adaptive_budget", s, p, ap, sample_budget, out_rgb, out_err, out_samples, stats);
+  return render_adaptive_passes("rt_render_adaptive_budget", s, p, ap, ADAPT_SAMPLES, sample_budget, out_rgb, out_err, out_samples, nullptr,
+                                stats);
+}
+
+extern "C" int rt_render_adaptive_rays(rt_scene* s, const rt_render_params* p, const rt_adaptive_params* ap, int64_t ray_budget,
+                                       float* out_rgb, float* out_err, int32_t* out_samples, int64_t* out_rays, rt_adaptive_stats* stats) {
+  return render_adaptive_passes("rt_render_adaptive_rays", s, p, ap, ADAPT_RAYS, ray_budget, out_rgb, out_err, out_samples, out_rays,
+                                stats);
 }
 
 // ------------------------------------------------------------------------------------ probes

@@ -33,6 +33,7 @@ struct ErrArgs {
   int err_bpp;             // batches per pixel slot of a task (32 / G), set by the launcher
   unsigned err_magic;      // multiply-shift magic of x / err_bpp for x < 32
   int32_t estimator;       // RT_ERR_EST_*: how err_store forms SE^2 from the batch sums
+  int32_t* err_rays;       // optional [entries]: closest-hit rays each traced pixel cost in the pass (RT_HIT_RAY_COUNT's count)
 };
 
 struct LaunchInfo {
@@ -53,29 +54,39 @@ cudaError_t launch_pt_warp(const SceneView<float>& sc, const RenderArgs& a, cuda
                            int n_nodes, int n_prims, int tree_depth);
 // the same kernels instantiated with per-pixel error accumulation (ERR): no image is stored; every traced
 // pixel gets its pass mean (the value launch_pt_warp stores, bit for bit) and squared standard error in
-// e.err_mean / e.err_var, indexed by list entry (e.pix_list) or pixel; needs S >= 2 and no partition
+// e.err_mean / e.err_var, and with e.err_rays its closest-hit rays, indexed by list entry (e.pix_list) or pixel;
+// needs S >= 2 and no partition
 cudaError_t launch_pt_warp_err(const SceneView<float>& sc, const RenderArgs& a, const ErrArgs& e, cudaStream_t st, int sm_count,
                                LaunchInfo* info, const char** why_not, int n_nodes, int n_prims, int tree_depth);
 // rt_adaptive.cu: fold a pass into the per-pixel sums, then compact the pixels still to trace
 cudaError_t launch_adaptive_combine(const ErrArgs& e, int pass, int max_passes, float target, float floor_, float* sum_m, float* sum_v,
                                     int32_t* n_pass, uint8_t* flags, int32_t* block_counts, int32_t* d_count, int32_t* next_list, int n_pixels,
                                     cudaStream_t st, LaunchInfo* info);
-// rt_adaptive.cu, sample-budget mode: the radix select's state between its kernels (device memory, zeroed once a call)
+// rt_adaptive.cu, budget modes: the radix select's state between its kernels (device memory, zeroed once a call)
 struct BudgetSelect {
-  unsigned prefix;  // digits of the K-th largest key T picked so far (after the last digit: T)
-  int k_rem;        // rank of T among the keys with this prefix (after the last digit: the ties with key T to take)
-  int K, C;         // pixels the next pass traces, candidates (e > target)
-  int scratch;      // total of the tie-offset scan
-  int pad_[3];
+  unsigned prefix;  // digits of the key T picked so far (after the last digit: T, the key at which the prefix is cut)
+  int pad_;
+  long long rem;    // weight of the prefix still to take among the keys with these digits (after the last digit: among the ties)
+  long long want;   // the spend target of the next pass, in weight
+  long long W;      // the candidates' total weight
+  long long scratch;  // total of the tie-offset scan
 };
 // fold a pass into the per-pixel sums and store e of every traced pixel in err_e
 cudaError_t launch_adaptive_combine_budget(const ErrArgs& e, int pass, float floor_, float* sum_m, float* sum_v, int32_t* n_pass,
                                            float* err_e, int n_pixels, cudaStream_t st, LaunchInfo* info);
-// list the K = min(C, Q, max(ceil(C/2), ceil(Q/r))) pixels of largest e (ties: lower pixel index first) in next_list, in
-// ascending order, and K in *d_count; Q = passes of one pixel the budget still pays for, r = passes left; hist: 256 zeros
-cudaError_t launch_adaptive_select_budget(const float* err_e, int n_pixels, float target, long long Q, int r, BudgetSelect* sel,
-                                          int32_t* hist, uint8_t* flags, int32_t* block_counts, int32_t* d_count, int32_t* next_list,
-                                          int sm_count, cudaStream_t st, LaunchInfo* info);
+// ray-budget mode: as above, and e.err_rays of every traced pixel into its ray total n_rays; err_e then holds the
+// selection key (e > target ? max(e / sqrt((P + 1) w), FLT_MIN) : 0) and weight the predicted rays w = ceil(n_rays / P)
+cudaError_t launch_adaptive_combine_rays(const ErrArgs& e, int pass, float target, float floor_, float* sum_m, float* sum_v, int32_t* n_pass,
+                                         long long* n_rays, int32_t* weight, float* err_e, int n_pixels, cudaStream_t st, LaunchInfo* info);
+// the longest prefix of the order (key descending, pixel index ascending) over the candidates (key = e > target ?
+// bits(e) : 0, key > 0) whose weight (weight[px], or 1 without weights) sums to at most T = min(rem, max(ceil(W / 2),
+// ceil(rem / r))), W the candidates' weight, rem = budget - *spent (budget without `spent`; rem <= 0: T = 0), r = passes
+// left; the pixels in next_list in ascending order and their number in *d_count.  hist: 256 zeros.  Without weights
+// and spent this is K = min(C, Q, max(ceil(C/2), ceil(Q/r))) pixels for Q = budget.
+cudaError_t launch_adaptive_select_budget(const float* err_e, const int32_t* weight, int n_pixels, float target, long long budget,
+                                          const unsigned long long* spent, int r, BudgetSelect* sel, unsigned long long* hist, uint8_t* flags,
+                                          int32_t* block_counts, long long* tie_offsets, int32_t* d_count, int32_t* next_list, int sm_count,
+                                          cudaStream_t st, LaunchInfo* info);
 cudaError_t launch_adaptive_final(const float* sum_m, const float* sum_v, const int32_t* n_pass, int spp, int n_pixels, float* rgb, float* err,
                                   int32_t* samples, cudaStream_t st, LaunchInfo* info);
 

@@ -515,7 +515,8 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
   float* acc = reinterpret_cast<float*>(slot_rays + 32);   // ACC_SEG: [32][3]; ACC_LANES: [G][3][32]
   // ERR: batch sums [32][3] behind the accumulator (ACC_REG has neither slot_rays nor acc: they go there)
   float* bsum = ACC == ACC_REG ? reinterpret_cast<float*>(slot_rays) : acc + (ACC == ACC_SEG ? 96 : 96 * cfg.group);
-  const bool count_rays = a.out_hit != nullptr && a.hit_mode == RT_HIT_RAY_COUNT;
+  // (ERR: each pixel's count goes to ea.err_rays instead of the side image)
+  const bool count_rays = ERR ? ea.err_rays != nullptr : a.out_hit != nullptr && a.hit_mode == RT_HIT_RAY_COUNT;
 
   const PixelMap pm = ERR ? make_pixel_map_list(a, ea) : make_pixel_map(a);
   const int N = a.num_of_rays;
@@ -828,6 +829,7 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
       __syncwarp();
       for (int g = 0; g < G && p0 + g < pm.n_pixels; ++g)
         err_store(ea, L, bsum, g, p0 + g, mk3<float>(acc[3 * g] * inv_spp, acc[3 * g + 1] * inv_spp, acc[3 * g + 2] * inv_spp), lane);
+      if (count_rays && lane < G && p0 + lane < pm.n_pixels) ea.err_rays[p0 + lane] = slot_rays[lane];
       __syncwarp();
     } else if (ACC == ACC_SEG) {
       __syncwarp();
@@ -852,7 +854,10 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
         }
         const long long p = p0 + g;
         if (ERR) {
-          if (p < pm.n_pixels) err_store(ea, L, bsum, g, p, mk3<float>(r * inv_spp, gr * inv_spp, b * inv_spp), lane);
+          if (p < pm.n_pixels) {
+            err_store(ea, L, bsum, g, p, mk3<float>(r * inv_spp, gr * inv_spp, b * inv_spp), lane);
+            if (count_rays && lane == 0) ea.err_rays[p] = slot_rays[g];
+          }
         } else if (lane == 0 && p < pm.n_pixels) {
           int col, row;
           pm.locate(p, col, row);
@@ -872,6 +877,7 @@ k_pt_warp(const __grid_constant__ SceneView<float> sc, const __grid_constant__ R
         if (p0 < pm.n_pixels) {
           __syncwarp();  // the batch sums of the task are complete
           err_store(ea, L, bsum, 0, p0, mk3<float>(sr * inv_spp, sg * inv_spp, sb_ * inv_spp), lane);
+          if (count_rays && lane == 0) ea.err_rays[p0] = (int)task_rays;
         }
         __syncwarp();
       } else if (lane == 0 && p0 < pm.n_pixels) {

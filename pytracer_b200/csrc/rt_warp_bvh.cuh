@@ -80,7 +80,8 @@ k_pt_warp_bvh(const __grid_constant__ SceneView<float> sc, const __grid_constant
   float* acc = reinterpret_cast<float*>(slot_rays + 32);  // [G][3][32]
   float2* walk_stacks = reinterpret_cast<float2*>(acc + cfg.group * 96);  // [stack_entries][32]
   float* bsum = reinterpret_cast<float*>(walk_stacks + bcfg.stack_entries * 32);  // ERR: [32][3] batch sums
-  const bool count_rays = a.out_hit != nullptr && a.hit_mode == RT_HIT_RAY_COUNT;
+  // (ERR: each pixel's count goes to ea.err_rays instead of the side image)
+  const bool count_rays = ERR ? ea.err_rays != nullptr : a.out_hit != nullptr && a.hit_mode == RT_HIT_RAY_COUNT;
   const float* planes = sc.invm + 12 * (size_t)sc.n_spheres;
   const int n_planes = sc.n_shapes - sc.n_spheres;
 
@@ -328,7 +329,10 @@ k_pt_warp_bvh(const __grid_constant__ SceneView<float> sc, const __grid_constant
       }
       const long long p = p0 + g;
       if (ERR) {
-        if (p < pm.n_pixels) err_store(ea, L, bsum, g, p, mk3<float>(r * inv_spp, gr * inv_spp, b * inv_spp), lane);
+        if (p < pm.n_pixels) {
+          err_store(ea, L, bsum, g, p, mk3<float>(r * inv_spp, gr * inv_spp, b * inv_spp), lane);
+          if (count_rays && lane == 0) ea.err_rays[p] = slot_rays[g];
+        }
       } else if (lane == 0 && p < pm.n_pixels) {
         int col, row;
         pm.locate(p, col, row);

@@ -117,6 +117,27 @@ class DeviceScene:
                                                           _ptr(err), _ptr(samples), C.byref(stats)))
         return out, err, samples, stats.as_dict()
 
+    def render_rays(self, params: _abi.rt_render_params, ray_budget: int, max_passes: int, target_error: float = 0.0,
+                    error_floor: float = 1e-2, out: Optional[np.ndarray] = None, estimator: str = "batch"):
+        """rt_render_adaptive_rays: (mean image, SE image, samples per pixel, closest-hit rays per pixel (int64), stats)
+        from a budget of ``ray_budget`` closest-hit rays and at most ``max_passes`` passes: pass 0 traces every pixel,
+        every further pass the pixels of largest error drop per predicted ray above ``target_error`` (rt_api.h gives
+        the rule)."""
+        H, W = params.height, params.width
+        if out is None:
+            out = np.empty((H, W, 3), dtype=np.float32)
+        assert out.dtype == np.float32 and out.shape == (H, W, 3) and out.flags.c_contiguous
+        err = np.empty((H, W, 3), dtype=np.float32)
+        samples = np.empty((H, W), dtype=np.int32)
+        rays = np.empty((H, W), dtype=np.int64)
+        ap = _abi.rt_adaptive_params()
+        ap.target_error, ap.error_floor, ap.max_passes = float(target_error), float(error_floor), int(max_passes)
+        ap.estimator = _abi.ERROR_ESTIMATORS[estimator] if isinstance(estimator, str) else int(estimator)
+        stats = _abi.rt_adaptive_stats()
+        _native.check(self._lib.rt_render_adaptive_rays(self._handle, C.byref(params), C.byref(ap), int(ray_budget), _ptr(out), _ptr(err),
+                                                        _ptr(samples), _ptr(rays), C.byref(stats)))
+        return out, err, samples, rays, stats.as_dict()
+
     def render_device(self, params: _abi.rt_render_params, out_ptr: int, hit_ptr: int = 0, stream: int = 0) -> None:
         """rt_render_device: enqueue on ``stream`` writing to device memory at ``out_ptr``."""
         _native.check(self._lib.rt_render_device(self._handle, C.byref(params), C.c_void_p(out_ptr),

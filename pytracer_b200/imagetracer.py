@@ -33,11 +33,13 @@ from .scene import Color, Point, Ray, Vec
 @dataclass
 class AdaptiveResult:
     """What ``fire_all_rays_adaptive`` returns besides the image: the standard error of every pixel's mean
-    (float32 [H][W][3]), the samples every pixel received (int32 [H][W]), the passes run and the call's counters."""
+    (float32 [H][W][3]), the samples every pixel received (int32 [H][W]), the passes run and the call's counters; with
+    a ray budget also the closest-hit rays every pixel received (int64 [H][W])."""
     error: np.ndarray
     samples: np.ndarray
     passes: int
     stats: dict = field(default_factory=dict)
+    rays: Optional[np.ndarray] = None
 
 
 class ImageTracer:
@@ -77,7 +79,7 @@ class ImageTracer:
     def fire_all_rays_adaptive(self, renderer, target_error: float = 0.0, max_samples_per_pixel: Optional[int] = None,
                                error_floor: float = 1e-2, callback=None, callback_time_s: float = 2.0,
                                error_estimator: str = "batch", mean_samples_per_pixel: Optional[int] = None,
-                               **callback_kwargs) -> AdaptiveResult:
+                               mean_rays_per_pixel: Optional[float] = None, **callback_kwargs) -> AdaptiveResult:
         """Path-traced image with a per-pixel Monte Carlo error map, optionally refined where it is noisy.
 
         Pass 0 is exactly ``fire_all_rays(renderer)``; every further pass traces ``samples_per_side ** 2`` more
@@ -94,7 +96,14 @@ class ImageTracer:
         (mean x width x height in all, the first pass included) instead of a threshold: after pass 0 every pass traces
         the pixels of largest relative error above ``target_error`` (0: any error), at least half of them while the
         budget lasts, until the budget or ``max_samples_per_pixel`` (then required: at least the mean and a multiple
-        of ``samples_per_side ** 2``) runs out; include/rt_api.h (rt_render_adaptive_budget) states the rule."""
+        of ``samples_per_side ** 2``) runs out; include/rt_api.h (rt_render_adaptive_budget) states the rule.
+
+        With ``mean_rays_per_pixel`` the budget is R = floor(mean x width x height) closest-hit rays instead (the unit
+        ``stats["rays_closest"]`` counts, the first pass included whatever it costs): after pass 0 every pass traces
+        the pixels whose next pass buys the largest drop in relative variance per predicted ray, until R or
+        ``max_samples_per_pixel`` (then required) runs out; ``stats["ray_budget"]`` holds R and the result's ``rays``
+        the rays of every pixel.  It excludes ``mean_samples_per_pixel``; include/rt_api.h (rt_render_adaptive_rays)
+        states the rule."""
         spp = self.samples_per_side ** 2
         if not isinstance(renderer, CudaRenderer) or renderer.algorithm != "pathtracing":
             raise ValueError("fire_all_rays_adaptive needs a path-tracing CudaRenderer")
@@ -112,6 +121,17 @@ class ImageTracer:
             raise ValueError(f"error_estimator must be one of {sorted(_abi.ERROR_ESTIMATORS)} (got {error_estimator!r})")
         if error_estimator == "paired" and self.samples_per_side % 2:
             raise ValueError(f"the paired error estimator needs an even samples_per_side (got {self.samples_per_side})")
+        ray_budget = None
+        if mean_rays_per_pixel is not None:
+            if mean_samples_per_pixel is not None:
+                raise ValueError("mean_rays_per_pixel and mean_samples_per_pixel exclude each other")
+            if not (np.isfinite(mean_rays_per_pixel) and mean_rays_per_pixel >= 0):
+                raise ValueError(f"mean_rays_per_pixel must be finite and >= 0 (got {mean_rays_per_pixel})")
+            if max_samples_per_pixel is None:
+                raise ValueError("mean_rays_per_pixel needs max_samples_per_pixel")
+            ray_budget = int(np.floor(float(mean_rays_per_pixel) * self.image.width * self.image.height))
+            if ray_budget >= 2 ** 63:
+                raise ValueError(f"mean_rays_per_pixel ({mean_rays_per_pixel}) is too large")
         if mean_samples_per_pixel is not None:
             if int(mean_samples_per_pixel) != mean_samples_per_pixel or mean_samples_per_pixel < spp:
                 raise ValueError(f"mean_samples_per_pixel ({mean_samples_per_pixel}) must be an integer of at least the "
@@ -130,7 +150,12 @@ class ImageTracer:
         if callback:
             callback(col=0, row=0, **callback_kwargs)
         scene = renderer.device_scene()
-        if mean_samples_per_pixel is None:
+        rays = None
+        if ray_budget is not None:
+            rgb, err, samples, rays, stats = scene.render_rays(self._params(renderer), ray_budget, max_passes, target_error, error_floor,
+                                                               out=self._adoptable_buffer(), estimator=error_estimator)
+            stats["ray_budget"] = ray_budget
+        elif mean_samples_per_pixel is None:
             rgb, err, samples, stats = scene.render_adaptive(self._params(renderer), target_error, max_passes, error_floor,
                                                              out=self._adoptable_buffer(), estimator=error_estimator)
         else:
@@ -146,7 +171,7 @@ class ImageTracer:
         install_array(self.image, rgb)
         if callback:
             callback(col=self.image.width - 1, row=self.image.height - 1, **callback_kwargs)
-        return AdaptiveResult(error=err, samples=samples, passes=passes, stats=stats)
+        return AdaptiveResult(error=err, samples=samples, passes=passes, stats=stats, rays=rays)
 
     # -- the product path
     def _fire_cuda(self, renderer: CudaRenderer, comm=None) -> None:

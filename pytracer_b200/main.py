@@ -60,9 +60,9 @@ def load_scene(path: str, variables, parser: str):
 
 
 def adaptive_cli_problem(algorithm, samples_per_pixel, gpus, variant, precision, target_error, max_samples_per_pixel,
-                         error_floor, error_estimator="batch", mean_samples_per_pixel=None):
-    """Why `render --error-output / --target-error / --max-samples-per-pixel / --mean-samples-per-pixel` cannot run as
-    asked (None: it can)."""
+                         error_floor, error_estimator="batch", mean_samples_per_pixel=None, mean_rays_per_pixel=None):
+    """Why `render --error-output / --target-error / --max-samples-per-pixel / --mean-samples-per-pixel /
+    --mean-rays-per-pixel` cannot run as asked (None: it can)."""
     if algorithm != "pathtracing":
         return "--error-output, --target-error and --max-samples-per-pixel need --algorithm pathtracing"
     if samples_per_pixel < 4:
@@ -75,7 +75,14 @@ def adaptive_cli_problem(algorithm, samples_per_pixel, gpus, variant, precision,
         return f"--target-error must be a finite number >= 0 (got {target_error})"
     if not error_floor > 0:
         return f"--error-floor must be > 0 (got {error_floor})"
-    if mean_samples_per_pixel is None:
+    if mean_rays_per_pixel is not None:
+        if mean_samples_per_pixel is not None:
+            return "--mean-rays-per-pixel and --mean-samples-per-pixel exclude each other"
+        if not (mean_rays_per_pixel >= 0 and mean_rays_per_pixel != float("inf")):
+            return f"--mean-rays-per-pixel must be a finite number >= 0 (got {mean_rays_per_pixel})"
+        if max_samples_per_pixel is None:
+            return "--mean-rays-per-pixel needs --max-samples-per-pixel"
+    elif mean_samples_per_pixel is None:
         if (target_error is not None and target_error > 0) != (max_samples_per_pixel is not None):
             return "--target-error and --max-samples-per-pixel go together"
     elif max_samples_per_pixel is None:
@@ -126,6 +133,9 @@ def cli():
 @click.option("--mean-samples-per-pixel", type=int, default=None,
               help="render to a sample budget of this many samples per pixel on average (with --max-samples-per-pixel): "
                    "after the first pass, trace the pixels of largest relative error (above --target-error, if given)")
+@click.option("--mean-rays-per-pixel", type=float, default=None,
+              help="render to a budget of this many closest-hit rays per pixel on average (with --max-samples-per-pixel): after "
+                   "the first pass, trace the pixels whose next pass buys the most error reduction per predicted ray")
 @click.option("--error-floor", type=float, default=1e-2, help="radiance below which the relative error is taken against this floor")
 @click.option("--error-estimator", type=click.Choice(["batch", "paired"]), default="batch",
               help="how the standard error is formed: batch (strata as independent samples) or paired (collapsed pairs "
@@ -133,7 +143,7 @@ def cli():
 @click.argument("input_scene_name", type=str)
 def render(width, height, algorithm, pfm_output, png_output, num_of_rays, max_depth, init_state, init_seq,
            samples_per_pixel, declare_float, variant, precision, parser, accel, gpus, launcher, error_output, target_error,
-           max_samples_per_pixel, mean_samples_per_pixel, error_floor, error_estimator, input_scene_name):
+           max_samples_per_pixel, mean_samples_per_pixel, mean_rays_per_pixel, error_floor, error_estimator, input_scene_name):
     import os
 
     if gpus > 1 and launcher == "torchrun" and "WORLD_SIZE" not in os.environ:  # one process per GPU: hand the same command line to torchrun
@@ -151,14 +161,14 @@ def render(width, height, algorithm, pfm_output, png_output, num_of_rays, max_de
         print(f"Error, the number of samples per pixel ({samples_per_pixel}) must be a perfect square")
         return
     adaptive = (error_output is not None or target_error is not None or max_samples_per_pixel is not None
-                or mean_samples_per_pixel is not None)
+                or mean_samples_per_pixel is not None or mean_rays_per_pixel is not None)
     if error_estimator != "batch" and not adaptive:
         print("Error, --error-estimator applies to --error-output and --target-error")
         sys.exit(1)
     if adaptive:
         problem = adaptive_cli_problem(algorithm, samples_per_pixel, gpus, variant, precision, target_error,
                                        max_samples_per_pixel, error_floor, error_estimator,
-                                       mean_samples_per_pixel=mean_samples_per_pixel)
+                                       mean_samples_per_pixel=mean_samples_per_pixel, mean_rays_per_pixel=mean_rays_per_pixel)
         if problem:
             print(f"Error, {problem}")
             sys.exit(1)
@@ -193,7 +203,8 @@ def render(width, height, algorithm, pfm_output, png_output, num_of_rays, max_de
     if adaptive:
         result = tracer.fire_all_rays_adaptive(renderer, target_error=target_error or 0.0,
                                                max_samples_per_pixel=max_samples_per_pixel, error_floor=error_floor,
-                                               error_estimator=error_estimator, mean_samples_per_pixel=mean_samples_per_pixel)
+                                               error_estimator=error_estimator, mean_samples_per_pixel=mean_samples_per_pixel,
+                                               mean_rays_per_pixel=mean_rays_per_pixel)
     else:
         tracer.fire_all_rays(renderer, comm=comm)
     elapsed = perf_counter() - start
@@ -205,7 +216,8 @@ def render(width, height, algorithm, pfm_output, png_output, num_of_rays, max_de
         print(f"{result.passes} pass(es) of {samples_per_pixel} samples; pixels per pass: "
               f"{', '.join(str(n) for n in st['pixels_in_pass'])}; {st['samples']} samples in all "
               f"({st['samples'] / (width * height):.1f} per pixel)"
-              + (f"; budget {st['sample_budget']} samples, {st['samples']} spent" if "sample_budget" in st else ""))
+              + (f"; budget {st['sample_budget']} samples, {st['samples']} spent" if "sample_budget" in st else "")
+              + (f"; budget {st['ray_budget']} rays, {st['rays_closest']} spent" if "ray_budget" in st else ""))
     if comm is not None and comm.rank != 0:
         return
     with open(pfm_output, "wb") as outf:

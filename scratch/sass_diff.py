@@ -19,7 +19,7 @@ def functions(path):
                 out[name] = body
             name, body = m.group(1), []
         elif name:
-            s = re.sub(r"/\*[0-9a-f]{4,}\*/", "", line).strip()  # instruction addresses
+            s = " ".join(re.sub(r"/\*[0-9a-f]{4,}\*/", "", line).split())  # instruction addresses; column widths
             if s and not s.startswith("/* 0x"):
                 body.append(s)
     if name:
